@@ -3,9 +3,18 @@
 TSP/VRP/IRP-50 greedy, at 1/2/4/8 B200).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--kind tsp] [--nodes 50] [--batch B]
+                    [--dump-outputs DIR]
 
 One "step" = one full greedy rollout (encoder forward + every decode step + every environment transition) over one
-batch of synthetic uniform instances.  Rank 0 prints ONE JSON line.  See DESIGN.md §6.
+batch of synthetic uniform instances; every timed GPU workload runs K steps (the cpu_baseline leg times one step of its
+bounded CPU sample).  Rank 0 prints ONE JSON line.  See DESIGN.md §6.
+
+  --dump-outputs DIR   after the timed steps, rank 0 writes what the headline workload computed in its last step as
+             DIR/<name>.npy (float32 / float64): costs, log-probs, action tapes and embeddings of a fixed sample of
+             instances for a rollout; rewards, log-probs, loss and the updated weights for --mode train.  The instances
+             and weights follow from --seed, so two builds run with the same arguments can be compared array by array:
+             a greedy rollout repeats bit for bit; a train step does not (float atomics in the backward perturb the
+             warm-up updates, and the sampled rollouts follow), so its arrays agree to rounding and in distribution.
 
   value / ms_per_step / roofline / e2e / cpu_baseline   the HEADLINE workload: greedy TSP-50, 65,536 instances per GPU
       value      whole-job instance-steps/s with the instances already resident in HBM (Philox on device)
@@ -67,7 +76,34 @@ def parse():
     ap.add_argument("--seed", type=int, default=69)
     ap.add_argument("--mode", default="rollout", choices=["rollout", "train"],
                     help="headline = greedy rollout (default) or one REINFORCE step (BASELINE.json configs[3])")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the headline workload computed in its last timed step to DIR/<name>.npy")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    return a
+
+
+def _sample(n, k):
+    """A fixed sorted sample of k of the indices 0..n-1 (all of them when n <= k), the same in every run."""
+    if n <= k:
+        return np.arange(n)
+    return np.sort(np.random.RandomState(0).choice(n, k, replace=False))
+
+
+def _to_host(t, rows=None):
+    t = t.detach()
+    if rows is not None:
+        t = t[torch.as_tensor(rows, device=t.device)]
+    t = t.cpu()
+    return t.numpy().astype(np.float64 if t.dtype == torch.float64 else np.float32)
+
+
+def write_outputs(d, arrays):
+    """--dump-outputs: one float32/float64 .npy per array (well under 64 MB in all, see the two dump sites)."""
+    os.makedirs(d, exist_ok=True)
+    for name, arr in arrays.items():
+        np.save(os.path.join(d, name + ".npy"), arr)
 
 
 # ------------------------------------------------------------------------------------------------ CPU arms
@@ -277,7 +313,7 @@ def _traffic(kind, N, B):
 
 
 # ------------------------------------------------------------------------------------------------ greedy rollout
-def rollout_workload(a, ctx, kind, N, B, steps, warmup, with_e2e):
+def rollout_workload(a, ctx, kind, N, B, steps, warmup, with_e2e, dump=None):
     import vrpx
     from agents.graph_encoder import run_encoder
 
@@ -291,7 +327,7 @@ def rollout_workload(a, ctx, kind, N, B, steps, warmup, with_e2e):
     env = Env(N, B, 0, seed=a.seed, instance_rng="philox", instance_offset=ctx.rank * B)  # shard = own reference batch
     ev = lambda: torch.cuda.Event(enable_timing=True)
 
-    def one_step(events=None):
+    def one_step(events=None, keep_emb=False):
         env.restart_episode()
         if events is not None:
             events[0].record()
@@ -303,6 +339,8 @@ def rollout_workload(a, ctx, kind, N, B, steps, warmup, with_e2e):
             out = model.decoder.rollout_episode(env, h, greedy=True, coupling=model.coupling)
             if events is not None:
                 events[2].record()
+        if keep_emb:  # only the dumped step: an earlier step's h would stay alive during the next one
+            out["emb"] = h
         return out
 
     for _ in range(max(warmup, 3)):
@@ -319,7 +357,7 @@ def rollout_workload(a, ctx, kind, N, B, steps, warmup, with_e2e):
         vrpx.lib().vrpx_debug_rollout_split(0)
     vrpx.lib().vrpx_debug_rollout_timing(1)  # CUDA events around the decode launches alone, on their launch stream
     for i in range(steps):
-        out = one_step(per_step_events[i])
+        out = one_step(per_step_events[i], keep_emb=dump is not None and i == steps - 1)
         total_inst_steps += out["steps"] * B  # includes the .item() sync on the step count
         kernel_ms.append(float(vrpx.lib().vrpx_debug_rollout_kernel_ms()))  # the step is already synchronised
     e1.record()
@@ -332,6 +370,14 @@ def rollout_workload(a, ctx, kind, N, B, steps, warmup, with_e2e):
     mean_cost = float(out["cost"].mean().item())
     vrpx.lib().vrpx_debug_rollout_timing(0)
     kern_ms = float(np.mean(kernel_ms))
+    if dump is not None:
+        # per-instance results of up to 131,072 instances, the action tapes of 8,192 and the embeddings of 256:
+        # at most 0.5 + 0.5 + 8.4 + 16.8 MB (N <= 128, at most 2N - 1 steps)
+        inst, tape_rows, emb_rows = _sample(B, 1 << 17), _sample(B, 8192), _sample(B, 256)
+        dump.update(cost=_to_host(out["cost"], inst), logp=_to_host(out["logp"], inst),
+                    tape=_to_host(out["tape"].t(), tape_rows).T.copy(), emb=_to_host(out["emb"], emb_rows),
+                    steps=np.array([out["steps"]], dtype=np.float64), instances=inst.astype(np.float64),
+                    tape_instances=tape_rows.astype(np.float64), emb_instances=emb_rows.astype(np.float64))
 
     e2e_ms, e2e_inst_steps, n_e2e, h2d, d2h = 0.0, 0.0, 0, 0, 0
     if with_e2e:
@@ -395,7 +441,7 @@ def rollout_workload(a, ctx, kind, N, B, steps, warmup, with_e2e):
 
 
 # ------------------------------------------------------------------------------------------------ train step
-def train_workload(a, ctx, kind, N, B, steps, warmup):
+def train_workload(a, ctx, kind, N, B, steps, warmup, dump=None):
     """One step = the body of TSPAgent.train's epoch without baseline_update (graph_tsp_agent.py:176-186): reset,
     sampled rollout with grad (train-mode BatchNorm), sampled baseline rollout, REINFORCE loss, backward, gradient
     all-reduce over ranks (NCCL; a no-op on one GPU), Adam."""
@@ -417,12 +463,14 @@ def train_workload(a, ctx, kind, N, B, steps, warmup):
         ar_events.append((x0, x1))
 
     agent._allreduce_gradients = timed_allreduce
+    last = {}
 
     def one():
         agent.model.train()
         loss_m, loss_b, logp = agent.step(env, (False, True))
         adv = (loss_m - loss_b) * -1
         loss = agent.policy_gradient_step(adv, logp)
+        last.update(reward=loss_m, baseline_reward=loss_b, logp=logp, loss=loss)
         return env.step_count, float(loss)
 
     for _ in range(max(warmup, 3)):
@@ -442,6 +490,12 @@ def train_workload(a, ctx, kind, N, B, steps, warmup):
     w1 = time.perf_counter()
     ms = e0.elapsed_time(e1)
     ar_ms = sum(x0.elapsed_time(x1) for x0, x1 in ar_events) / steps
+    if dump is not None:
+        # per-instance rewards and log-probs of up to 131,072 instances (1.5 MB) and the updated weights (4.6 MB)
+        inst = _sample(B, 1 << 17)
+        dump.update({k: _to_host(last[k], inst) for k in ("reward", "baseline_reward", "logp")})
+        dump.update(loss=_to_host(last["loss"].reshape(1)), instances=inst.astype(np.float64))
+        dump.update({"param." + k: _to_host(v) for k, v in agent.model.state_dict().items() if v.is_floating_point()})
     (ms, ar_ms), (inst_steps,) = ctx.reduce([ms, ar_ms], [float(inst_steps)])
     res = None
     if ctx.rank == 0:
@@ -478,20 +532,22 @@ def main():
 
     ctx = Ctx(a)
     B, N = a.batch, a.nodes
+    dump = {} if (a.dump_outputs and ctx.rank == 0) else None
     if a.mode == "train":
-        head = train_workload(a, ctx, a.kind, N, B, a.steps, a.warmup)
+        head = train_workload(a, ctx, a.kind, N, B, a.steps, a.warmup, dump=dump)
         metric = "train_instance_steps_per_sec"
     else:
-        head = rollout_workload(a, ctx, a.kind, N, B, a.steps, a.warmup, with_e2e=True)
+        head = rollout_workload(a, ctx, a.kind, N, B, a.steps, a.warmup, with_e2e=True, dump=dump)
         metric = "instance_steps_per_sec"
+    if dump is not None:
+        write_outputs(a.dump_outputs, dump)
     extras = {}
     default_headline = (a.mode, a.kind, N, B) == ("rollout", "tsp", 50, 65536)
     if default_headline and not a.no_extras and not a.no_split:
-        k = max(2, min(a.steps, 5))
-        extras["vrp50_greedy_b65536"] = rollout_workload(a, ctx, "vrp", 50, 65536, k, 3, with_e2e=False)
-        extras["irp50_greedy_b65536"] = rollout_workload(a, ctx, "irp", 50, 65536, k, 3, with_e2e=False)
-        extras["c4_train_step_tsp50_b65536"] = train_workload(a, ctx, "tsp", 50, 65536, max(2, min(a.steps, 3)), 3)
-        extras["c5_vrp100_greedy_b131072"] = rollout_workload(a, ctx, "vrp", 100, 131072, max(2, min(a.steps, 3)), 3, with_e2e=False)
+        extras["vrp50_greedy_b65536"] = rollout_workload(a, ctx, "vrp", 50, 65536, a.steps, 3, with_e2e=False)
+        extras["irp50_greedy_b65536"] = rollout_workload(a, ctx, "irp", 50, 65536, a.steps, 3, with_e2e=False)
+        extras["c4_train_step_tsp50_b65536"] = train_workload(a, ctx, "tsp", 50, 65536, a.steps, 3)
+        extras["c5_vrp100_greedy_b131072"] = rollout_workload(a, ctx, "vrp", 100, 131072, a.steps, 3, with_e2e=False)
     if ctx.rank == 0:
         line = {"metric": metric, "value": head["value"], "unit": "instance-steps/s", "n_gpus": ctx.world,
                 "steps": a.steps, "warmup": max(a.warmup, 3), "ms_per_step": head["ms_per_step"], "higher_is_better": True,

@@ -13,19 +13,15 @@ GOLDEN = os.path.join(ROOT, "tests", "golden")
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a B200 (sm_100) GPU; run with `-m gpu` on the GPU box")
-    config.addinivalue_line("markers", "reference: needs /root/reference (build container only)")
 
 
 def pytest_collection_modifyitems(config, items):
     import torch
 
     have_gpu = torch.cuda.is_available()
-    have_ref = os.path.isdir("/root/reference/agents")
     for item in items:
         if "gpu" in item.keywords and not have_gpu:
             item.add_marker(pytest.mark.skip(reason="no CUDA device in this container"))
-        if "reference" in item.keywords and not have_ref:
-            item.add_marker(pytest.mark.skip(reason="/root/reference not present"))
 
 
 @pytest.fixture(scope="session")

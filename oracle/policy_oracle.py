@@ -31,9 +31,17 @@ def _bn(x2d, sd, prefix, train, eps=1e-5):
     return (x2d - mean) / torch.sqrt(var + eps) * w + b
 
 
-def encoder_forward(sd, x, depot_onehot=None, train=False, num_layers=3):
+def encoder_forward(sd, x, depot_onehot=None, train=False, num_layers=3, chunk=None, relu=None):
     """graph_encoder.py:41-58 (GraphEncoder) / :95-138 (GraphDemandEncoder) /
-    :183-198 (MultiHeadAttentionLayer).  x (B,N,f) f32; depot_onehot (B,N) bool or None."""
+    :183-198 (MultiHeadAttentionLayer).  x (B,N,f) f32; depot_onehot (B,N) bool or None.
+
+    chunk (optional): run attention and feed-forward on `chunk` instances at a time, so that a large batch (or its
+    float64 / forward-mode evaluation) fits in memory.  BatchNorm statistics still span all B*N rows; the arithmetic
+    is the same as with chunk=None.
+
+    relu (optional): relu(pre, layer, first) replaces torch.relu in the feed-forward of `layer`, pre (b,N,512) being
+    the pre-activations of instances first .. first + b - 1.  Lets a float64 evaluation follow the ReLU gate of an
+    fp32 computation where a pre-activation lies within rounding of zero."""
     B, N, f = x.shape
     E = sd["encoder.node_embed.weight"].shape[0]
     h = x @ sd["encoder.node_embed.weight"].T + sd["encoder.node_embed.bias"]
@@ -42,23 +50,38 @@ def encoder_forward(sd, x, depot_onehot=None, train=False, num_layers=3):
         hd = x[:, :, :2] @ sd["encoder.depot_embed.weight"].T + sd["encoder.depot_embed.bias"]
         h = torch.where(depot_onehot[:, :, None], hd, h)
     dh = E // H
+
+    def per_chunk(fn, h):
+        if chunk is None or chunk >= B:
+            return fn(h, 0)
+        return torch.cat([fn(h[i:i + chunk], i) for i in range(0, B, chunk)])
+
     for l in range(num_layers):
         p = f"encoder.attention_layers.{l}."
         Wi, bi = sd[p + "attention_layer.in_proj_weight"], sd[p + "attention_layer.in_proj_bias"]
         Wo, bo = sd[p + "attention_layer.out_proj.weight"], sd[p + "attention_layer.out_proj.bias"]
-        qkv = h @ Wi.T + bi  # rows ordered [q;k;v]
-        q, k, v = qkv.split(E, dim=-1)
-        q = q.view(B, N, H, dh).transpose(1, 2)
-        k = k.view(B, N, H, dh).transpose(1, 2)
-        v = v.view(B, N, H, dh).transpose(1, 2)
-        s = (q @ k.transpose(-1, -2)) / math.sqrt(dh)
-        a = torch.softmax(s, dim=-1) @ v  # (B,H,N,dh)
-        a = a.transpose(1, 2).reshape(B, N, E)
-        o = a @ Wo.T + bo
-        h = _bn((h + o).reshape(B * N, E), sd, p + "bn1", train).view(B, N, E)
-        ff = torch.relu(h @ sd[p + "ff.0.weight"].T + sd[p + "ff.0.bias"])
-        ff = ff @ sd[p + "ff.2.weight"].T + sd[p + "ff.2.bias"]
-        h = _bn((h + ff).reshape(B * N, E), sd, p + "bn2", train).view(B, N, E)
+
+        def attention(h, first):
+            b = h.shape[0]
+            qkv = h @ Wi.T + bi  # rows ordered [q;k;v]
+            q, k, v = qkv.split(E, dim=-1)
+            q = q.view(b, N, H, dh).transpose(1, 2)
+            k = k.view(b, N, H, dh).transpose(1, 2)
+            v = v.view(b, N, H, dh).transpose(1, 2)
+            s = (q @ k.transpose(-1, -2)) / math.sqrt(dh)
+            a = torch.softmax(s, dim=-1) @ v  # (b,H,N,dh)
+            a = a.transpose(1, 2).reshape(b, N, E)
+            o = a @ Wo.T + bo
+            return h + o
+
+        def feed_forward(h, first):
+            ff = h @ sd[p + "ff.0.weight"].T + sd[p + "ff.0.bias"]
+            ff = torch.relu(ff) if relu is None else relu(ff, l, first)
+            ff = ff @ sd[p + "ff.2.weight"].T + sd[p + "ff.2.bias"]
+            return h + ff
+
+        h = _bn(per_chunk(attention, h).reshape(B * N, E), sd, p + "bn1", train).view(B, N, E)
+        h = _bn(per_chunk(feed_forward, h).reshape(B * N, E), sd, p + "bn2", train).view(B, N, E)
     return h
 
 

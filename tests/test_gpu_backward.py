@@ -1,7 +1,12 @@
 """GPU parity of the hand-written REINFORCE backward (csrc/decoder_bwd.cu, csrc/encoder_bwd.cu, vrpx/backward.py)
 against (a) torch autograd on the fp32 oracle for dL/dh and the decoder parameters, and (b) the gradients the
 UNMODIFIED reference produced for the same teacher-forced tape (tests/golden/policy_*.npz: per-parameter gradient
-norms and leading elements; train-mode BatchNorm, loss = mean(advantage * log_prob), graph_tsp_agent.py:179-186)."""
+norms and leading elements; train-mode BatchNorm, loss = mean(advantage * log_prob), graph_tsp_agent.py:179-186).
+
+These run at B <= 32 (N 4 ... 20): `k_decoder_bwd` is a single CTA, glimpse-mask partners stay in the instance's own
+tile and the weight gradients stay on the warp-level GEMMs.  The large-batch paths of the same backward (multi-CTA tile
+loop, far partners, coupling groups, `k_gemm_tn_tc`, train-step gradient magnitudes, the C4 shape) are checked against
+float64 in tests/test_gpu_backward_scale.py."""
 import os
 
 import numpy as np

@@ -84,7 +84,9 @@ class GraphEncoder(nn.Module):
         self.attention_layers = nn.ModuleList(
             [MultiHeadAttentionLayer(embedding_dim=embedding_dim, hidden_dim=hidden_dim, num_heads=num_heads)
              for _ in range(num_attention_layers)])
-        self.gemm_path = 0  # 0: tcgen05 f16-split (production), 1: fp32 SIMT cross-check
+        # 0: tcgen05 f16-split (production), 1: fp32 SIMT GEMMs (cross-check); the backward's weight gradients run on
+        # tcgen05 on both paths once B*N >= 8192 rows (vrpx/backward.py)
+        self.gemm_path = 0
 
     def forward(self, x: torch.Tensor) -> torch.Tensor:
         """x (num_graphs, num_nodes, f) -> embeddings (num_graphs, num_nodes, 128), on x's device."""

@@ -89,10 +89,11 @@ def decoder_backward(dec, env, h, roll, wts, gemm_path=0):
                                        int(roll["coupling"]), C.byref(trace), vrpx.ptr(sv["qg"]), vrpx.ptr(wts),
                                        C.byref(gs), vrpx.ptr(ws), nbytes, st))
     # ---- per-episode terms: q~ also contains A_g·g + a_c (every step), A_f·h[first] (steps >= 1), a_q0 (step 0)
-    # the per-episode sums D are gradients too: the two products below that run on the f16-split tensor-core kernels get
-    # them scaled to 2^-2 (see _grad_gain; the sums are final, nothing amplifies them further) and are scaled back
+    # the per-episode sums D are gradients too: the products below run on the f16-split tensor-core kernels (the weight
+    # gradients ag_t / af_t at B >= 8192 on either gemm_path), so they get them scaled to 2^-2 (see _grad_gain; the sums
+    # are final, nothing amplifies them further) and are scaled back
     Dsum = g["D0"] + g["D1"]
-    gs_, g1_ = (_grad_gain(Dsum, -2), _grad_gain(g["D1"], -2)) if gemm_path == 0 else (1.0, 1.0)
+    gs_, g1_ = _grad_gain(Dsum, -2), _grad_gain(g["D1"], -2)
     DsumS = Dsum * gs_ if gs_ != 1.0 else Dsum
     D1S = g["D1"] * g1_ if g1_ != 1.0 else g["D1"]
     G = torch.empty((B, 128), dtype=torch.float32, device=dev)
@@ -146,7 +147,9 @@ def encoder_backward(enc, env, depot, saved, dH, gemm_path=0):
     keep = []
     wt = vrpx.EncoderWeightsT()
     gr = vrpx.EncoderGrads()
-    gain = _grad_gain(dH) if gemm_path == 0 else 1.0     # the fp32 SIMT cross-check path needs no scaling
+    # gemm_path = 1 runs the data-gradient GEMMs and the attention backward in fp32, but the weight gradients go through
+    # the f16-split k_gemm_tn_tc on both paths once B*N >= 8192 rows, so both need the gain
+    gain = _grad_gain(dH)
     if gain != 1.0:
         dH.mul_(gain)
     # the kernels accumulate into a zeroed flat buffer (one view per parameter); it is scaled back and added to .grad below

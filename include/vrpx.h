@@ -200,9 +200,11 @@ VRPX_API int vrpx_encoder_backward(const vrpx_encoder_weights* w, const vrpx_enc
  *   m_c   [128]        W_kp^T · W_ao · (W_o · b_v + b_o) / sqrt(128)
  *   qk_w  [768][128]   optional (may be NULL): rows 0..383 = W_q[:, last block] / sqrt(48) (IRP: W_q · W_ctx), rows
  *                      384..767 = W_k — the rank-48 factors of al_t per head.  With it (and the larger workspace of
- *                      vrpx_rollout_table_workspace_bytes) vrpx_rollout builds, once per episode, the score table
- *                      S1[b][l][head][n] = (A_l h[b,l])_head · h[b,n] and the decode steps t >= 2 read their glimpse
- *                      scores from it instead of recomputing A_l · h[last] and the score pass every step.
+ *                      vrpx_rollout_table_workspace_bytes) a whole-episode vrpx_rollout call builds, once per episode,
+ *                      the score table S1[b][l][head][n] = (A_l h[b,l])_head · h[b,n] and runs every decode step as a
+ *                      few launches over the whole batch; the steps t >= 2 read their glimpse scores from the table
+ *                      instead of recomputing A_l · h[last] and the score pass every step.  Without it, every step
+ *                      runs in the persistent kernel (classic mode).
  * The key bias b_k shifts every score of a head equally and cancels in the softmax. */
 typedef struct vrpx_decoder_weights {
   const float *ag_t, *af_t, *al_t, *a_c, *a_q0, *a_load;
@@ -223,8 +225,9 @@ VRPX_API int64_t vrpx_rollout_workspace_bytes(int64_t B, int32_t N);
 /* Byte offset inside the rollout workspace of the per-episode query table Q~g [B][1024] f32 (read back by the
  * recompute-based backward); the header in front of it holds the barrier/done counters and the pre-split copy of m_t. */
 VRPX_API int64_t vrpx_rollout_workspace_qg_offset(void);
-/* Workspace size that additionally holds the per-episode glimpse score tables (see qk_w above).  A whole-episode call
- * (t_begin == 0, Tmax >= 3) given at least this much workspace and a non-NULL qk_w runs in table mode. */
+/* Workspace size that additionally holds the per-episode glimpse score tables (see qk_w above) and the buffers the
+ * split-step launches hand between them.  A whole-episode call (t_begin == 0, Tmax >= 3) given at least this much
+ * workspace and a non-NULL qk_w runs in table mode; any other call runs the classic loop in the persistent kernel. */
 VRPX_API int64_t vrpx_rollout_table_workspace_bytes(int32_t kind, int64_t B, int32_t N);
 
 /* The rollout loop TSPModel/VRPModel/IRPModel.forward (agents/graph_tsp_agent.py:78-92,
@@ -260,10 +263,11 @@ VRPX_API int vrpx_rollout(const vrpx_env* env, const vrpx_decoder_weights* w, co
  *   vrpx_debug_rollout_kernel_ms  waits for the last bracketed launch and returns its duration (-1 if none) */
 VRPX_API void vrpx_debug_rollout_profile(long long* dev_counters);
 VRPX_API void vrpx_debug_rollout_timing(int32_t enable);
-/* A/B switches of the whole-episode table-mode rollout (default 1):
- *   bit 0  set: every decode step is a handful of launches over the whole batch (rollout_steps.cu);
- *          clear: every step inside the persistent kernel (cross-check and A/B measurements)
- *   bit 1  set: build the score table with the two-kernel form (tcgen05 GEMM + k_score_table) instead of the fused kernel;
+/* A/B switch of the whole-episode rollout (default 1):
+ *   bit 0  set: table mode as described at vrpx_rollout_table_workspace_bytes (score tables, then every decode step is
+ *          a handful of launches over the whole batch, rollout_steps.cu);
+ *          clear: whole-episode calls skip the tables and run the classic loop in the persistent kernel (cross-check
+ *          and A/B measurements)
  *   (programmatic dependent launch of the step kernels was measured and removed: 36.38 vs 36.36 ms per decode loop) */
 VRPX_API void vrpx_debug_rollout_split(int32_t enable);
 VRPX_API float vrpx_debug_rollout_kernel_ms(void);

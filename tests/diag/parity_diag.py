@@ -152,7 +152,7 @@ if __name__ == "__main__":
     if what in ("all", "ckpt"):
         for kind in ("tsp", "vrp"):
             for tag in ("a", "b"):
-                for gp, mode in ((0, "tables_split"), (1, "tables_split"), (0, "classic"), (1, "classic"), (1, "tables_persistent")):
+                for gp, mode in ((0, "tables_split"), (1, "tables_split"), (0, "classic"), (1, "classic")):
                     ckpt_case(kind, tag, gp, mode)
     if what in ("all", "golden"):
         for mode in MODES:
@@ -166,7 +166,6 @@ if __name__ == "__main__":
             for mode in ("tables_split", "classic"):
                 for gp in (0, 1):
                     slice_case(kind, N, B, S, gp, mode)
-        slice_case("tsp", 50, 65536, 256, 0, "tables_persistent")
         slice_case("tsp", 50, 65536, 256, 0, "tables_split", coupling=256)
         slice_case("irp", 40, 4096, 128, 0, "tables_split", seed=7)
         slice_case("irp", 40, 4096, 128, 1, "classic", seed=7)

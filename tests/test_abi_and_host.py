@@ -130,7 +130,7 @@ def test_rollout_workspace_layout_is_consistent():
             table = int(L.vrpx_rollout_table_workspace_bytes(kind, B, N))
             # Q~g [B][1024] f32 right behind the header, then the two glimpse-mask snapshots [2][B][4] u32
             assert plain == off + B * 1024 * 4 + 2 * B * 16
-            # the table workspace also holds S0 (, SL), S1 [B][N][8][N], a QK slice, c [B][1024], q^ [B][128], m_t^T
+            # the table workspace also holds S0 (, SL), S1 [B][N][8][N], c [B][1024], q^ [B][128], m_t^T
             floor = plain + B * 8 * N * 4 + B * N * 8 * N * 4 + B * 1024 * 4 + B * 128 * 4 + 1024 * 128 * 4
             assert table >= floor, (kind, B, N, table, floor)
             assert table % 256 == 0

@@ -1,5 +1,5 @@
 """GPU parity AT THE SIZES THE BENCHMARKS RUN (BASELINE.json configs 3-5): the kernel instantiations behind the
-published numbers (N = 40 / 50 / 100 template paths, table rows staged per step, whole-batch mask coupling G = B =
+published numbers (N = 40 / 50 / 100 template paths, score tables, whole-batch mask coupling G = B =
 65,536 / 131,072) against reference-recorded traces (tests/golden/policy_*_large.npz) and against the oracle.
 
 Tolerances (north_star): logits / embeddings / costs 1e-5 relative with an absolute floor of 1e-5 for magnitudes
@@ -14,8 +14,9 @@ import torch
 pytestmark = pytest.mark.gpu
 
 LARGE_CASES = [(40, 8, 30), (50, 8, 31), (100, 8, 32)]
-# decode-loop variants: (score_tables, split-step launches)
-MODES = {"tables_split": (True, 1), "tables_persistent": (True, 0), "classic": (False, 1)}
+# decode-loop variants: (decoder.score_tables, vrpx_debug_rollout_split).  "split_off" allocates the table workspace but
+# clears the switch, so the call skips the tables and runs the classic loop in the persistent kernel (bench.py --no-split)
+MODES = {"tables_split": (True, 1), "split_off": (True, 0), "classic": (False, 1)}
 
 
 def _cls(kind):
@@ -39,7 +40,8 @@ def _large(golden_dir, kind):
 def test_reference_logits_embeddings_at_benchmark_node_counts(golden_dir, kind, gemm_path, mode):
     """Replay the reference's greedy tape at N = 40 / 50 / 100: every masked pointer logit of every step, ALL embeddings
     and the costs match the unmodified reference to 1e-5 — for the production decode loop (score tables + split-step
-    launches), the all-persistent table loop and the classic loop, on the tcgen05 and the SIMT GEMM paths."""
+    launches) and the classic loop in the persistent kernel, chosen by decoder.score_tables or by the debug switch with
+    the table workspace in place, on the tcgen05 and the SIMT GEMM paths."""
     import vrpx
 
     z = _large(golden_dir, kind)

@@ -1,5 +1,6 @@
 """Per-phase cycle breakdown of the persistent rollout kernel (debug counters, thread 0 of every CTA).
-The split-step launches are switched off so that every decode step runs inside the persistent kernel."""
+The split-step launches are switched off, so the whole episode runs the classic loop (no score tables) inside the
+persistent kernel."""
 import ctypes as C
 import os
 import sys

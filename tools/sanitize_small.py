@@ -47,12 +47,10 @@ for Env, Agent, N, B in ((TSPEnv, TSPAgent, 12, 40), (VRPEnv, VRPAgent, 9, 24), 
     a = np.array([np.flatnonzero(mask[b] == 0)[0] for b in range(B)])
     env.step(a[:, None])
     agent = Agent(seed=3)
-    for tables, split in ((True, 1), (True, 0), (False, 1)):
+    for tables in (True, False):
         agent.model.decoder.score_tables = tables
-        L.vrpx_debug_rollout_split(split)
         env.reset()
         loss = agent.evaluate(env)
-    L.vrpx_debug_rollout_split(1)
     agent.model.decoder.score_tables = True
     agent.model.train()
     loss_m, loss_b, logp = agent.step(env, (False, True))

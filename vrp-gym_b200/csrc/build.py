@@ -13,7 +13,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 OUT = os.path.join(os.path.dirname(HERE), "vrpx", "libvrpx.so")
-SOURCES = ["env.cu", "mt19937_legacy.cu", "encoder.cu", "gemm_tc4.cu", "gemm_tn_tc.cu", "ff_fused.cu", "attn_fused.cu", "rollout.cu", "rollout_steps.cu", "score_table.cu", "score_table_fused.cu", "decoder_bwd.cu", "encoder_bwd.cu", "attention_bwd.cu"]
+SOURCES = ["env.cu", "mt19937_legacy.cu", "encoder.cu", "gemm_tc4.cu", "gemm_tn_tc.cu", "ff_fused.cu", "attn_fused.cu", "rollout.cu", "rollout_steps.cu", "score_table_fused.cu", "decoder_bwd.cu", "encoder_bwd.cu", "attention_bwd.cu"]
 HEADERS = ["common.cuh", "tc_common.cuh", "f16split.cuh", "env_rules.cuh", "gemm.cuh", "tile_gemm.cuh", "glimpse_mma.cuh", "rollout.cuh", os.path.join(ROOT, "include", "vrpx.h")]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = [

@@ -20,8 +20,6 @@
 namespace vrpx {
 
 
-int64_t score_table_slice(int64_t B);
-int build_score_table(const float* h, const float* qk_w, int64_t B, int N, float* qk_buf, float* s1, cudaStream_t stream);
 int build_score_table_fused(const float* h, const float* qk_w, int64_t B, int N, __half* w16, float* s1, cudaStream_t stream);
 
 // Rollout tile: RMT x 16 instances.  With 16 instances per tile the working set that has to survive in L2 between the
@@ -49,7 +47,6 @@ __global__ void __launch_bounds__(NT, 1) k_rollout(const RolloutParams p) {
   float* Xs = reinterpret_cast<float*>(smem_raw);
   float* QC = reinterpret_cast<float*>(smem_raw + SMEM_X_MMA);
   float* Wb = reinterpret_cast<float*>(smem_raw + SMEM_X_MMA + SMEM_QC_MMA);
-  float* TB = reinterpret_cast<float*>(smem_raw + SMEM_TOTAL);   // [RTM][tb_segs][8 N] staged table rows (table mode)
   __shared__ float s_loadf[RTM], s_lp[RTM];
   __shared__ int s_anyleft, s_act[RTM];
 
@@ -109,33 +106,6 @@ __global__ void __launch_bounds__(NT, 1) k_rollout(const RolloutParams p) {
     grid_barrier(p.bar, bar_target);
   }
 
-  // Table mode: the rows S1[b][last], S0[b] (, SL[b]) the NEXT tile will need are copied to shared memory with cp.async
-  // while the current tile runs its pointer-logit phase, so the dependent chain cur -> table row -> softmax does not
-  // sit exposed at the head of every tile.  One warp per instance, issued and consumed by the same warp.
-  const int tb_row = NH * N;                    // floats per staged segment
-  const int tb_stride = p.tb_segs * tb_row;     // floats per instance
-  bool staged = false;                          // TB holds the rows of the tile about to be processed
-  auto stage_tables = [&](int64_t ntile) {
-    const int64_t nbase = ntile * RTM;
-    const int ncnt = (int)((B - nbase < RTM) ? (B - nbase) : RTM);
-    for (int m = warp; m < ncnt; m += NT / 32) {
-      const int64_t b = nbase + m;
-      const int last = __ldcg(p.env.cur + b);
-      float* dst = TB + m * tb_stride;
-      const float* src1 = p.s1 + (((size_t)b * N + last) * NH) * N;
-      for (int i = lane; i < tb_row / 4; i += 32) cp_async16(dst + 4 * i, src1 + 4 * i);
-      if (p.tb_segs >= 2) {
-        const float* src0 = p.s0 + (size_t)b * tb_row;
-        for (int i = lane; i < tb_row / 4; i += 32) cp_async16(dst + tb_row + 4 * i, src0 + 4 * i);
-      }
-      if (p.tb_segs >= 3) {
-        const float* srcl = p.sl + (size_t)b * tb_row;
-        for (int i = lane; i < tb_row / 4; i += 32) cp_async16(dst + 2 * tb_row + 4 * i, srcl + 4 * i);
-      }
-    }
-    cp_async_commit();
-  };
-
   int t = p.t0;
   for (; t < p.t0 + p.Tmax; ++t) {
     const int trel = t - p.t0;
@@ -146,19 +116,16 @@ __global__ void __launch_bounds__(NT, 1) k_rollout(const RolloutParams p) {
       const int64_t base = tile * RTM;
       const int cnt = (int)((B - base < RTM) ? (B - base) : RTM);
       if (tid == 0) s_anyleft = 0;
-      // table mode: from step 2 on the glimpse scores come from the per-episode tables (no GEMM-A, no score pass)
-      const bool tbl_step = p.s1 != nullptr && t >= 2;
       // ---------------- P0: gather last-node embeddings, vehicle load; pull this tile's Q~g rows towards L2
-      if (!tbl_step)
-        for (int i = tid; i < cnt * 32; i += NT)
-          asm volatile("prefetch.global.L2 [%0];" ::"l"(reinterpret_cast<const char*>(p.qg + base * QW) + (size_t)i * 128));
+      for (int i = tid; i < cnt * 32; i += NT)
+        asm volatile("prefetch.global.L2 [%0];" ::"l"(reinterpret_cast<const char*>(p.qg + base * QW) + (size_t)i * 128));
       for (int m = warp; m < RTM; m += NT / 32) {
         float4 xv = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (m < cnt && t > 0 && !tbl_step) {
+        if (m < cnt && t > 0) {
           int last = p.env.cur[base + m];
           xv = __ldg(reinterpret_cast<const float4*>(h + ((base + m) * N + last) * E) + lane);
         }
-        if (!tbl_step) *reinterpret_cast<float4*>(Xs + m * XS_LD + lane * 4) = xv;
+        *reinterpret_cast<float4*>(Xs + m * XS_LD + lane * 4) = xv;
         const float lf = (m < cnt) ? (float)p.env.load[base + m] : 0.f;
         if (lane == 0) s_loadf[m] = lf;
         if (m < cnt && p.mask_hist && lane < 4)
@@ -229,9 +196,7 @@ __global__ void __launch_bounds__(NT, 1) k_rollout(const RolloutParams p) {
         }
       };
       // ---------------- P1: q~
-      if (tbl_step) {
-        // nothing: scores are gathered from S1/S0 in P2
-      } else if (t == 0) {
+      if (t == 0) {
         for (int o = tid; o < cnt * QW; o += NT) {
           int m = o >> 10, c = o & (QW - 1);
           float y = p.qg[(base + m) * QW + c] + p.w.a_q0[c];
@@ -248,30 +213,6 @@ __global__ void __launch_bounds__(NT, 1) k_rollout(const RolloutParams p) {
               [&](int m, int c, float v0, float v1) {
                 if (m < cnt) *reinterpret_cast<float2*>(p.qg + (base + m) * QW + c) = make_float2(v0, v1);
               });
-        }
-        if (t == 1 && p.s1) {
-          // table mode: Q~g is final now -> S0[b][head][n] = Q~g[b]_head · h[b,n]  (IRP: SL from a_load as well)
-          __syncthreads();
-          for (int m = warp; m < cnt; m += NT / 32) {
-            const int64_t b = base + m;
-            float* slot = QC + m * RQ_LD;
-            const float4* hrow = reinterpret_cast<const float4*>(h + b * N * E);
-            const int tq = lane & 3;
-            for (int i = lane; i < QW / 4; i += 32)
-              *reinterpret_cast<float4*>(slot + 4 * i) = __ldcg(reinterpret_cast<const float4*>(p.qg + b * QW) + i);
-            __syncwarp();
-            float* s0 = p.s0 + (size_t)b * NH * N;
-            glimpse_scores(slot, hrow, [&](int n, int which, float v) { s0[(2 * tq + which) * N + n] = v; });
-            if (kind == VRPX_IRP) {
-              __syncwarp();
-              for (int i = lane; i < QW / 4; i += 32)
-                *reinterpret_cast<float4*>(slot + 4 * i) = __ldg(reinterpret_cast<const float4*>(p.w.a_load) + i);
-              __syncwarp();
-              float* sl = p.sl + (size_t)b * NH * N;
-              glimpse_scores(slot, hrow, [&](int n, int which, float v) { sl[(2 * tq + which) * N + n] = v; });
-            }
-          }
-          __syncthreads();
         }
         tile_gemm_wide_mma_sw<RMT, RNST>(                                          // q~ = Q~g (+ load · a_load) + A_l · h[last]
             Xs, XS_LD, p.w.al_t, Wb,
@@ -296,64 +237,29 @@ __global__ void __launch_bounds__(NT, 1) k_rollout(const RolloutParams p) {
         float* slot = QC + m * RQ_LD;
         const int g = lane >> 2, t = lane & 3;
         const float4* hrow = reinterpret_cast<const float4*>(h + b * N * E);
-        float pr[NH][4];
-        if (!tbl_step) {
-          // ---- pass 1: scores = q~_h · h_n + scrambled additive mask
-          // masks of the instances whose rows the reference adds to heads 2t and 2t+1 (mask.repeat(H,1), graph_decoder.py:93)
-          uint32_t nb0[4], nb1[4];
-          {
-            const uint32_t* m0 = gm_rd + quirk_row(b, 2 * t, p.G) * 4;
-            const uint32_t* m1 = gm_rd + quirk_row(b, 2 * t + 1, p.G) * 4;
+        // ---- pass 1: scores = q~_h · h_n + scrambled additive mask
+        // masks of the instances whose rows the reference adds to heads 2t and 2t+1 (mask.repeat(H,1), graph_decoder.py:93)
+        uint32_t nb0[4], nb1[4];
+        {
+          const uint32_t* m0 = gm_rd + quirk_row(b, 2 * t, p.G) * 4;
+          const uint32_t* m1 = gm_rd + quirk_row(b, 2 * t + 1, p.G) * 4;
 #pragma unroll
-            for (int i = 0; i < 4; ++i) { nb0[i] = __ldcg(m0 + i); nb1[i] = __ldcg(m1 + i); }
-          }
-          glimpse_scores(slot, hrow, [&](int n, int which, float v) {
-            const uint32_t wsel = which ? nb1[n >> 5] : nb0[n >> 5];
-            slot[(2 * t + which) * E + n] = v + (float)((wsel >> (n & 31)) & 1u);
-          });
-          __syncwarp();
-          VRPX_PROF(6)
-#pragma unroll
-          for (int hh = 0; hh < NH; ++hh)
-#pragma unroll
-            for (int i = 0; i < 4; ++i) {
-              const int n = lane + 32 * i;
-              pr[hh][i] = (n < N) ? slot[hh * E + n] : -INFINITY;
-            }
-        } else {
-          // ---- table mode: scores = S1[b][last] + S0[b] (+ load · SL[b]) + scrambled additive mask
-          const float* r1;
-          const float* r0 = p.s0 + (size_t)b * NH * N;
-          const float* rl = p.sl + (size_t)b * NH * N;
-          if (staged) {
-            cp_async_wait<0>();
-            __syncwarp();
-            r1 = TB + m * tb_stride;
-            if (p.tb_segs >= 2) r0 = r1 + tb_row;
-            if (p.tb_segs >= 3) rl = r1 + 2 * tb_row;
-          } else {
-            const int last = __ldcg(p.env.cur + b);
-            r1 = p.s1 + (((size_t)b * N + last) * NH) * N;
-          }
-          const float lf = s_loadf[m];
-          // lane j holds mask word (j & 3) of the instance whose mask the reference adds to head j >> 2
-          const uint32_t mword = __ldcg(gm_rd + quirk_row(b, lane >> 2, p.G) * 4 + (lane & 3));
-#pragma unroll
-          for (int hh = 0; hh < NH; ++hh)
-#pragma unroll
-            for (int i = 0; i < 4; ++i) {
-              const int n = lane + 32 * i;
-              const uint32_t wsel = __shfl_sync(0xffffffffu, mword, hh * 4 + i);
-              float v = -INFINITY;
-              if (n < N) {
-                v = r1[hh * N + n] + r0[hh * N + n];   // generic loads: shared (staged) or global (L2-coherent data)
-                if (kind == VRPX_IRP) v = fmaf(lf, rl[hh * N + n], v);
-                v += (float)((wsel >> lane) & 1u);
-              }
-              pr[hh][i] = v;
-            }
-          VRPX_PROF(6)
+          for (int i = 0; i < 4; ++i) { nb0[i] = __ldcg(m0 + i); nb1[i] = __ldcg(m1 + i); }
         }
+        glimpse_scores(slot, hrow, [&](int n, int which, float v) {
+          const uint32_t wsel = which ? nb1[n >> 5] : nb0[n >> 5];
+          slot[(2 * t + which) * E + n] = v + (float)((wsel >> (n & 31)) & 1u);
+        });
+        __syncwarp();
+        VRPX_PROF(6)
+        float pr[NH][4];
+#pragma unroll
+        for (int hh = 0; hh < NH; ++hh)
+#pragma unroll
+          for (int i = 0; i < 4; ++i) {
+            const int n = lane + 32 * i;
+            pr[hh][i] = (n < N) ? slot[hh * E + n] : -INFINITY;
+          }
         // softmax per head over nodes (lane = node, 4 strides cover N <= 128)
 #pragma unroll
         for (int hh = 0; hh < NH; ++hh) {
@@ -443,19 +349,6 @@ __global__ void __launch_bounds__(NT, 1) k_rollout(const RolloutParams p) {
 
       // ---------------- P3: q^ = C · M^T + m_c  -> Xs
       tile_gemm_tall_f16<RNST>(reinterpret_cast<const uint2*>(QC), p.m16, Wb, p.w.m_c, QC, Xs, XS_LD);
-
-      // table mode: start copying the next tile's table rows (its `cur` is final: written one step ago, or — when the
-      // next tile is this CTA's first tile of the NEXT step — earlier in this step)
-      staged = false;
-      if (p.s1 && p.tb_segs > 0) {
-        int64_t ntile = tile + gridDim.x;
-        int tn = t;
-        if (ntile >= ntiles) { ntile = blockIdx.x; tn = t + 1; }
-        if (tn >= 2 && ntile != tile) {
-          stage_tables(ntile);
-          staged = true;
-        }
-      }
       VRPX_PROF(3)
       // ---------------- P4: logits, action, environment transition
       bool unfinished = false;
@@ -606,7 +499,6 @@ __global__ void __launch_bounds__(NT, 1) k_rollout(const RolloutParams p) {
     VRPX_PROF(5)
     if (ld_acquire_i(p.notdone + trel) == 0) { ++t; break; }
   }
-  cp_async_wait<0>();
   if (p.prof && tid == 0)
     for (int i = 0; i < 8; ++i) atomicAdd(reinterpret_cast<unsigned long long*>(p.prof) + i, (unsigned long long)prof_acc[i]);
   if (blockIdx.x == 0 && tid == 0) *p.steps = t;
@@ -614,7 +506,6 @@ __global__ void __launch_bounds__(NT, 1) k_rollout(const RolloutParams p) {
 
 static long long* g_rollout_prof = nullptr;
 static int g_split_steps = 1;                        // vrpx_debug_rollout_split (bit 0)
-static int g_fused_tables = 1;                       // vrpx_debug_rollout_split (bit 1 clear = fused score-table kernel)
 static int g_time_kernel = 0;                        // vrpx_debug_rollout_timing
 static cudaEvent_t g_ev0 = nullptr, g_ev1 = nullptr;
 static bool g_ev_valid = false;
@@ -631,10 +522,7 @@ extern "C" {
 /* Debug hook: device buffer of 8 x int64 that accumulates per-phase cycles of thread 0 of every CTA (NULL disables). */
 void vrpx_debug_rollout_profile(long long* dev_counters) { g_rollout_prof = dev_counters; }
 
-void vrpx_debug_rollout_split(int32_t enable) {
-  g_split_steps = enable & 1;
-  g_fused_tables = (enable & 2) ? 0 : 1;   // bit 1: build the score table with the two-kernel form (A/B measurements)
-}
+void vrpx_debug_rollout_split(int32_t enable) { g_split_steps = enable & 1; }
 
 void vrpx_debug_rollout_timing(int32_t enable) {
   g_time_kernel = enable;
@@ -657,10 +545,11 @@ int64_t vrpx_rollout_workspace_bytes(int64_t B, int32_t N) {
 
 int64_t vrpx_rollout_workspace_qg_offset(void) { return kRolloutHdr; }
 
-// table-mode workspace: header | Q~g | gmask | S0 | SL (IRP) | S1 | QK slice | c | q^ | m_t^T, every segment 256-byte aligned
+// table-mode workspace: header | Q~g | gmask | S0 | SL (IRP) | S1 | c | q^ | transposed and split weights, every segment
+// 256-byte aligned
 namespace {
 struct TableLayout {
-  int64_t s0, sl, s1, qk, cbuf, qhat, mnt, agn, afn, w16b, qkw16, total;
+  int64_t s0, sl, s1, cbuf, qhat, mnt, agn, afn, w16b, qkw16, total;
 };
 inline int64_t align256(int64_t x) { return (x + 255) & ~(int64_t)255; }
 TableLayout table_layout(int kind, int64_t B, int N) {
@@ -669,9 +558,8 @@ TableLayout table_layout(int kind, int64_t B, int N) {
   L.s0 = align256(vrpx_rollout_workspace_bytes(B, N));
   L.sl = align256(L.s0 + B * NH * N * f);
   L.s1 = (kind == VRPX_IRP) ? align256(L.sl + B * NH * N * f) : L.sl;
-  L.qk = align256(L.s1 + B * N * NH * N * f);
   // split-step mode (rollout_steps.cu): glimpse vectors, folded queries, transposed m_t
-  L.cbuf = align256(L.qk + score_table_slice(B) * N * 768 * f);
+  L.cbuf = align256(L.s1 + B * N * NH * N * f);
   L.qhat = align256(L.cbuf + B * QW * f);
   L.mnt = align256(L.qhat + B * E * f);
   L.agn = align256(L.mnt + (int64_t)QW * E * f);
@@ -736,19 +624,18 @@ int vrpx_rollout(const vrpx_env* env, const vrpx_decoder_weights* w, const float
   p.s0 = p.sl = nullptr;
   p.cbuf = p.qhat = nullptr;
   SplitWorkspace sw{nullptr, nullptr, nullptr, nullptr};
-  // table mode: whole-episode call with the large workspace and the rank-48 factors
-  if (w->qk_w && t_begin == 0 && Tmax >= 3) {
+  // Split-step form (default for whole-episode calls with the large workspace and the rank-48 factors): per-episode score
+  // tables, then every step is a handful of launches over the whole batch (rollout_steps.cu).  The persistent kernel
+  // below serves the classic mode, resumed single-step calls and vrpx_debug_rollout_split(0).
+  if (g_split_steps && w->qk_w && t_begin == 0 && Tmax >= 3) {
     const TableLayout L = table_layout(env->kind, env->B, env->N);
-    if (ws_bytes >= L.total && (reinterpret_cast<uintptr_t>(ws) & 15) == 0) {
+    if (ws_bytes >= L.total) {
       char* base = reinterpret_cast<char*>(ws);
       float* s1 = reinterpret_cast<float*>(base + L.s1);
       int rc;
       {
         NvtxRange nvtx_tables("vrpx:score_tables");
-        if (g_fused_tables)   // projection + table in one kernel (score_table_fused.cu); the two-kernel form is the A/B switch
-          rc = build_score_table_fused(h, w->qk_w, env->B, env->N, reinterpret_cast<__half*>(base + L.qkw16), s1, stream);
-        else
-          rc = build_score_table(h, w->qk_w, env->B, env->N, reinterpret_cast<float*>(base + L.qk), s1, stream);
+        rc = build_score_table_fused(h, w->qk_w, env->B, env->N, reinterpret_cast<__half*>(base + L.qkw16), s1, stream);
       }
       if (rc) return rc;
       p.s1 = s1;
@@ -762,24 +649,11 @@ int vrpx_rollout(const vrpx_env* env, const vrpx_decoder_weights* w, const float
       sw.w16b = reinterpret_cast<__half*>(base + L.w16b);
     }
   }
-  // Split-step mode (default for whole-episode table-mode calls): every step is a handful of launches over the whole
-  // batch (rollout_steps.cu); the persistent kernel below serves the classic mode, resumed single-step calls and the
-  // all-persistent A/B switch
-  const bool split = p.s1 != nullptr && g_split_steps;
+  const bool split = p.s1 != nullptr;
   GemmPlan plan_b;
   if (split) {
     int rc = prepare_split_weights(p, sw, &plan_b, stream);
     if (rc) return rc;
-  }
-  // shared-memory staging of the table rows: as many segments as fit beside the GEMM buffers
-  p.tb_segs = 0;
-  size_t smem_total = SMEM_TOTAL;
-  if (p.s1) {
-    const size_t avail = 227 * 1024 - SMEM_TOTAL - 1024;   // 1 KiB for the static __shared__ arrays
-    const size_t seg = (size_t)RTM * NH * env->N * sizeof(float);
-    const int want = (env->kind == VRPX_IRP) ? 3 : 2;
-    p.tb_segs = (int)((avail / seg < (size_t)want) ? avail / seg : (size_t)want);
-    smem_total += p.tb_segs * seg;
   }
   VRPX_CHECK_ARG((int64_t)(Tmax + 1 + 8) * 4 <= kRolloutSmall, "Tmax too large for workspace header");
 
@@ -804,7 +678,7 @@ int vrpx_rollout(const vrpx_env* env, const vrpx_decoder_weights* w, const float
   }
   k_split_m16<<<(QW / 2) * E / 256, 256, 0, stream>>>(w->m_t, reinterpret_cast<uint2*>(reinterpret_cast<char*>(ws) + kRolloutSmall));
   VRPX_LAUNCH_CHECK();
-  VRPX_CUDA(cudaFuncSetAttribute(k_rollout, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_total));
+  VRPX_CUDA(cudaFuncSetAttribute(k_rollout, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_TOTAL));
   int64_t ntiles = (env->B + RTM - 1) / RTM;
   int grid = (int)((ntiles < (int64_t)num_sms()) ? ntiles : (int64_t)num_sms());
   void* args[] = {(void*)&p};
@@ -816,7 +690,7 @@ int vrpx_rollout(const vrpx_env* env, const vrpx_decoder_weights* w, const float
     VRPX_CUDA(cudaEventRecord(g_ev0, stream));
   }
   NvtxRange nvtx_decode("vrpx:decode_loop");
-  VRPX_CUDA(cudaLaunchCooperativeKernel((void*)k_rollout, dim3(grid), dim3(NT), args, smem_total, stream));
+  VRPX_CUDA(cudaLaunchCooperativeKernel((void*)k_rollout, dim3(grid), dim3(NT), args, SMEM_TOTAL, stream));
   count_launch();
   if (g_time_kernel) {
     VRPX_CUDA(cudaEventRecord(g_ev1, stream));

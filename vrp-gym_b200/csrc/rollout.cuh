@@ -30,15 +30,15 @@ struct RolloutParams {
   unsigned* bar;      // grid barrier counter
   int* notdone;       // [Tmax + 1]
   long long* prof;    // optional [8] cycle counters per phase (debug, vrpx_debug_rollout_profile)
-  // table mode (score_table.cu): per-episode glimpse score tables, all NULL in the classic mode
-  const float* s1;    // [B][N][8][N]  (A_l h[b,l])_head · h[b,n], built before the launch
+  // split-step mode: per-episode glimpse score tables (S1 from score_table_fused.cu before the first step, S0 / SL
+  // written at step 1 by rollout_steps.cu), all NULL in the persistent kernel
+  const float* s1;    // [B][N][8][N]  (A_l h[b,l])_head · h[b,n]
   float* s0;          // [B][8][N]     Q~g[b]_head · h[b,n], built at step 1 (after the `first` fold)
   float* sl;          // [B][8][N]     IRP: a_load_head · h[b,n]
   const uint2* m16;   // [512][128] m_t pre-split for the fp16 tensor path (k_split_m16, tile_gemm.cuh)
   // split-step mode (rollout_steps.cu): glimpse vectors c [B][1024] and folded queries q^ [B][128] in global memory
   float* cbuf;
   float* qhat;
-  int tb_segs;        // table rows staged in shared memory per instance: 0 none, 1 = S1, 2 = S1 + S0, 3 = S1 + S0 + SL
 };
 
 // rollout_steps.cu: a whole-episode table-mode rollout as launches over the whole batch — steps 0 and 1 (run_first_steps:

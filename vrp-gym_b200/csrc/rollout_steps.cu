@@ -11,8 +11,9 @@
 //                    once per 128 instances instead of once per 16
 //   k_step_pointer   one warp per instance: logits 10 tanh(q^ · h_n), mask, argmax / Philox sample / teacher action,
 //                    log-prob; then one thread per instance runs the environment transition (env_rules.cuh)
-// Same arithmetic as phases P2 and P4 of the persistent kernel (the code is carried over); the results differ only by
-// the summation order inside GEMM-B.  Steps 0 and 1 (and the classic mode, resumed calls) stay in the persistent kernel.
+// Softmax, glimpse values and pointer phase are those of phases P2 and P4 of the persistent kernel (the code is carried
+// over); against its classic loop the results differ only by the evaluation order of the scores (tables) and the
+// summation order inside GEMM-B.  The classic mode and resumed single-step calls run in the persistent kernel.
 // The launches are asynchronous on the caller's stream: no host round trip per step.  An episode that finishes early
 // (VRP / IRP) turns the remaining launches into no-ops through the per-step `notdone` counters.
 #include "gemm.cuh"

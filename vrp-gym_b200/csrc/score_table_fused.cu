@@ -1,9 +1,19 @@
-// score_table_fused.cu — the per-episode glimpse score table in ONE kernel: projection on tcgen05, table on mma.sync.
+// score_table_fused.cu — the per-episode glimpse score table of the split-step rollout (table mode of vrpx_rollout) in
+// ONE kernel: projection on tcgen05, table on mma.sync.
 //
-//     S1[b][l][head][n] = q'[b,l,head,:] · k'[b,n,head,:],   q' = h · (W_l / sqrt(48))^T,  k' = h · W_k^T     (score_table.cu)
+// The decoder's glimpse scores at step t >= 1 are  s[b,head,n] = q~[b,head] · h[b,n]  with
+// q~ = A_l · h[b,last] + Q~g[b]  (agents/graph_decoder.py:75-94 after the folding of vrpx/packing.py).  The part that
+// depends on the step, (A_l h[b,l])_head · h[b,n], takes only N different values of l per instance, and A_l has rank 48
+// per head (A_l,head = W_k,head^T · W_l,head / sqrt(48), the reference's own query/key projections).  So once per
+// episode
 //
-// The two-kernel form (a (B·N) x 768 tcgen05 GEMM that writes q' | k' to HBM, then k_score_table that reads them back)
-// moves 10 GB each way at C4 for 1.7 GB of embeddings in and 5.2 GB of table out.  Here q' and k' never leave the SM:
+//     S1[b][l][head][n] = q'[b,l,head,:] · k'[b,n,head,:],   q' = h · (W_l / sqrt(48))^T,  k' = h · W_k^T
+//
+// and the decode steps read the 8·N scores of row (b, last) instead of running the 128 -> 1024 query GEMM and the
+// 8·N·128 score pass every step.  Algorithmic cost: the table holds B·N·8·N floats (5.2 GB at TSP-50, B = 65536).
+//
+// Writing q' | k' ((B·N) x 768) to HBM and reading them back would move 10 GB each way at C4 for 1.7 GB of embeddings in
+// and 5.2 GB of table out.  Here q' and k' never leave the SM:
 //   * a tile = TI = floor(128 / N) whole instances (TI·N <= 128 rows of h), so that a tile's projection holds everything the
 //     table rows of its instances need;
 //   * CTAs are SPECIALISED by head pair: CTA type g = blockIdx % 4 keeps the 96 KiB of split weights of heads 2g, 2g+1
@@ -11,7 +21,8 @@
 //     would need > 10 TB/s from L2).  The four types of a tile run side by side, so h comes from DRAM once;
 //   * per (tile, head): D[128 x 96] = XA · W_head^T on tcgen05 (A = the tile as f16 hi/lo in tensor memory, cross terms
 //     first, gemm_tc4.cu), then the epilogue warps move D to shared memory — q' rows as fp32, k' rows already split and in
-//     mma.sync fragment order — and compute the table rows of the tile's instances with the inner loop of k_score_table.
+//     mma.sync fragment order — and compute the table rows of the tile's instances on mma.sync.m16n8k16 with f16 hi/lo
+//     halves (f16split.cuh, unscaled lo: q' and k' are O(1) projections), ~fp32 accuracy.
 // Roles (16 warps): 0-3 X converters (raw fp32 smem tile -> XA in TMEM), 4 TMA producer, 5 MMA issuer (whole warp,
 // elected lane), 8-15 epilogue + table (8 warps: two per TMEM lane quarter; table tasks = instance x 16-row query tile).
 // TMEM: XA 128 columns | D 2 x 128 (96 used).  Shared memory: weights 96 KiB | raw X 64 KiB | q' 26 KiB | k' fragments 37.5 KiB.
@@ -230,8 +241,9 @@ k_score_table_fused(const __grid_constant__ CUtensorMap mapX, const __grid_const
                   make_float4(__uint_as_float(v[4 * c]) * OUT_SCALE, __uint_as_float(v[4 * c + 1]) * OUT_SCALE,
                               __uint_as_float(v[4 * c + 2]) * OUT_SCALE, __uint_as_float(v[4 * c + 3]) * OUT_SCALE);
           } else {
-            // key n of instance i -> fragment order of k_score_table: [key][k16 step c][slot tt] =
-            // {hi(dims 16c+2tt, +1), hi(dims 16c+2tt+8, +9), lo(..), lo(..)}
+            // key n of instance i -> B-fragment order of the table loop below, 16 B per [key][k16 step c][slot tt] =
+            // {hi(dims 16c+2tt, +1), hi(dims 16c+2tt+8, +9), lo(..), lo(..)}: one conflict-free LDS.128 per B fragment,
+            // the hi / lo pairs adjacent as the two-register HMMA operand
             const int i = r / N, n = r - i * N;
             uint4* dst = Kf + (size_t)(i * KP + n) * 12;
 #pragma unroll

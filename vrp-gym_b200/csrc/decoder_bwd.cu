@@ -164,39 +164,16 @@ __global__ void __launch_bounds__(NT, 1) k_decoder_bwd(const DecBwdParams p) {
         float pr[NH][4];
 #pragma unroll
         for (int hh = 0; hh < NH; ++hh) {
-          float mx = -INFINITY;
 #pragma unroll
           for (int i = 0; i < 4; ++i) {
-            int n = lane + 32 * i;
+            const int n = lane + 32 * i;
             pr[hh][i] = (n < N) ? slot[hh * E + n] : -INFINITY;
-            mx = fmaxf(mx, pr[hh][i]);
           }
-          mx = warp_max(mx);
-          float sum = 0.f;
-#pragma unroll
-          for (int i = 0; i < 4; ++i) {
-            int n = lane + 32 * i;
-            pr[hh][i] = (n < N) ? expf(pr[hh][i] - mx) : 0.f;
-            sum += pr[hh][i];
-          }
-          sum = warp_sum(sum);
-          float inv = 1.0f / sum;
-#pragma unroll
-          for (int i = 0; i < 4; ++i) pr[hh][i] *= inv;
+          warp_node_softmax(pr[hh], N);
         }
         __syncwarp();
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-          int n = lane + 32 * i;
-          if (n < N) {
-            const float4 a0 = make_float4(pr[0][i], pr[1][i], pr[2][i], pr[3][i]);
-            const float4 a1 = make_float4(pr[4][i], pr[5][i], pr[6][i], pr[7][i]);
-            *reinterpret_cast<float4*>(slot + n * 8) = a0;
-            *reinterpret_cast<float4*>(slot + n * 8 + 4) = a1;
-            *reinterpret_cast<float4*>(sc_p + n * 8) = a0;
-            *reinterpret_cast<float4*>(sc_p + n * 8 + 4) = a1;
-          }
-        }
+        warp_store_by_node(slot, pr, N, lane);
+        warp_store_by_node(sc_p, pr, N, lane);
         __syncwarp();
         warp_glimpse_values(slot, hrow, N, lane);   // c[head][dim] = sum_n p_hn h_n -> slot
       }
@@ -379,14 +356,7 @@ __global__ void __launch_bounds__(NT, 1) k_decoder_bwd(const DecBwdParams p) {
             }
           }
           __syncwarp();
-#pragma unroll
-          for (int i = 0; i < 4; ++i) {
-            int n = lane + 32 * i;
-            if (n < N) {
-              *reinterpret_cast<float4*>(slot + n * 8) = make_float4(ds[0][i], ds[1][i], ds[2][i], ds[3][i]);
-              *reinterpret_cast<float4*>(slot + n * 8 + 4) = make_float4(ds[4][i], ds[5][i], ds[6][i], ds[7][i]);
-            }
-          }
+          warp_store_by_node(slot, ds, N, lane);
           __syncwarp();
           // pass Y: dH[b,n] += sum_h (p_hn dc_h + ds_hn q~_h) + dz_n q^     (one RMW of dH per node and step)
           {

@@ -1,5 +1,5 @@
 // env_rules.cuh — the per-instance environment transition, shared by the API-mode step kernel
-// (env.cu) and the fused persistent rollout kernel (rollout.cu) so both run identical rules.
+// (env.cu) and the decode loops of the rollout (rollout_env_step, rollout.cuh) so both run identical rules.
 //
 // Reference semantics (SURVEY App. A.1):
 //   step:  visited[a]=1 (tsp.py:86); r = -||xy[cur]-xy[a]|| (tsp.py:98, vrp_graph.py:137-146);

@@ -12,9 +12,12 @@
 //       log-prob, then the environment transition (env_rules.cuh) in f64
 // followed by a grid-wide barrier: the reference's glimpse mask of instance b reads the masks of
 // instances (8b+h) mod G (SURVEY App. B-3), so all instances advance in lock-step.
+// The per-instance work of P2 and P4 is done by the helpers of glimpse_mma.cuh and rollout.cuh, which the split-step
+// kernels (rollout_steps.cu) call as well.
 //
 // Step-invariant work the reference repeats every step (K/V/kp projections, graph mean) is folded into
 // host-packed weights (vrpx/packing.py) and the per-episode Q~g table built in the prologue.
+#include "glimpse_mma.cuh"
 #include "rollout.cuh"
 
 namespace vrpx {
@@ -134,67 +137,6 @@ __global__ void __launch_bounds__(NT, 1) k_rollout(const RolloutParams p) {
       }
       __syncthreads();
       VRPX_PROF(0)
-      // ---- glimpse score pass on the tensor pipe: S[node][head] = H_b[node][:] · q[head][:]  (m16n8k8, M = 16 nodes,
-      // N = 8 heads), q = 8 x 128 floats in shared memory.  Fragment coordinates g = lane >> 2, tq = lane & 3.  The K
-      // (embedding) axis is permuted so that every thread streams whole float4 chunks: chunk c (0..7) of thread tq
-      // covers dims 16c + 4tq + {0,1,2,3}; k-step 2c + u uses mma k-index tq <-> dim 16c+4tq+2u and k-index tq+4 <->
-      // dim 16c+4tq+2u+1, for A (node rows) and B (q) alike.  store(n, which, v): node n, head 2tq + which.
-      auto glimpse_scores = [&](const float* q, const float4* hrow, auto&& store) {
-        const int g = lane >> 2, tq = lane & 3;
-        float4 qv[8];   // q[head g][dims of this thread]
-#pragma unroll
-        for (int c = 0; c < 8; ++c) qv[c] = *reinterpret_cast<const float4*>(q + g * E + 16 * c + 4 * tq);
-        __syncwarp();
-        for (int n0 = 0; n0 < N; n0 += 16) {
-          const int na = n0 + g, nbb = n0 + g + 8;
-          // six independent accumulator chains (3 split terms x even/odd k-step): a single chain would serialise the
-          // 96 mma of a node tile on the tensor-pipe latency
-          float acc6[2][3][4];
-#pragma unroll
-          for (int a_ = 0; a_ < 2; ++a_)
-#pragma unroll
-            for (int b_ = 0; b_ < 3; ++b_)
-#pragma unroll
-              for (int i = 0; i < 4; ++i) acc6[a_][b_][i] = 0.f;
-#pragma unroll
-          for (int half = 0; half < 2; ++half) {
-            float4 va[4], vb[4];
-#pragma unroll
-            for (int cc = 0; cc < 4; ++cc) {
-              const int c = half * 4 + cc;
-              va[cc] = (na < N) ? __ldg(hrow + na * (E / 4) + 4 * c + tq) : make_float4(0.f, 0.f, 0.f, 0.f);
-              vb[cc] = (nbb < N) ? __ldg(hrow + nbb * (E / 4) + 4 * c + tq) : make_float4(0.f, 0.f, 0.f, 0.f);
-            }
-#pragma unroll
-            for (int cc = 0; cc < 4; ++cc) {
-              const int c = half * 4 + cc;
-              const float ae[4] = {va[cc].x, va[cc].y, va[cc].z, va[cc].w};
-              const float be[4] = {vb[cc].x, vb[cc].y, vb[cc].z, vb[cc].w};
-              const float qe[4] = {qv[c].x, qv[c].y, qv[c].z, qv[c].w};
-#pragma unroll
-              for (int u = 0; u < 2; ++u) {
-                uint32_t ah[4], al[4], bh0, bl0, bh1, bl1;
-                split_tf32(ae[2 * u], ah[0], al[0]);       // (row g,   k = tq)
-                split_tf32(be[2 * u], ah[1], al[1]);       // (row g+8, k = tq)
-                split_tf32(ae[2 * u + 1], ah[2], al[2]);   // (row g,   k = tq+4)
-                split_tf32(be[2 * u + 1], ah[3], al[3]);   // (row g+8, k = tq+4)
-                split_tf32(qe[2 * u], bh0, bl0);           // (k = tq,   n = g)
-                split_tf32(qe[2 * u + 1], bh1, bl1);       // (k = tq+4, n = g)
-                mma_tf32_16x8x8(acc6[u][0], al, bh0, bh1);
-                mma_tf32_16x8x8(acc6[u][1], ah, bl0, bl1);
-                mma_tf32_16x8x8(acc6[u][2], ah, bh0, bh1);
-              }
-            }
-          }
-          float acc[4];
-#pragma unroll
-          for (int i = 0; i < 4; ++i)
-            acc[i] = ((acc6[0][0][i] + acc6[1][0][i]) + (acc6[0][1][i] + acc6[1][1][i])) + (acc6[0][2][i] + acc6[1][2][i]);
-          // C fragment: acc[0], acc[1] = node na, heads 2tq, 2tq+1;  acc[2], acc[3] = node nbb
-          if (na < N) { store(na, 0, acc[0]); store(na, 1, acc[1]); }
-          if (nbb < N) { store(nbb, 0, acc[2]); store(nbb, 1, acc[3]); }
-        }
-      };
       // ---------------- P1: q~
       if (t == 0) {
         for (int o = tid; o < cnt * QW; o += NT) {
@@ -235,20 +177,20 @@ __global__ void __launch_bounds__(NT, 1) k_rollout(const RolloutParams p) {
       for (int m = warp; m < cnt; m += NT / 32) {
         const int64_t b = base + m;
         float* slot = QC + m * RQ_LD;
-        const int g = lane >> 2, t = lane & 3;
+        const int tq = lane & 3;
         const float4* hrow = reinterpret_cast<const float4*>(h + b * N * E);
         // ---- pass 1: scores = q~_h · h_n + scrambled additive mask
-        // masks of the instances whose rows the reference adds to heads 2t and 2t+1 (mask.repeat(H,1), graph_decoder.py:93)
+        // masks of the instances whose rows the reference adds to heads 2tq and 2tq+1 (mask.repeat(H,1), graph_decoder.py:93)
         uint32_t nb0[4], nb1[4];
         {
-          const uint32_t* m0 = gm_rd + quirk_row(b, 2 * t, p.G) * 4;
-          const uint32_t* m1 = gm_rd + quirk_row(b, 2 * t + 1, p.G) * 4;
+          const uint32_t* m0 = gm_rd + quirk_row(b, 2 * tq, p.G) * 4;
+          const uint32_t* m1 = gm_rd + quirk_row(b, 2 * tq + 1, p.G) * 4;
 #pragma unroll
           for (int i = 0; i < 4; ++i) { nb0[i] = __ldcg(m0 + i); nb1[i] = __ldcg(m1 + i); }
         }
-        glimpse_scores(slot, hrow, [&](int n, int which, float v) {
+        warp_glimpse_scores(slot, hrow, N, lane, [&](int n, int which, float v) {
           const uint32_t wsel = which ? nb1[n >> 5] : nb0[n >> 5];
-          slot[(2 * t + which) * E + n] = v + (float)((wsel >> (n & 31)) & 1u);
+          slot[(2 * tq + which) * E + n] = v + (float)((wsel >> (n & 31)) & 1u);
         });
         __syncwarp();
         VRPX_PROF(6)
@@ -260,87 +202,16 @@ __global__ void __launch_bounds__(NT, 1) k_rollout(const RolloutParams p) {
             const int n = lane + 32 * i;
             pr[hh][i] = (n < N) ? slot[hh * E + n] : -INFINITY;
           }
-        // softmax per head over nodes (lane = node, 4 strides cover N <= 128)
 #pragma unroll
-        for (int hh = 0; hh < NH; ++hh) {
-          float mx = -INFINITY;
-#pragma unroll
-          for (int i = 0; i < 4; ++i) mx = fmaxf(mx, pr[hh][i]);
-          mx = warp_max(mx);
-          float sum = 0.f;
-#pragma unroll
-          for (int i = 0; i < 4; ++i) {
-            int n = lane + 32 * i;
-            pr[hh][i] = (n < N) ? expf(pr[hh][i] - mx) : 0.f;
-            sum += pr[hh][i];
-          }
-          sum = warp_sum(sum);
-          float inv = 1.0f / sum;
-#pragma unroll
-          for (int i = 0; i < 4; ++i) pr[hh][i] *= inv;
-        }
+        for (int hh = 0; hh < NH; ++hh) warp_node_softmax(pr[hh], N);
         __syncwarp();
-        // probabilities to the slot as P[n][8]
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-          int n = lane + 32 * i;
-          if (n < N) {
-            *reinterpret_cast<float4*>(slot + n * 8) = make_float4(pr[0][i], pr[1][i], pr[2][i], pr[3][i]);
-            *reinterpret_cast<float4*>(slot + n * 8 + 4) = make_float4(pr[4][i], pr[5][i], pr[6][i], pr[7][i]);
-          }
-        }
+        warp_store_by_node(slot, pr, N, lane);
         __syncwarp();
         VRPX_PROF(7)
-        // ---- pass 2 on the tensor pipe: c[head][dim] = sum_n P[n][head] h_n[dim]  (M = 16 dims, N = 8 heads, K = 8 nodes)
-        // Thread g streams the float4 chunks 8c' + g (dims 32c' + 4g + e) of node rows n0+t and n0+t+4; m-tile
-        // j = 2c' + u has row g <-> dim 32c'+4g+2u and row g+8 <-> dim 32c'+4g+2u+1.  B = P[n][head] from the slot.
+        // ---- pass 2: c[head][dim] = sum_n P[n][head] h_n[dim], stored over P as the fp16-split A operand of GEMM-B
         float cacc[8][4];
-#pragma unroll
-        for (int j = 0; j < 8; ++j)
-#pragma unroll
-          for (int i = 0; i < 4; ++i) cacc[j][i] = 0.f;
-        for (int n0 = 0; n0 < N; n0 += 8) {
-          const int na = n0 + t, nbb = n0 + t + 4;
-          float4 va[4], vb[4];
-#pragma unroll
-          for (int cq = 0; cq < 4; ++cq) {
-            va[cq] = (na < N) ? __ldg(hrow + na * (E / 4) + 8 * cq + g) : make_float4(0.f, 0.f, 0.f, 0.f);
-            vb[cq] = (nbb < N) ? __ldg(hrow + nbb * (E / 4) + 8 * cq + g) : make_float4(0.f, 0.f, 0.f, 0.f);
-          }
-          uint32_t bh0, bl0, bh1, bl1;
-          split_tf32((na < N) ? slot[na * 8 + g] : 0.f, bh0, bl0);      // (k = t,   n = head g)
-          split_tf32((nbb < N) ? slot[nbb * 8 + g] : 0.f, bh1, bl1);    // (k = t+4, n = head g)
-#pragma unroll
-          for (int cq = 0; cq < 4; ++cq) {
-            const float ae[4] = {va[cq].x, va[cq].y, va[cq].z, va[cq].w};
-            const float be[4] = {vb[cq].x, vb[cq].y, vb[cq].z, vb[cq].w};
-#pragma unroll
-            for (int u = 0; u < 2; ++u) {
-              uint32_t ah[4], al[4];
-              split_tf32(ae[2 * u], ah[0], al[0]);       // (row g   = dim 32cq+4g+2u,   k = t   = node na)
-              split_tf32(ae[2 * u + 1], ah[1], al[1]);   // (row g+8 = dim 32cq+4g+2u+1, k = t)
-              split_tf32(be[2 * u], ah[2], al[2]);       // (row g,   k = t+4 = node nbb)
-              split_tf32(be[2 * u + 1], ah[3], al[3]);   // (row g+8, k = t+4)
-              mma_tf32_16x8x8(cacc[2 * cq + u], al, bh0, bh1);
-              mma_tf32_16x8x8(cacc[2 * cq + u], ah, bl0, bl1);
-              mma_tf32_16x8x8(cacc[2 * cq + u], ah, bh0, bh1);
-            }
-          }
-        }
-        __syncwarp();  // every lane is done reading P before c overwrites the slot
-        // C fragment of m-tile j = 2cq+u: [0] (dim d, head 2t), [1] (dim d, head 2t+1), [2] (dim d+1, head 2t),
-        // [3] (dim d+1, head 2t+1) with d = 32cq + 4g + 2u  ->  the A operand of GEMM-B, pre-split for the fp16 tensor
-        // path (tile_gemm.cuh): row m of C16, k = head * 128 + dim; per head and cq one 16-byte chunk = the two k-pairs
-        // (d0, d0+1), (d0+2, d0+3), d0 = 32cq + 4g, at the swizzled chunk (head*32 + 8cq + g) ^ (t << 1)
-        uint4* crow = reinterpret_cast<uint4*>(slot);
-#pragma unroll
-        for (int cq = 0; cq < 4; ++cq)
-#pragma unroll
-          for (int e = 0; e < 2; ++e) {
-            const uint2 p01 = split_f16x2(cacc[2 * cq][e], cacc[2 * cq][e + 2]);           // dims d0, d0+1 of head 2t+e
-            const uint2 p23 = split_f16x2(cacc[2 * cq + 1][e], cacc[2 * cq + 1][e + 2]);   // dims d0+2, d0+3
-            crow[(((2 * t + e) * 32 + 8 * cq + g) ^ (t << 1))] = make_uint4(p01.x, p01.y, p23.x, p23.y);
-          }
+        warp_glimpse_values_acc(cacc, slot, N, lane, glimpse_rows_global(hrow, N, lane));
+        warp_glimpse_store_c16(reinterpret_cast<uint4*>(slot), cacc, lane);
       }
       // rows >= cnt of C must be finite for GEMM-B (results unused): zero them
       for (int o = cnt * QW + tid; o < RTM * QW; o += NT) QC[(o >> 10) * RQ_LD + (o & (QW - 1))] = 0.f;
@@ -390,102 +261,18 @@ __global__ void __launch_bounds__(NT, 1) k_rollout(const RolloutParams p) {
           bool ok = n < N && !((mw[n >> 5] >> (n & 31)) & 1u);
           u[i] = ok ? slot[n] : -INFINITY;
         }
-        if (p.logits) {
-          float* lo = p.logits + ((int64_t)trel * B + b) * N;
-#pragma unroll
-          for (int i = 0; i < 4; ++i)
-            if (lane * 4 + i < N) lo[lane * 4 + i] = u[i];
-        }
-        // max + first-max index (argmax tie rule: lowest index)
-        float mx = u[0];
-        int am = lane * 4;
-#pragma unroll
-        for (int i = 1; i < 4; ++i)
-          if (u[i] > mx) { mx = u[i]; am = lane * 4 + i; }
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) {
-          float omx = __shfl_xor_sync(0xffffffffu, mx, o);
-          int oam = __shfl_xor_sync(0xffffffffu, am, o);
-          if (omx > mx || (omx == mx && oam < am)) { mx = omx; am = oam; }
-        }
-        int a = am;
-        float lp = 0.f;
-        if (p.mode != VRPX_GREEDY) {
-          float ex[4], loc = 0.f;
-#pragma unroll
-          for (int i = 0; i < 4; ++i) {
-            ex[i] = (u[i] == -INFINITY) ? 0.f : expf(u[i] - mx);
-            loc += ex[i];
-          }
-          float incl = loc;  // inclusive scan of lane totals
-#pragma unroll
-          for (int o = 1; o < 32; o <<= 1) {
-            float y = __shfl_up_sync(0xffffffffu, incl, o);
-            if (lane >= o) incl += y;
-          }
-          float total = __shfl_sync(0xffffffffu, incl, 31);
-          if (p.mode == VRPX_SAMPLE) {
-            uint64_t gid = p.offset + (uint64_t)b;
-            uint4 r = philox4x32_10(make_uint4((uint32_t)gid, (uint32_t)(gid >> 32), (uint32_t)t, 0x5eedu),
-                                    make_uint2((uint32_t)p.seed, (uint32_t)(p.seed >> 32)));
-            float thr = u24(r.x) * total;
-            float cum = incl - loc;
-            int pick = 1 << 30;
-#pragma unroll
-            for (int i = 0; i < 4; ++i) {
-              cum += ex[i];
-              if (ex[i] > 0.f && cum > thr && pick == (1 << 30)) pick = lane * 4 + i;
-            }
-#pragma unroll
-            for (int o = 16; o > 0; o >>= 1) pick = min(pick, __shfl_xor_sync(0xffffffffu, pick, o));
-            a = (pick == (1 << 30)) ? am : pick;  // rounding guard: fall back to the mode
-          } else {
-            a = (int)p.tape[(int64_t)trel * B + b];
-          }
-          // log-prob of the taken action (graph_decoder.py:107)
-          const int ai = a & 3;
-          float usel = ai == 0 ? u[0] : (ai == 1 ? u[1] : (ai == 2 ? u[2] : u[3]));
-          float ua = __shfl_sync(0xffffffffu, usel, a >> 2);
-          lp = (ua - mx) - logf(total);
-        }
-        if (lane == 0) { s_act[m] = a; s_lp[m] = lp; }
+        const PointerChoice c = warp_pointer_choice(u, p, b, t, trel, lane);
+        if (lane == 0) { s_act[m] = c.a; s_lp[m] = c.lp; }
       }
       __syncthreads();
       // environment transition: one THREAD per instance, so the dependent global loads (state -> coordinates) of the
       // whole tile overlap instead of running back to back on lane 0 of each warp
       if (tid < cnt) {
-        const int m = tid;
-        const int64_t b = base + m;
-        const int a = s_act[m];
-        if (p.tape && p.mode != VRPX_TEACHER) p.tape[(int64_t)trel * B + b] = (uint8_t)a;
-        Bits128 v;
+        const int64_t b = base + tid;
+        const EnvStepResult r = rollout_env_step(p, b, s_act[tid], s_lp[tid], t, trel);
 #pragma unroll
-        for (int i = 0; i < 4; ++i) v.w[i] = p.env.visited[b * 4 + i];
-        int cur = p.env.cur[b];
-        double load = p.env.load[b];
-        const int depot = p.env.depot[b];
-        const double* dem = p.env.demand ? p.env.demand + b * N : nullptr;
-        StepResult r = env_transition(kind, N, p.env.xy + b * N * 2, dem, depot, a, v, cur, load);
-        p.env.cur[b] = cur;
-        p.env.load[b] = load;
-#pragma unroll
-        for (int i = 0; i < 4; ++i) p.env.visited[b * 4 + i] = v.w[i];
-        Bits128 dm = v;   // decoder-visible mask after this step
-        if (kind == VRPX_IRP) {
-          Bits128 x = demand_exceeds(dem, N, load);
-#pragma unroll
-          for (int i = 0; i < 4; ++i) {
-            dm.w[i] = v.w[i] | x.w[i];
-            p.env.mask[b * 4 + i] = dm.w[i];
-          }
-        }
-#pragma unroll
-        for (int i = 0; i < 4; ++i) gm_wr[b * 4 + i] = dm.w[i];
-        // f32 accumulation of f32(reward) in step order (graph_tsp_agent.py:85); cost = -acc_loss
-        p.cost[b] = (t == 0 ? 0.f : p.cost[b]) + (float)r.dist;
-        if (p.mode != VRPX_GREEDY) p.logp[b] = (t == 0 ? 0.f : p.logp[b]) + s_lp[m];
-        else if (t == 0) p.logp[b] = 0.f;
-        if (!r.all_before) unfinished = true;
+        for (int i = 0; i < 4; ++i) gm_wr[b * 4 + i] = r.mask.w[i];
+        unfinished = r.unfinished;
       }
       if (unfinished) s_anyleft = 1;  // benign race: all writers store 1
       __syncthreads();

@@ -1,5 +1,5 @@
-// rollout.cuh — parameter block shared by the persistent rollout kernel (rollout.cu) and the split-step kernels
-// (rollout_steps.cu).
+// rollout.cuh — parameter block and the per-instance end of a decode step (action choice, environment step), shared by
+// the persistent rollout kernel (rollout.cu) and the split-step kernels (rollout_steps.cu).
 #pragma once
 #include "gemm.cuh"
 #include "tile_gemm.cuh"
@@ -54,5 +54,116 @@ struct SplitWorkspace {
 int prepare_split_weights(const RolloutParams& p, const SplitWorkspace& w, GemmPlan* plan_b, cudaStream_t stream);
 int run_first_steps(const RolloutParams& p, const SplitWorkspace& w, const GemmPlan& plan_b, cudaStream_t stream);
 int run_split_steps(const RolloutParams& p, int t_first, const GemmPlan& plan_b, cudaStream_t stream);
+
+// ---------------------------------------------------------------- the end of a decode step, after the pointer logits
+// (phase P4 of the persistent kernel and the split-step pointer kernel)
+struct PointerChoice {
+  int a;      // action
+  float lp;   // its log-prob (0 in greedy mode)
+};
+
+// One warp picks instance b's action at step t (trel = t - p.t0) from its masked logits: u[i] = node 4 lane + i, -inf
+// where masked or beyond N.  Writes them to p.logits when requested; argmax with ties to the lowest index, the Philox
+// inverse-CDF sample (counter (offset + b, t, 0x5eed)) or the teacher's action; log-prob of the taken action
+// (graph_decoder.py:107).  Every lane returns the same choice.
+__device__ __forceinline__ PointerChoice warp_pointer_choice(const float (&u)[4], const RolloutParams& p, int64_t b, int t,
+                                                             int trel, int lane) {
+  if (p.logits) {
+    float* lo = p.logits + ((int64_t)trel * p.env.B + b) * p.env.N;
+#pragma unroll
+    for (int i = 0; i < 4; ++i)
+      if (lane * 4 + i < p.env.N) lo[lane * 4 + i] = u[i];
+  }
+  // max + first-max index (argmax tie rule: lowest index)
+  float mx = u[0];
+  int am = lane * 4;
+#pragma unroll
+  for (int i = 1; i < 4; ++i)
+    if (u[i] > mx) { mx = u[i]; am = lane * 4 + i; }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    const float omx = __shfl_xor_sync(0xffffffffu, mx, o);
+    const int oam = __shfl_xor_sync(0xffffffffu, am, o);
+    if (omx > mx || (omx == mx && oam < am)) { mx = omx; am = oam; }
+  }
+  PointerChoice c{am, 0.f};
+  if (p.mode != VRPX_GREEDY) {
+    float ex[4], loc = 0.f;
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+      ex[i] = (u[i] == -INFINITY) ? 0.f : expf(u[i] - mx);
+      loc += ex[i];
+    }
+    float incl = loc;  // inclusive scan of lane totals
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const float y = __shfl_up_sync(0xffffffffu, incl, o);
+      if (lane >= o) incl += y;
+    }
+    const float total = __shfl_sync(0xffffffffu, incl, 31);
+    if (p.mode == VRPX_SAMPLE) {
+      const uint64_t gid = p.offset + (uint64_t)b;
+      const uint4 r = philox4x32_10(make_uint4((uint32_t)gid, (uint32_t)(gid >> 32), (uint32_t)t, 0x5eedu),
+                                    make_uint2((uint32_t)p.seed, (uint32_t)(p.seed >> 32)));
+      const float thr = u24(r.x) * total;
+      float cum = incl - loc;
+      int pick = 1 << 30;
+#pragma unroll
+      for (int i = 0; i < 4; ++i) {
+        cum += ex[i];
+        if (ex[i] > 0.f && cum > thr && pick == (1 << 30)) pick = lane * 4 + i;
+      }
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) pick = min(pick, __shfl_xor_sync(0xffffffffu, pick, o));
+      c.a = (pick == (1 << 30)) ? am : pick;  // rounding guard: fall back to the mode
+    } else {
+      c.a = (int)p.tape[(int64_t)trel * p.env.B + b];
+    }
+    const int ai = c.a & 3;
+    const float usel = ai == 0 ? u[0] : (ai == 1 ? u[1] : (ai == 2 ? u[2] : u[3]));
+    const float ua = __shfl_sync(0xffffffffu, usel, c.a >> 2);
+    c.lp = (ua - mx) - logf(total);
+  }
+  return c;
+}
+
+struct EnvStepResult {
+  bool unfinished;   // some node is still unvisited after this step's visit (the instance's `done` is false)
+  Bits128 mask;      // decoder-visible mask after the step
+};
+
+// One thread steps instance b at step t (trel = t - p.t0) with action a of log-prob lp: tape write (sample / greedy), env_transition
+// (env_rules.cuh), state write-back, the IRP mask (rule R4), and the f32 accumulation of cost and log-prob in step order.
+__device__ __forceinline__ EnvStepResult rollout_env_step(const RolloutParams& p, int64_t b, int a, float lp, int t,
+                                                          int trel) {
+  const int N = p.env.N, kind = p.env.kind;
+  if (p.tape && p.mode != VRPX_TEACHER) p.tape[(int64_t)trel * p.env.B + b] = (uint8_t)a;
+  Bits128 v;
+#pragma unroll
+  for (int i = 0; i < 4; ++i) v.w[i] = p.env.visited[b * 4 + i];
+  int cur = p.env.cur[b];
+  double load = p.env.load[b];
+  const int depot = p.env.depot[b];
+  const double* dem = p.env.demand ? p.env.demand + b * N : nullptr;
+  const StepResult r = env_transition(kind, N, p.env.xy + b * N * 2, dem, depot, a, v, cur, load);
+  p.env.cur[b] = cur;
+  p.env.load[b] = load;
+#pragma unroll
+  for (int i = 0; i < 4; ++i) p.env.visited[b * 4 + i] = v.w[i];
+  EnvStepResult res{!r.all_before, v};
+  if (kind == VRPX_IRP) {
+    const Bits128 x = demand_exceeds(dem, N, load);
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+      res.mask.w[i] = v.w[i] | x.w[i];
+      p.env.mask[b * 4 + i] = res.mask.w[i];
+    }
+  }
+  // f32 accumulation of f32(reward) in step order (graph_tsp_agent.py:85); cost = -acc_loss
+  p.cost[b] = (t == 0 ? 0.f : p.cost[b]) + (float)r.dist;
+  if (p.mode != VRPX_GREEDY) p.logp[b] = (t == 0 ? 0.f : p.logp[b]) + lp;
+  else if (t == 0) p.logp[b] = 0.f;
+  return res;
+}
 
 }  // namespace vrpx

@@ -11,9 +11,11 @@
 //                    once per 128 instances instead of once per 16
 //   k_step_pointer   one warp per instance: logits 10 tanh(q^ · h_n), mask, argmax / Philox sample / teacher action,
 //                    log-prob; then one thread per instance runs the environment transition (env_rules.cuh)
-// Softmax, glimpse values and pointer phase are those of phases P2 and P4 of the persistent kernel (the code is carried
-// over); against its classic loop the results differ only by the evaluation order of the scores (tables) and the
-// summation order inside GEMM-B.  The classic mode and resumed single-step calls run in the persistent kernel.
+// Softmax, glimpse values and pointer phase are those of phases P2 and P4 of the persistent kernel: both call the helpers
+// of glimpse_mma.cuh (warp_node_softmax, warp_store_by_node, warp_glimpse_values_acc) and rollout.cuh
+// (warp_pointer_choice, rollout_env_step).  Against its classic loop the results differ only by the evaluation order of
+// the scores (tables) and the summation order inside GEMM-B.  The classic mode and resumed single-step calls run in the
+// persistent kernel.
 // The launches are asynchronous on the caller's stream: no host round trip per step.  An episode that finishes early
 // (VRP / IRP) turns the remaining launches into no-ops through the per-step `notdone` counters.
 #include "gemm.cuh"
@@ -135,52 +137,17 @@ __global__ void __launch_bounds__(GW_MAX * 32, 2) k_step_glimpse(const RolloutPa
       }
     }
   }
-  // ---- softmax per head over nodes (lane = node; only the ceil(N / 32) strides that hold nodes are touched)
 #pragma unroll
-  for (int hh = 0; hh < NH; ++hh) {
-    float mx = pr[hh][0];
-#pragma unroll
-    for (int i = 1; i < 4; ++i)
-      if (32 * i < N) mx = fmaxf(mx, pr[hh][i]);
-    mx = warp_max(mx);
-    float sum = 0.f;
-#pragma unroll
-    for (int i = 0; i < 4; ++i)
-      if (32 * i < N) {
-        pr[hh][i] = expf(pr[hh][i] - mx);   // exp(-inf) = 0 for the lanes beyond N (ex2.approx was measured: no time gained,
-                                            // mean logit error 4x larger)
-        sum += pr[hh][i];
-      }
-    sum = warp_sum(sum);
-    const float inv = 1.0f / sum;
-#pragma unroll
-    for (int i = 0; i < 4; ++i)
-      if (32 * i < N) pr[hh][i] *= inv;
-  }
-  // probabilities to the slot as P[n][8]
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    const int n = lane + 32 * i;
-    if (n < N) {
-      *reinterpret_cast<float4*>(slot + n * 8) = make_float4(pr[0][i], pr[1][i], pr[2][i], pr[3][i]);
-      *reinterpret_cast<float4*>(slot + n * 8 + 4) = make_float4(pr[4][i], pr[5][i], pr[6][i], pr[7][i]);
-    }
-  }
+  for (int hh = 0; hh < NH; ++hh) warp_node_softmax(pr[hh], N);
+  warp_store_by_node(slot, pr, N, lane);
   __syncwarp();
-  // ---- c[head][dim] = sum_n P[n][head] h_n[dim] on the tensor pipe (M = 16 dims, N = 8 heads, K = 8 nodes).
-  // Thread g reads the float4 chunks 8c' + g (dims 32c' + 4g + e) of node rows n0+tq and n0+tq+4; m-tile
-  // j = 2c' + u has row g <-> dim 32c'+4g+2u and row g+8 <-> dim 32c'+4g+2u+1.  B = P[n][head] from the slot.
+  // ---- c[head][dim] = sum_n P[n][head] h_n[dim], the node rows from the ring
   float cacc[8][4];
-#pragma unroll
-  for (int j = 0; j < 8; ++j)
-#pragma unroll
-    for (int i = 0; i < 4; ++i) cacc[j][i] = 0.f;
-  for (int sidx = 0; sidx < nsl; ++sidx) {
+  warp_glimpse_values_acc(cacc, slot, N, lane, [&](int n0, float4 (&va)[4], float4 (&vb)[4]) {
+    const int sidx = n0 >> 3;
     cp_async_wait<GNS - 1>();   // slice sidx has landed (one group per slice, possibly empty, keeps the count uniform)
     __syncwarp();
-    const int n0 = 8 * sidx, na = n0 + tq, nbb = n0 + tq + 4;
     const unsigned char* st = ring + (sidx % GNS) * G_SLICE;
-    float4 va[4], vb[4];
 #pragma unroll
     for (int cq = 0; cq < 4; ++cq) {
       va[cq] = *reinterpret_cast<const float4*>(st + tq * G_ROW + (8 * cq + g) * 16);
@@ -189,48 +156,18 @@ __global__ void __launch_bounds__(GW_MAX * 32, 2) k_step_glimpse(const RolloutPa
     if (n0 + 8 > N) {   // uniform: only the last slice has rows beyond N (stale ring contents)
 #pragma unroll
       for (int cq = 0; cq < 4; ++cq) {
-        if (na >= N) va[cq] = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (nbb >= N) vb[cq] = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (n0 + tq >= N) va[cq] = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (n0 + tq + 4 >= N) vb[cq] = make_float4(0.f, 0.f, 0.f, 0.f);
       }
     }
     __syncwarp();   // every lane has read the stage before it is refilled
     if (sidx + GNS < nsl) issue_slice(sidx + GNS);
     else cp_async_commit();
-    uint32_t bh0, bl0, bh1, bl1;
-    split_tf32((na < N) ? slot[na * 8 + g] : 0.f, bh0, bl0);      // (k = tq,   n = head g)
-    split_tf32((nbb < N) ? slot[nbb * 8 + g] : 0.f, bh1, bl1);    // (k = tq+4, n = head g)
-#pragma unroll
-    for (int cq = 0; cq < 4; ++cq) {
-      const float ae[4] = {va[cq].x, va[cq].y, va[cq].z, va[cq].w};
-      const float be[4] = {vb[cq].x, vb[cq].y, vb[cq].z, vb[cq].w};
-#pragma unroll
-      for (int u = 0; u < 2; ++u) {
-        uint32_t ah[4], al[4];
-        split_tf32(ae[2 * u], ah[0], al[0]);       // (row g   = dim 32cq+4g+2u,   k = tq   = node na)
-        split_tf32(ae[2 * u + 1], ah[1], al[1]);   // (row g+8 = dim 32cq+4g+2u+1, k = tq)
-        split_tf32(be[2 * u], ah[2], al[2]);       // (row g,   k = tq+4 = node nbb)
-        split_tf32(be[2 * u + 1], ah[3], al[3]);   // (row g+8, k = tq+4)
-        mma_tf32_16x8x8(cacc[2 * cq + u], al, bh0, bh1);
-        mma_tf32_16x8x8(cacc[2 * cq + u], ah, bl0, bl1);
-        mma_tf32_16x8x8(cacc[2 * cq + u], ah, bh0, bh1);
-      }
-    }
-  }
+  });
   cp_async_wait<0>();
-  __syncwarp();
-  // C fragment of m-tile j = 2cq+u: [0] (dim d, head 2tq), [1] (dim d, head 2tq+1), [2] (dim d+1, head 2tq),
-  // [3] (dim d+1, head 2tq+1) with d = 32cq + 4g + 2u  ->  c[head][dim] staged in the (now idle) ring, then one
-  // coalesced copy
+  // c staged in the (now idle) ring, then one coalesced copy
   float* cst = reinterpret_cast<float*>(ring);
-#pragma unroll
-  for (int cq = 0; cq < 4; ++cq)
-#pragma unroll
-    for (int u = 0; u < 2; ++u) {
-      const int d = 32 * cq + 4 * g + 2 * u, j = 2 * cq + u;
-      *reinterpret_cast<float2*>(cst + (2 * tq) * E + d) = make_float2(cacc[j][0], cacc[j][2]);
-      *reinterpret_cast<float2*>(cst + (2 * tq + 1) * E + d) = make_float2(cacc[j][1], cacc[j][3]);
-    }
-  __syncwarp();
+  warp_glimpse_store_c(cst, cacc, lane);
   float4* dst = reinterpret_cast<float4*>(p.cbuf + b * QW);
   for (int i = lane; i < QW / 4; i += 32) dst[i] = *reinterpret_cast<const float4*>(cst + 4 * i);
 }
@@ -327,98 +264,13 @@ __global__ void __launch_bounds__(SW * 32) k_step_pointer(const RolloutParams p,
       const bool ok = n < N && !((mw[n >> 5] >> (n & 31)) & 1u);
       u[i] = ok ? (idle ? 0.f : slot[n]) : -INFINITY;   // idle: one candidate, any finite logit gives action = depot, log-prob 0
     }
-    if (p.logits) {
-      float* lo = p.logits + ((int64_t)trel * B + b) * N;
-#pragma unroll
-      for (int i = 0; i < 4; ++i)
-        if (lane * 4 + i < N) lo[lane * 4 + i] = u[i];
-    }
-    // max + first-max index (argmax tie rule: lowest index)
-    float mx = u[0];
-    int am = lane * 4;
-#pragma unroll
-    for (int i = 1; i < 4; ++i)
-      if (u[i] > mx) { mx = u[i]; am = lane * 4 + i; }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-      const float omx = __shfl_xor_sync(0xffffffffu, mx, o);
-      const int oam = __shfl_xor_sync(0xffffffffu, am, o);
-      if (omx > mx || (omx == mx && oam < am)) { mx = omx; am = oam; }
-    }
-    int a = am;
-    float lp = 0.f;
-    if (p.mode != VRPX_GREEDY) {
-      float ex[4], loc = 0.f;
-#pragma unroll
-      for (int i = 0; i < 4; ++i) {
-        ex[i] = (u[i] == -INFINITY) ? 0.f : expf(u[i] - mx);
-        loc += ex[i];
-      }
-      float incl = loc;  // inclusive scan of lane totals
-#pragma unroll
-      for (int o = 1; o < 32; o <<= 1) {
-        const float y = __shfl_up_sync(0xffffffffu, incl, o);
-        if (lane >= o) incl += y;
-      }
-      const float total = __shfl_sync(0xffffffffu, incl, 31);
-      if (p.mode == VRPX_SAMPLE) {
-        const uint64_t gid = p.offset + (uint64_t)b;
-        const uint4 r = philox4x32_10(make_uint4((uint32_t)gid, (uint32_t)(gid >> 32), (uint32_t)t, 0x5eedu),
-                                      make_uint2((uint32_t)p.seed, (uint32_t)(p.seed >> 32)));
-        const float thr = u24(r.x) * total;
-        float cum = incl - loc;
-        int pick = 1 << 30;
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-          cum += ex[i];
-          if (ex[i] > 0.f && cum > thr && pick == (1 << 30)) pick = lane * 4 + i;
-        }
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) pick = min(pick, __shfl_xor_sync(0xffffffffu, pick, o));
-        a = (pick == (1 << 30)) ? am : pick;  // rounding guard: fall back to the mode
-      } else {
-        a = (int)p.tape[(int64_t)trel * B + b];
-      }
-      // log-prob of the taken action (graph_decoder.py:107)
-      const int ai = a & 3;
-      const float usel = ai == 0 ? u[0] : (ai == 1 ? u[1] : (ai == 2 ? u[2] : u[3]));
-      const float ua = __shfl_sync(0xffffffffu, usel, a >> 2);
-      lp = (ua - mx) - logf(total);
-    }
-    if (lane == 0) { s_act[warp] = a; s_lp[warp] = lp; }
+    const PointerChoice c = warp_pointer_choice(u, p, b, t, trel, lane);
+    if (lane == 0) { s_act[warp] = c.a; s_lp[warp] = c.lp; }
   }
   __syncthreads();
   // environment transition: one THREAD per instance (the dependent global loads of the CTA's instances overlap)
-  bool unfinished = false;
-  if (tid < cnt) {
-    const int m = tid;
-    const int64_t b = base + m;
-    const int a = s_act[m];
-    if (p.tape && p.mode != VRPX_TEACHER) p.tape[(int64_t)trel * B + b] = (uint8_t)a;
-    Bits128 v;
-#pragma unroll
-    for (int i = 0; i < 4; ++i) v.w[i] = p.env.visited[b * 4 + i];
-    int cur = p.env.cur[b];
-    double load = p.env.load[b];
-    const int depot = p.env.depot[b];
-    const double* dem = p.env.demand ? p.env.demand + b * N : nullptr;
-    StepResult r = env_transition(kind, N, p.env.xy + b * N * 2, dem, depot, a, v, cur, load);
-    p.env.cur[b] = cur;
-    p.env.load[b] = load;
-#pragma unroll
-    for (int i = 0; i < 4; ++i) p.env.visited[b * 4 + i] = v.w[i];
-    if (kind == VRPX_IRP) {
-      Bits128 x = demand_exceeds(dem, N, load);
-#pragma unroll
-      for (int i = 0; i < 4; ++i) p.env.mask[b * 4 + i] = v.w[i] | x.w[i];
-    }
-    // f32 accumulation of f32(reward) in step order (graph_tsp_agent.py:85); cost = -acc_loss
-    p.cost[b] = (t == 0 ? 0.f : p.cost[b]) + (float)r.dist;
-    if (p.mode != VRPX_GREEDY) p.logp[b] = (t == 0 ? 0.f : p.logp[b]) + s_lp[m];
-    else if (t == 0) p.logp[b] = 0.f;
-    if (!r.all_before) unfinished = true;
-  }
-  if (unfinished) s_anyleft = 1;  // benign race: all writers store 1
+  if (tid < cnt && rollout_env_step(p, base + tid, s_act[tid], s_lp[tid], t, trel).unfinished)
+    s_anyleft = 1;   // benign race: all writers store 1
   __syncthreads();
   if (tid == 0 && s_anyleft) atomicAdd(p.notdone + trel, 1);
 }
@@ -429,8 +281,8 @@ __global__ void __launch_bounds__(SW * 32) k_step_pointer(const RolloutParams p,
 // step 1 completes the per-episode tables (Q~g += A_f h[first]; S0 = Q~g_head · h_n; IRP: SL = a_load_head · h_n).  They
 // used to run inside the persistent kernel (4.7 ms at C4, L2-bound on 16-instance tiles); here they are whole-batch
 // launches like every later step: a mean / gather kernel, a batched tcgen05 GEMM for the 128 -> 1024 query fold, and a
-// glimpse kernel that computes the scores from q~ itself (one warp per instance, mma.sync TF32 3-term, the score and value
-// passes of the persistent kernel's phase P2) instead of reading them from the tables.
+// glimpse kernel that computes the scores from q~ itself (one warp per instance, mma.sync TF32 3-term: the score and value
+// contractions of glimpse_mma.cuh) instead of reading them from the tables.
 
 // G[b] = mean_n h[b, n]  (graph_decoder.py:75-77), one warp per instance
 __global__ void __launch_bounds__(256) k_episode_mean(const float* __restrict__ h, int64_t B, int N, float* __restrict__ G) {
@@ -554,33 +406,9 @@ __global__ void __launch_bounds__(FW * 32, 2) k_step_glimpse_first(const Rollout
         pr[hh][i] += (float)((wsel >> lane) & 1u);   // -inf stays -inf for the lanes beyond N
       }
   }
-  // ---- softmax per head over nodes (lane = node, 4 strides cover N <= 128)
 #pragma unroll
-  for (int hh = 0; hh < NH; ++hh) {
-    float mx = -INFINITY;
-#pragma unroll
-    for (int i = 0; i < 4; ++i) mx = fmaxf(mx, pr[hh][i]);
-    mx = warp_max(mx);
-    float sum = 0.f;
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      const int n = lane + 32 * i;
-      pr[hh][i] = (n < N) ? expf(pr[hh][i] - mx) : 0.f;
-      sum += pr[hh][i];
-    }
-    sum = warp_sum(sum);
-    const float inv = 1.0f / sum;
-#pragma unroll
-    for (int i = 0; i < 4; ++i) pr[hh][i] *= inv;
-  }
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    const int n = lane + 32 * i;
-    if (n < N) {
-      *reinterpret_cast<float4*>(slot + n * 8) = make_float4(pr[0][i], pr[1][i], pr[2][i], pr[3][i]);
-      *reinterpret_cast<float4*>(slot + n * 8 + 4) = make_float4(pr[4][i], pr[5][i], pr[6][i], pr[7][i]);
-    }
-  }
+  for (int hh = 0; hh < NH; ++hh) warp_node_softmax(pr[hh], N);
+  warp_store_by_node(slot, pr, N, lane);
   __syncwarp();
   // ---- c[head][dim] = sum_n P[n][head] h_n[dim] (the second pass over the instance's embeddings comes from L2)
   warp_glimpse_values(slot, hrow, N, lane);

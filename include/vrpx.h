@@ -339,6 +339,11 @@ VRPX_API int vrpx_debug_qkv_attention(const float* X, const float* in_proj_w, co
                                       float* att, void* stream);
 VRPX_API void vrpx_debug_encoder_fuse_attention(int32_t enable);
 
+/* Test hook of the score-table kernel of the split-step rollout (csrc/score_table_fused.cu):
+ * s1 [B][N][8][N] = per-head q'·k' of every (last, node) pair with q' = h·(W_l/sqrt(48))^T, k' = h·W_k^T, from h [B·N][128]
+ * and qk_w [768][128] (rows 0..383 W_l/sqrt(48), 384..767 W_k, head-major; vrpx/packing.py fold_decoder). */
+VRPX_API int vrpx_debug_score_table(const float* h, const float* qk_w, int64_t B, int32_t N, float* s1, void* stream);
+
 /* Test hook of the attention backward (csrc/attention_bwd.cu): dqkv [B·N][384] = d(loss)/d(qkv) of the per-instance
  * 8-head attention core given qkv [B·N][384], its output att [B·N][128] and datt = d(loss)/d(att)
  * (path 0: mma.sync f16-split kernel = production; path 1: fp32 SIMT kernel). */

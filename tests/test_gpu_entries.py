@@ -63,7 +63,8 @@ def test_graph_demand_encoder_entry():
         assert _rel(h.numpy(), ref.numpy()) < 1e-5
 
 
-@pytest.mark.parametrize("kind,N,B", [("tsp", 8, 2), ("vrp", 20, 16), ("irp", 30, 9)])
+@pytest.mark.parametrize("kind,N,B", [("tsp", 8, 2), ("vrp", 20, 16), ("irp", 30, 9), ("tsp", 128, 3), ("vrp", 65, 5),
+                                      ("irp", 97, 4)])
 def test_single_step_decoder_episode_vs_oracle(kind, N, B):
     """Drive a whole episode the way the reference's model loop does (graph_tsp_agent.py:78-88): per step
     `decoder(emb, mask[, load], rollout=True)` -> env step on the host (env oracle) -> next mask.  Every greedy action is

@@ -238,3 +238,58 @@ def test_attention_backward_mma(B, N):
     for c0 in (0, 128, 256):
         r = ref[:, c0:c0 + 128]
         assert (outs[0][:, c0:c0 + 128].double() - r).abs().max().item() <= 2e-5 * r.abs().max().item(), c0
+
+
+def _score_table_tile(N):
+    """Instances per tile of csrc/score_table_fused.cu (build_score_table_fused): whole instances in 128 rows, capped so
+    that the k' fragments of a tile fit its KMAX = 200 keys."""
+    nt = (N + 7) // 8
+    bucket = 3 if nt <= 3 else (7 if nt <= 7 else (13 if nt <= 13 else 16))
+    return min(128 // N, 1 + (200 - 8 * bucket) // (8 * nt))
+
+
+# every N: B leaves a ragged last tile of 1 .. TI - 1 instances (TI = 1 above N = 64); then more than 37 tiles, so that
+# each of the 37 streams of head-pair CTAs walks several tiles, in the three upper template buckets
+SCORE_TABLE_CASES = [(N, 2 * _score_table_tile(N) + (1 + N % (_score_table_tile(N) - 1) if _score_table_tile(N) > 1 else 1))
+                     for N in range(2, 129)] + [(20, 2003), (50, 2001), (105, 1999), (128, 2000)]
+# largest error / largest |S1| of its (instance, head) block: measured 2.2e-6 on a B200 (1000 W power limit)
+SCORE_TABLE_TOL = 1e-5
+
+
+def test_score_table_fused_kernel():
+    """csrc/score_table_fused.cu: S1[b][l][head][n] = q'[b,l,head] · k'[b,n,head] with q' = h (W_l / sqrt(48))^T and
+    k' = h W_k^T (the rank-48 factors of the decoder's step query, vrpx/packing.py qk_w) against float64, for every
+    N = 2 .. 128 (template buckets NT8 = 3 / 7 / 13 / 16, tiles of TI = 1 .. 23 instances, the float2 store of even N and
+    the scalar store of odd N) and multi-tile streams.  S1 and a guard tail behind it start as NaN: every element of
+    [B][N][8][N] is written and nothing beyond it."""
+    import vrpx
+    from agents import TSPAgent
+    from vrpx import packing
+
+    dev = vrpx.require_device()
+    L = vrpx.lib()
+    qk_w = packing.fold_decoder(TSPAgent(seed=5).model.decoder, False)["qk_w"].to(dev, torch.float32).contiguous()
+    wq = qk_w[:384].double().view(8, 48, 128)
+    wk = qk_w[384:].double().view(8, 48, 128)
+    g = torch.Generator(device=dev).manual_seed(17)
+    guard = 4096
+    worst = (0.0, None)
+    for N, B in SCORE_TABLE_CASES:
+        h = torch.randn(B, N, 128, generator=g, device=dev)     # BatchNorm output scale
+        n1 = B * N * 8 * N
+        s1 = torch.full((n1 + guard,), float("nan"), device=dev)
+        vrpx.check(L.vrpx_debug_score_table(vrpx.ptr(h), vrpx.ptr(qk_w), B, N, vrpx.ptr(s1), vrpx.stream_ptr(dev)))
+        torch.cuda.synchronize()
+        assert bool(torch.isnan(s1[n1:]).all()), (N, B, "wrote beyond S1")
+        got = s1[:n1].view(B, N, 8, N)
+        assert not bool(torch.isnan(got).any()), (N, B, "S1 element not written")
+        hd = h.double()
+        q = torch.einsum("bld,hjd->bhlj", hd, wq)
+        k = torch.einsum("bnd,hjd->bhnj", hd, wk)
+        ref = torch.einsum("bhlj,bhnj->blhn", q, k)
+        err = (got.double() - ref).abs().amax(dim=(1, 3))        # (B, 8) per (instance, head) block
+        scale = ref.abs().amax(dim=(1, 3))
+        r = (err / scale).max().item()
+        worst = max(worst, (r, (N, B)), key=lambda w: w[0])
+        assert r <= SCORE_TABLE_TOL, (N, B, r)
+    print(f"\n[score table] max error / block max {worst[0]:.3g} at (N, B) = {worst[1]}")

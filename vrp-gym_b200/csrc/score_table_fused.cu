@@ -363,3 +363,11 @@ int build_score_table_fused(const float* h, const float* qk_w, int64_t B, int N,
 }
 
 }  // namespace vrpx
+
+extern "C" int vrpx_debug_score_table(const float* h, const float* qk_w, int64_t B, int32_t N, float* s1, void* stream) {
+  VRPX_CHECK_ARG(h && qk_w && s1, "NULL argument");
+  VRPX_DEVICE_GUARD(h);
+  __half* w16 = vrpx::tc4::split_scratch((cudaStream_t)stream);
+  if (!w16) return VRPX_ERR_CUDA;
+  return vrpx::build_score_table_fused(h, qk_w, B, N, w16, s1, (cudaStream_t)stream);
+}

@@ -157,6 +157,7 @@ def lib():
     L.vrpx_debug_qkv_attention.argtypes = [vp, vp, vp, i64, i32, vp, vp]
     L.vrpx_debug_encoder_fuse_attention.argtypes = [i32]
     L.vrpx_debug_encoder_fuse_attention.restype = None
+    L.vrpx_debug_score_table.argtypes = [vp, vp, i64, i32, vp, vp]
     if L.vrpx_abi_version() != ABI_VERSION:
         raise VrpxError("libvrpx.so ABI version mismatch")
     _lib = L

@@ -118,6 +118,4 @@ __device__ __forceinline__ double u53(uint32_t a, uint32_t b) {
 }
 __device__ __forceinline__ float u24(uint32_t a) { return (float)(a >> 8) * (1.0f / 16777216.0f); }
 
-__device__ __forceinline__ bool bit_test(const uint32_t w[4], int n) { return (w[n >> 5] >> (n & 31)) & 1u; }
-
 }  // namespace vrpx

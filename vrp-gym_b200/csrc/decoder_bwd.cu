@@ -3,7 +3,7 @@
 //
 // Given the action tape, every decode step depends only on (h, tape, packed weights): step t reads
 // last = tape[t-1], first = tape[0], the recorded masks and loads.  So instead of storing (B,T,·) activations the
-// backward RECOMPUTES each step's forward (same tile GEMMs / per-instance phases as rollout.cu) and immediately
+// backward RECOMPUTES each step's forward (same tile GEMMs / per-instance helpers as rollout.cu) and immediately
 // back-propagates d(logp_{b,t}) * w_b, accumulating
 //     dH            (B,N,128)   gradient w.r.t. the encoder output (all paths: scores, glimpse values, pointer
 //                               logits, h[last]; the graph-mean / h[first] terms are added by the epilogue)
@@ -17,7 +17,7 @@
 // c_h = sum_n p_hn h_n;  q^ = M c + m_c;  z_n = q^·h_n;  u_n = 10 tanh z_n;  pi = softmax(u | unmasked).
 #include "gemm.cuh"
 #include "glimpse_mma.cuh"
-#include "tile_gemm.cuh"
+#include "rollout.cuh"
 
 namespace vrpx {
 
@@ -41,13 +41,47 @@ struct DecBwdParams {
 constexpr size_t BWD_X = (size_t)TM * XS_LD * sizeof(float), BWD_QC = (size_t)TM * QC_LD * sizeof(float);
 constexpr size_t BWD_SMEM = BWD_X + BWD_QC + SMEM_W + BWD_X;
 
-__device__ __forceinline__ void red_add4(float* p, float4 v) {
-  asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(p), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w)
-               : "memory");
-}
-
 __device__ __forceinline__ void red_add2(float* p, float a, float b) {
   asm volatile("red.global.add.v2.f32 [%0], {%1, %2};" ::"l"(p), "f"(a), "f"(b) : "memory");
+}
+
+// dst[r][c] += sum_m A[m][r] Bm[m][c] for the 16 x 64 block r < 16, c < 64, m over the TM instances of the tile (the
+// weight gradients of B5 / B8).  Tensor pipe, TF32 3-term: A fragment (row r, col m) = A[m][r], B fragment (row m, col c)
+// = Bm[m][c]; every accumulator sums the k-steps in order, then red.global.add.
+__device__ __forceinline__ void warp_outer_product_tm(const float* A, int lda, const float* Bm, int ldb, float* dst, int ldd,
+                                                      int lane) {
+  const int g = lane >> 2, t4 = lane & 3;
+  float acc[8][4];
+#pragma unroll
+  for (int j = 0; j < 8; ++j)
+#pragma unroll
+    for (int i = 0; i < 4; ++i) acc[j][i] = 0.f;
+#pragma unroll
+  for (int ks = 0; ks < TM / 8; ++ks) {
+    uint32_t ah[4], al[4];
+    const float* r0 = A + (ks * 8 + t4) * lda + g;
+    const float* r1 = r0 + 4 * lda;
+    split_tf32(r0[0], ah[0], al[0]);
+    split_tf32(r0[8], ah[1], al[1]);
+    split_tf32(r1[0], ah[2], al[2]);
+    split_tf32(r1[8], ah[3], al[3]);
+    const float* b0p = Bm + (ks * 8 + t4) * ldb + g;
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+      uint32_t bh0, bl0, bh1, bl1;
+      split_tf32(b0p[8 * j], bh0, bl0);
+      split_tf32(b0p[4 * ldb + 8 * j], bh1, bl1);
+      mma_tf32_16x8x8(acc[j], al, bh0, bh1);
+      mma_tf32_16x8x8(acc[j], ah, bl0, bl1);
+      mma_tf32_16x8x8(acc[j], ah, bh0, bh1);
+    }
+  }
+#pragma unroll
+  for (int j = 0; j < 8; ++j) {
+    float* d = dst + (size_t)g * ldd + 8 * j + 2 * t4;
+    red_add2(d, acc[j][0], acc[j][1]);
+    red_add2(d + 8 * ldd, acc[j][2], acc[j][3]);
+  }
 }
 
 __global__ void __launch_bounds__(NT, 1) k_decoder_bwd(const DecBwdParams p) {
@@ -109,23 +143,15 @@ __global__ void __launch_bounds__(NT, 1) k_decoder_bwd(const DecBwdParams p) {
       // ---------------- B1: q~ (recompute)
       if (t == 0) {
         for (int o = tid; o < cnt * QW; o += NT) {
-          int m = o >> 10, c = o & (QW - 1);
-          float y = p.qg0[(base + m) * QW + c] + p.a_q0[c];
-          if (kind == VRPX_IRP) y = fmaf(s_loadf[m], p.a_load[c], y);
-          QC[m * QC_LD + c] = y;
+          const int m = o >> 10, c = o & (QW - 1);
+          QC[m * QC_LD + c] = step0_query(p.qg0 + (base + m) * QW, p.a_q0, p.a_load, kind == VRPX_IRP, s_loadf[m], c);
         }
       } else {
         tile_gemm_wide_mma_sw<2, 2>(
             Xs, XS_LD, p.al_t, Wb,
-            [&](int m, int c) -> float2 {
-              if (m >= cnt) return make_float2(0.f, 0.f);
-              float2 q = *reinterpret_cast<const float2*>(p.qg + (base + m) * QW + c);
-              if (kind == VRPX_IRP) {
-                const float2 al = *reinterpret_cast<const float2*>(p.a_load + c);
-                const float lf = s_loadf[m];
-                q = make_float2(fmaf(lf, al.x, q.x), fmaf(lf, al.y, q.y));
-              }
-              return q;
+            [&](int m, int c) {
+              return (m < cnt) ? glimpse_query_init(p.qg + (base + m) * QW, p.a_load, kind == VRPX_IRP, s_loadf[m], c)
+                               : make_float2(0.f, 0.f);
             },
             [&](int m, int c, float v0, float v1) {
               if (m < cnt) *reinterpret_cast<float2*>(QC + m * QC_LD + c) = make_float2(v0, v1);
@@ -164,11 +190,7 @@ __global__ void __launch_bounds__(NT, 1) k_decoder_bwd(const DecBwdParams p) {
         float pr[NH][4];
 #pragma unroll
         for (int hh = 0; hh < NH; ++hh) {
-#pragma unroll
-          for (int i = 0; i < 4; ++i) {
-            const int n = lane + 32 * i;
-            pr[hh][i] = (n < N) ? slot[hh * E + n] : -INFINITY;
-          }
+          warp_load_by_head(pr[hh], slot + hh * E, N, lane);
           warp_node_softmax(pr[hh], N);
         }
         __syncwarp();
@@ -257,51 +279,12 @@ __global__ void __launch_bounds__(NT, 1) k_decoder_bwd(const DecBwdParams p) {
       }
 
       // ---------------- B5: d m_t[k][e] += sum_m c[m][k] dq^[m][e]     (1024 x 128 outputs, K = 32)
-      // Tensor pipe: A fragment (row k, col m) = c[m][k] read from QC, B fragment (row m, col e) = dq^[m][e] from DQ;
-      // warp w owns rows [64w, 64w + 64) of d m_t.
-      {
-        const int g = lane >> 2, t4 = lane & 3;
-        for (int mt = 0; mt < 4; ++mt) {
+      // warp w owns rows [64w, 64w + 64) of d m_t
+      for (int mt = 0; mt < 4; ++mt)
+        for (int nh = 0; nh < 2; ++nh) {
           const int k0 = warp * 64 + mt * 16;
-          uint32_t ah[TM / 8][4], al[TM / 8][4];
-#pragma unroll
-          for (int ks = 0; ks < TM / 8; ++ks) {
-            const float* r0 = QC + (ks * 8 + t4) * QC_LD + k0 + g;
-            const float* r1 = r0 + 4 * QC_LD;
-            split_tf32(r0[0], ah[ks][0], al[ks][0]);
-            split_tf32(r0[8], ah[ks][1], al[ks][1]);
-            split_tf32(r1[0], ah[ks][2], al[ks][2]);
-            split_tf32(r1[8], ah[ks][3], al[ks][3]);
-          }
-#pragma unroll
-          for (int nh = 0; nh < 2; ++nh) {
-            float acc[8][4];
-#pragma unroll
-            for (int j = 0; j < 8; ++j)
-#pragma unroll
-              for (int i = 0; i < 4; ++i) acc[j][i] = 0.f;
-#pragma unroll
-            for (int ks = 0; ks < TM / 8; ++ks) {
-              const float* b0p = DQ + (ks * 8 + t4) * XS_LD + nh * 64 + g;
-#pragma unroll
-              for (int j = 0; j < 8; ++j) {
-                uint32_t bh0, bl0, bh1, bl1;
-                split_tf32(b0p[8 * j], bh0, bl0);
-                split_tf32(b0p[4 * XS_LD + 8 * j], bh1, bl1);
-                mma_tf32_16x8x8(acc[j], al[ks], bh0, bh1);
-                mma_tf32_16x8x8(acc[j], ah[ks], bl0, bl1);
-                mma_tf32_16x8x8(acc[j], ah[ks], bh0, bh1);
-              }
-            }
-#pragma unroll
-            for (int j = 0; j < 8; ++j) {
-              float* dst = p.d_m_t + (size_t)(k0 + g) * E + nh * 64 + 8 * j + 2 * t4;
-              red_add2(dst, acc[j][0], acc[j][1]);
-              red_add2(dst + 8 * E, acc[j][2], acc[j][3]);
-            }
-          }
+          warp_outer_product_tm(QC + k0, QC_LD, DQ + nh * 64, XS_LD, p.d_m_t + (size_t)k0 * E + nh * 64, E, lane);
         }
-      }
       __syncthreads();
 
       // ---------------- B6: dc = dq^ · M  -> QC (c is dead now)
@@ -417,45 +400,10 @@ __global__ void __launch_bounds__(NT, 1) k_decoder_bwd(const DecBwdParams p) {
 
       if (t > 0) {
         // ---------------- B8: d al_t[j][c] += sum_m x_l[m][j] dq~[m][c]     (128 x 1024 outputs, K = 32)
-        // Tensor pipe: A fragment (row j, col m) = x_l[m][j] from Xs, B fragment (row m, col c) = dq~[m][c] from QC;
-        // warp w owns columns [64w, 64w + 64) of d al_t, looping over the eight 16-row j tiles.
-        {
-          const int g = lane >> 2, t4 = lane & 3;
-          for (int mt = 0; mt < 8; ++mt) {
-            const int j0 = mt * 16;
-            float acc[8][4];
-#pragma unroll
-            for (int j = 0; j < 8; ++j)
-#pragma unroll
-              for (int i = 0; i < 4; ++i) acc[j][i] = 0.f;
-#pragma unroll
-            for (int ks = 0; ks < TM / 8; ++ks) {
-              uint32_t ah[4], al[4];
-              const float* r0 = Xs + (ks * 8 + t4) * XS_LD + j0 + g;
-              const float* r1 = r0 + 4 * XS_LD;
-              split_tf32(r0[0], ah[0], al[0]);
-              split_tf32(r0[8], ah[1], al[1]);
-              split_tf32(r1[0], ah[2], al[2]);
-              split_tf32(r1[8], ah[3], al[3]);
-              const float* b0p = QC + (ks * 8 + t4) * QC_LD + warp * 64 + g;
-#pragma unroll
-              for (int j = 0; j < 8; ++j) {
-                uint32_t bh0, bl0, bh1, bl1;
-                split_tf32(b0p[8 * j], bh0, bl0);
-                split_tf32(b0p[4 * QC_LD + 8 * j], bh1, bl1);
-                mma_tf32_16x8x8(acc[j], al, bh0, bh1);
-                mma_tf32_16x8x8(acc[j], ah, bl0, bl1);
-                mma_tf32_16x8x8(acc[j], ah, bh0, bh1);
-              }
-            }
-#pragma unroll
-            for (int j = 0; j < 8; ++j) {
-              float* dst = p.d_al_t + (size_t)(j0 + g) * QW + warp * 64 + 8 * j + 2 * t4;
-              red_add2(dst, acc[j][0], acc[j][1]);
-              red_add2(dst + 8 * QW, acc[j][2], acc[j][3]);
-            }
-          }
-        }
+        // warp w owns columns [64w, 64w + 64) of d al_t, looping over the eight 16-row j tiles
+        for (int mt = 0; mt < 8; ++mt)
+          warp_outer_product_tm(Xs + mt * 16, XS_LD, QC + warp * 64, QC_LD, p.d_al_t + (size_t)(mt * 16) * QW + warp * 64,
+                                QW, lane);
         __syncthreads();
         // ---------------- B9: dx_l = dq~ · A_l -> DQ, then dH[b, last] += dx_l
         tile_gemm_tall_mma_sw<2, 4, 4>(QC, QC_LD, p.al_n, Wb, nullptr, Wb, DQ, XS_LD);
@@ -531,16 +479,6 @@ __global__ void __launch_bounds__(256) k_gemm_tn_atomic(const float* __restrict_
 //   B fragment (k = t / t+4, n = g)        = Bm[r0 + t (+4)][n0 + g]
 constexpr int TN_LD = 64 + 8;   // (8t + g) % 32 distinct banks for both fragment patterns
 
-__device__ __forceinline__ void tn_split(float x, uint32_t& hi, uint32_t& lo) {
-  hi = __float_as_uint(x) & 0xffffe000u;
-  lo = __float_as_uint(x - __uint_as_float(hi));
-}
-__device__ __forceinline__ void tn_mma(float (&c)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
-  asm volatile("mma.sync.aligned.m16n8k8.row.col.f32.tf32.tf32.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-               : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
-               : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
-
 __global__ void __launch_bounds__(128) k_gemm_tn_mma(const float* __restrict__ A, const float* __restrict__ Bm,
                                                       float* __restrict__ C, int64_t R, int M, int N,
                                                       int64_t rows_per_cta) {
@@ -587,19 +525,19 @@ __global__ void __launch_bounds__(128) k_gemm_tn_mma(const float* __restrict__ A
     for (int ks = 0; ks < 4; ++ks) {
       uint32_t ah[4], al[4];
       const float* ap = &As[buf][ks * 8 + t][warp * 16 + g];
-      tn_split(ap[0], ah[0], al[0]);               // (m = g,   k = t)
-      tn_split(ap[8], ah[1], al[1]);               // (m = g+8, k = t)
-      tn_split(ap[4 * TN_LD], ah[2], al[2]);       // (m = g,   k = t+4)
-      tn_split(ap[4 * TN_LD + 8], ah[3], al[3]);   // (m = g+8, k = t+4)
+      split_tf32(ap[0], ah[0], al[0]);               // (m = g,   k = t)
+      split_tf32(ap[8], ah[1], al[1]);               // (m = g+8, k = t)
+      split_tf32(ap[4 * TN_LD], ah[2], al[2]);       // (m = g,   k = t+4)
+      split_tf32(ap[4 * TN_LD + 8], ah[3], al[3]);   // (m = g+8, k = t+4)
       const float* bp = &Bs[buf][ks * 8 + t][g];
 #pragma unroll
       for (int j = 0; j < 8; ++j) {
         uint32_t bh0, bl0, bh1, bl1;
-        tn_split(bp[8 * j], bh0, bl0);
-        tn_split(bp[4 * TN_LD + 8 * j], bh1, bl1);
-        tn_mma(acc[j], al, bh0, bh1);
-        tn_mma(acc[j], ah, bl0, bl1);
-        tn_mma(acc[j], ah, bh0, bh1);
+        split_tf32(bp[8 * j], bh0, bl0);
+        split_tf32(bp[4 * TN_LD + 8 * j], bh1, bl1);
+        mma_tf32_16x8x8(acc[j], al, bh0, bh1);
+        mma_tf32_16x8x8(acc[j], ah, bl0, bl1);
+        mma_tf32_16x8x8(acc[j], ah, bh0, bh1);
       }
     }
     __syncthreads();
@@ -626,21 +564,15 @@ __global__ void __launch_bounds__(256) k_colsum_atomic(const float* __restrict__
   }
 }
 
-// Per-episode decoder terms: G[b] = mean_n h[b,n]; Xf[b] = h[b, tape[0][b]]   (one warp per instance)
+// Per-episode decoder terms: G[b] = mean_n h[b,n]; Xf[b] = h[b, tape[0][b]] unless Xf is NULL   (one warp per instance)
 __global__ void __launch_bounds__(256) k_episode_gather(const float* __restrict__ h, const uint8_t* __restrict__ tape,
                                                          int64_t B, int N, float* __restrict__ G, float* __restrict__ Xf) {
   const int64_t b = (int64_t)blockIdx.x * 8 + (threadIdx.x >> 5);
   const int lane = threadIdx.x & 31;
   if (b >= B) return;
-  const float4* hp = reinterpret_cast<const float4*>(h + b * N * E) + lane;
-  float4 g = make_float4(0.f, 0.f, 0.f, 0.f);
-  for (int n = 0; n < N; ++n) {
-    float4 v = __ldg(hp + n * (E / 4));
-    g.x += v.x; g.y += v.y; g.z += v.z; g.w += v.w;
-  }
-  const float inv = 1.0f / (float)N;
-  reinterpret_cast<float4*>(G + b * E)[lane] = make_float4(g.x * inv, g.y * inv, g.z * inv, g.w * inv);
-  if (Xf) reinterpret_cast<float4*>(Xf + b * E)[lane] = __ldg(hp + (int)tape[b] * (E / 4));
+  reinterpret_cast<float4*>(G + b * E)[lane] = warp_graph_mean(h, b, N, lane);
+  if (Xf)
+    reinterpret_cast<float4*>(Xf + b * E)[lane] = __ldg(reinterpret_cast<const float4*>(h + (b * N + (int)tape[b]) * E) + lane);
 }
 
 // dH[b,n] += dG[b] / N for every n;  dH[b, tape[0][b]] += dXf[b]
@@ -669,6 +601,13 @@ __global__ void __launch_bounds__(256) k_episode_scatter(float* __restrict__ dH,
 static int g_tn_path = 0;   // vrpx_debug_gemm_tn_path
 
 namespace vrpx {
+int launch_episode_gather(const float* h, const uint8_t* tape0, int64_t B, int N, float* G, float* Xf,
+                          cudaStream_t stream) {
+  k_episode_gather<<<(unsigned)((B + 7) / 8), 256, 0, stream>>>(h, tape0, B, N, G, Xf);
+  VRPX_LAUNCH_CHECK();
+  return VRPX_OK;
+}
+
 int colsum_launch(const float* X, int64_t R, int Ccols, float* out, cudaStream_t stream) {
   int64_t ctas = (R + 511) / 512;
   int64_t maxc = (int64_t)num_sms() * 8;
@@ -775,9 +714,7 @@ int vrpx_colsum_accumulate(const float* X, int64_t R, int32_t Ccols, float* out,
 int vrpx_episode_gather(const float* h, const uint8_t* tape0, int64_t B, int32_t N, float* G, float* Xf, void* stream) {
   VRPX_CHECK_ARG(h && G && B >= 1 && (Xf == nullptr || tape0 != nullptr), "bad argument");
   VRPX_DEVICE_GUARD(h);
-  k_episode_gather<<<(unsigned)((B + 7) / 8), 256, 0, (cudaStream_t)stream>>>(h, tape0, B, N, G, Xf);
-  VRPX_LAUNCH_CHECK();
-  return VRPX_OK;
+  return launch_episode_gather(h, tape0, B, N, G, Xf, (cudaStream_t)stream);
 }
 
 int vrpx_episode_scatter(float* dH, const uint8_t* tape0, int64_t B, int32_t N, const float* dG, const float* dXf,

@@ -72,6 +72,15 @@ __device__ __forceinline__ void warp_glimpse_scores(const float* q, const float4
   }
 }
 
+// One head's scores src[n] in the layout of warp_node_softmax: x[i] = node lane + 32 i, -inf for nodes >= N
+__device__ __forceinline__ void warp_load_by_head(float (&x)[4], const float* src, int N, int lane) {
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const int n = lane + 32 * i;
+    x[i] = (n < N) ? src[n] : -INFINITY;
+  }
+}
+
 // Softmax of one head's scores over the nodes, in place: x[i] holds node lane + 32 i (lane = node, 4 strides cover
 // N <= 128), -inf for nodes >= N.  The exponential is evaluated only in the ceil(N / 32) strides that hold nodes: in them
 // a lane beyond N gets exp(-inf) = 0, and a stride without nodes is 0 without it, so the result is bit for bit what

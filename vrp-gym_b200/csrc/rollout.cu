@@ -71,19 +71,9 @@ __global__ void __launch_bounds__(NT, 1) k_rollout(const RolloutParams p) {
   for (int64_t tile = blockIdx.x; tile < ntiles && p.t0 == 0; tile += gridDim.x) {
     const int64_t base = tile * RTM;
     const int cnt = (int)((B - base < RTM) ? (B - base) : RTM);
-    for (int m = warp; m < RTM; m += NT / 32) {
-      float4 g = make_float4(0.f, 0.f, 0.f, 0.f);
-      if (m < cnt) {
-        const float4* hp = reinterpret_cast<const float4*>(h + (base + m) * N * E) + lane;
-        for (int n = 0; n < N; ++n) {
-          float4 v = __ldg(hp + n * (E / 4));
-          g.x += v.x; g.y += v.y; g.z += v.z; g.w += v.w;
-        }
-        float inv = 1.0f / (float)N;
-        g.x *= inv; g.y *= inv; g.z *= inv; g.w *= inv;
-      }
-      *reinterpret_cast<float4*>(Xs + m * XS_LD + lane * 4) = g;
-    }
+    for (int m = warp; m < RTM; m += NT / 32)
+      *reinterpret_cast<float4*>(Xs + m * XS_LD + lane * 4) =
+          (m < cnt) ? warp_graph_mean(h, base + m, N, lane) : make_float4(0.f, 0.f, 0.f, 0.f);
     __syncthreads();
     tile_gemm_wide_mma_sw<RMT, RNST>(                                              // Q~g = A_g · g + a_c
         Xs, XS_LD, p.w.ag_t, Wb, [&](int, int c) { return *reinterpret_cast<const float2*>(p.w.a_c + c); },
@@ -131,19 +121,15 @@ __global__ void __launch_bounds__(NT, 1) k_rollout(const RolloutParams p) {
         *reinterpret_cast<float4*>(Xs + m * XS_LD + lane * 4) = xv;
         const float lf = (m < cnt) ? (float)p.env.load[base + m] : 0.f;
         if (lane == 0) s_loadf[m] = lf;
-        if (m < cnt && p.mask_hist && lane < 4)
-          p.mask_hist[((int64_t)trel * B + base + m) * 4 + lane] = __ldcg(p.env.mask + (base + m) * 4 + lane);
-        if (m < cnt && p.load_hist && lane == 0) p.load_hist[(int64_t)trel * B + base + m] = lf;
+        if (m < cnt) record_trace(p, base + m, trel, lf, lane);
       }
       __syncthreads();
       VRPX_PROF(0)
       // ---------------- P1: q~
       if (t == 0) {
         for (int o = tid; o < cnt * QW; o += NT) {
-          int m = o >> 10, c = o & (QW - 1);
-          float y = p.qg[(base + m) * QW + c] + p.w.a_q0[c];
-          if (kind == VRPX_IRP) y = fmaf(s_loadf[m], p.w.a_load[c], y);
-          QC[m * RQ_LD + c] = y;
+          const int m = o >> 10, c = o & (QW - 1);
+          QC[m * RQ_LD + c] = step0_query(p.qg + (base + m) * QW, p.w.a_q0, p.w.a_load, kind == VRPX_IRP, s_loadf[m], c);
         }
       } else {
         if (t == 1 && kind != VRPX_IRP) {
@@ -159,14 +145,8 @@ __global__ void __launch_bounds__(NT, 1) k_rollout(const RolloutParams p) {
         tile_gemm_wide_mma_sw<RMT, RNST>(                                          // q~ = Q~g (+ load · a_load) + A_l · h[last]
             Xs, XS_LD, p.w.al_t, Wb,
             [&](int m, int c) {
-              if (m >= cnt) return make_float2(0.f, 0.f);
-              float2 q = *reinterpret_cast<const float2*>(p.qg + (base + m) * QW + c);
-              if (kind == VRPX_IRP) {
-                const float2 al = *reinterpret_cast<const float2*>(p.w.a_load + c);
-                const float lf = s_loadf[m];
-                q = make_float2(fmaf(lf, al.x, q.x), fmaf(lf, al.y, q.y));
-              }
-              return q;
+              return (m < cnt) ? glimpse_query_init(p.qg + (base + m) * QW, p.w.a_load, kind == VRPX_IRP, s_loadf[m], c)
+                               : make_float2(0.f, 0.f);
             },
             [&](int m, int c, float v0, float v1) { *reinterpret_cast<float2*>(QC + m * RQ_LD + c) = make_float2(v0, v1); });
       }
@@ -180,7 +160,6 @@ __global__ void __launch_bounds__(NT, 1) k_rollout(const RolloutParams p) {
         const int tq = lane & 3;
         const float4* hrow = reinterpret_cast<const float4*>(h + b * N * E);
         // ---- pass 1: scores = q~_h · h_n + scrambled additive mask
-        // masks of the instances whose rows the reference adds to heads 2tq and 2tq+1 (mask.repeat(H,1), graph_decoder.py:93)
         uint32_t nb0[4], nb1[4];
         {
           const uint32_t* m0 = gm_rd + quirk_row(b, 2 * tq, p.G) * 4;
@@ -196,14 +175,10 @@ __global__ void __launch_bounds__(NT, 1) k_rollout(const RolloutParams p) {
         VRPX_PROF(6)
         float pr[NH][4];
 #pragma unroll
-        for (int hh = 0; hh < NH; ++hh)
-#pragma unroll
-          for (int i = 0; i < 4; ++i) {
-            const int n = lane + 32 * i;
-            pr[hh][i] = (n < N) ? slot[hh * E + n] : -INFINITY;
-          }
-#pragma unroll
-        for (int hh = 0; hh < NH; ++hh) warp_node_softmax(pr[hh], N);
+        for (int hh = 0; hh < NH; ++hh) {
+          warp_load_by_head(pr[hh], slot + hh * E, N, lane);
+          warp_node_softmax(pr[hh], N);
+        }
         __syncwarp();
         warp_store_by_node(slot, pr, N, lane);
         __syncwarp();
@@ -250,17 +225,11 @@ __global__ void __launch_bounds__(NT, 1) k_rollout(const RolloutParams p) {
           }
         }
         __syncwarp();
-        // own mask (graph_decoder.py:98), 4 consecutive nodes per lane
         uint32_t mw[4];
 #pragma unroll
         for (int i = 0; i < 4; ++i) mw[i] = __ldcg(p.env.mask + b * 4 + i);
         float u[4];
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-          int n = lane * 4 + i;
-          bool ok = n < N && !((mw[n >> 5] >> (n & 31)) & 1u);
-          u[i] = ok ? slot[n] : -INFINITY;
-        }
+        warp_masked_logits(u, slot, mw, N, lane, false);
         const PointerChoice c = warp_pointer_choice(u, p, b, t, trel, lane);
         if (lane == 0) { s_act[m] = c.a; s_lp[m] = c.lp; }
       }
@@ -445,30 +414,11 @@ int vrpx_rollout(const vrpx_env* env, const vrpx_decoder_weights* w, const float
   VRPX_CHECK_ARG((int64_t)(Tmax + 1 + 8) * 4 <= kRolloutSmall, "Tmax too large for workspace header");
 
   VRPX_CUDA(cudaMemsetAsync(ws, 0, kRolloutSmall, stream));
-  if (split) {
-    if (g_time_kernel) {
-      if (!g_ev0) {
-        VRPX_CUDA(cudaEventCreate(&g_ev0));
-        VRPX_CUDA(cudaEventCreate(&g_ev1));
-      }
-      VRPX_CUDA(cudaEventRecord(g_ev0, stream));
-    }
-    NvtxRange nvtx_decode("vrpx:decode_loop");
-    int rc = run_first_steps(p, sw, plan_b, stream);
-    if (rc) return rc;
-    if ((rc = run_split_steps(p, t_begin + 2, plan_b, stream))) return rc;   // also writes the step count
-    if (g_time_kernel) {
-      VRPX_CUDA(cudaEventRecord(g_ev1, stream));
-      g_ev_valid = true;
-    }
-    return VRPX_OK;
+  if (!split) {
+    k_split_m16<<<(QW / 2) * E / 256, 256, 0, stream>>>(w->m_t, reinterpret_cast<uint2*>(reinterpret_cast<char*>(ws) + kRolloutSmall));
+    VRPX_LAUNCH_CHECK();
+    VRPX_CUDA(cudaFuncSetAttribute(k_rollout, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_TOTAL));
   }
-  k_split_m16<<<(QW / 2) * E / 256, 256, 0, stream>>>(w->m_t, reinterpret_cast<uint2*>(reinterpret_cast<char*>(ws) + kRolloutSmall));
-  VRPX_LAUNCH_CHECK();
-  VRPX_CUDA(cudaFuncSetAttribute(k_rollout, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_TOTAL));
-  int64_t ntiles = (env->B + RTM - 1) / RTM;
-  int grid = (int)((ntiles < (int64_t)num_sms()) ? ntiles : (int64_t)num_sms());
-  void* args[] = {(void*)&p};
   if (g_time_kernel) {
     if (!g_ev0) {
       VRPX_CUDA(cudaEventCreate(&g_ev0));
@@ -477,8 +427,17 @@ int vrpx_rollout(const vrpx_env* env, const vrpx_decoder_weights* w, const float
     VRPX_CUDA(cudaEventRecord(g_ev0, stream));
   }
   NvtxRange nvtx_decode("vrpx:decode_loop");
-  VRPX_CUDA(cudaLaunchCooperativeKernel((void*)k_rollout, dim3(grid), dim3(NT), args, SMEM_TOTAL, stream));
-  count_launch();
+  if (split) {
+    int rc = run_first_steps(p, sw, plan_b, stream);
+    if (rc) return rc;
+    if ((rc = run_split_steps(p, t_begin + 2, plan_b, stream))) return rc;   // also writes the step count
+  } else {
+    int64_t ntiles = (env->B + RTM - 1) / RTM;
+    int grid = (int)((ntiles < (int64_t)num_sms()) ? ntiles : (int64_t)num_sms());
+    void* args[] = {(void*)&p};
+    VRPX_CUDA(cudaLaunchCooperativeKernel((void*)k_rollout, dim3(grid), dim3(NT), args, SMEM_TOTAL, stream));
+    count_launch();
+  }
   if (g_time_kernel) {
     VRPX_CUDA(cudaEventRecord(g_ev1, stream));
     g_ev_valid = true;

@@ -1,5 +1,6 @@
-// rollout.cuh — parameter block and the per-instance end of a decode step (action choice, environment step), shared by
-// the persistent rollout kernel (rollout.cu) and the split-step kernels (rollout_steps.cu).
+// rollout.cuh — parameter block and the per-instance parts of a decode step outside the glimpse (graph mean, query,
+// masked pointer logits, action choice, environment step), shared by the persistent rollout kernel (rollout.cu), the
+// split-step kernels (rollout_steps.cu) and the recompute of the REINFORCE backward (decoder_bwd.cu).
 #pragma once
 #include "gemm.cuh"
 #include "tile_gemm.cuh"
@@ -54,9 +55,61 @@ struct SplitWorkspace {
 int prepare_split_weights(const RolloutParams& p, const SplitWorkspace& w, GemmPlan* plan_b, cudaStream_t stream);
 int run_first_steps(const RolloutParams& p, const SplitWorkspace& w, const GemmPlan& plan_b, cudaStream_t stream);
 int run_split_steps(const RolloutParams& p, int t_first, const GemmPlan& plan_b, cudaStream_t stream);
+// decoder_bwd.cu: G[b] = mean_n h[b, n] (warp_graph_mean) and, unless Xf is NULL, Xf[b] = h[b, tape0[b]]
+int launch_episode_gather(const float* h, const uint8_t* tape0, int64_t B, int N, float* G, float* Xf, cudaStream_t stream);
 
-// ---------------------------------------------------------------- the end of a decode step, after the pointer logits
+// G[b] = mean_n h[b, n] (graph_decoder.py:75-77), one warp per instance: lane l returns dims 4l .. 4l+3
+__device__ __forceinline__ float4 warp_graph_mean(const float* __restrict__ h, int64_t b, int N, int lane) {
+  const float4* hp = reinterpret_cast<const float4*>(h + b * N * E) + lane;
+  float4 g = make_float4(0.f, 0.f, 0.f, 0.f);
+  for (int n = 0; n < N; ++n) {
+    const float4 v = __ldg(hp + n * (E / 4));
+    g.x += v.x; g.y += v.y; g.z += v.z; g.w += v.w;
+  }
+  const float inv = 1.0f / (float)N;
+  return make_float4(g.x * inv, g.y * inv, g.z * inv, g.w * inv);
+}
+
+// ---------------------------------------------------------------- the folded glimpse query q~ of one instance
+// qg = the instance's Q~g row, lf = its vehicle load as f32; the load term a_load exists for IRP only.
+// Step 0 (graph_decoder.py:79-81), dim c: the learned placeholder a_q0 takes the place of A_l h[last]
+__device__ __forceinline__ float step0_query(const float* qg, const float* a_q0, const float* a_load, bool irp, float lf,
+                                             int c) {
+  const float y = qg[c] + a_q0[c];
+  return irp ? fmaf(lf, a_load[c], y) : y;
+}
+// Steps >= 1, dims c, c+1: Q~g (+ lf · a_load), the initial accumulators of the GEMM-A tile q~ = that + A_l h[last]
+__device__ __forceinline__ float2 glimpse_query_init(const float* qg, const float* a_load, bool irp, float lf, int c) {
+  float2 q = *reinterpret_cast<const float2*>(qg + c);
+  if (irp) {
+    const float2 al = *reinterpret_cast<const float2*>(a_load + c);
+    q = make_float2(fmaf(lf, al.x, q.x), fmaf(lf, al.y, q.y));
+  }
+  return q;
+}
+
+// Write the trace the backward replays (RolloutParams::mask_hist / load_hist) for instance b before step trel
+__device__ __forceinline__ void record_trace(const RolloutParams& p, int64_t b, int trel, float lf, int lane) {
+  if (p.mask_hist && lane < 4) p.mask_hist[((int64_t)trel * p.env.B + b) * 4 + lane] = __ldcg(p.env.mask + b * 4 + lane);
+  if (p.load_hist && lane == 0) p.load_hist[(int64_t)trel * p.env.B + b] = lf;
+}
+
+// ---------------------------------------------------------------- the pointer phase: logits, action, environment step
 // (phase P4 of the persistent kernel and the split-step pointer kernel)
+
+// Masked logits u[i] of node 4 lane + i (graph_decoder.py:98): slot[n] where the own mask words mw leave node n open,
+// -inf where masked or beyond N.  `idle` (a finished instance, see instance_idle in rollout_steps.cu): its single open
+// node gets 0, which gives the same action and log-prob as any finite logit, and slot is not read.
+__device__ __forceinline__ void warp_masked_logits(float (&u)[4], const float* slot, const uint32_t (&mw)[4], int N, int lane,
+                                                   bool idle) {
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const int n = lane * 4 + i;
+    const bool ok = n < N && !((mw[n >> 5] >> (n & 31)) & 1u);
+    u[i] = ok ? (idle ? 0.f : slot[n]) : -INFINITY;
+  }
+}
+
 struct PointerChoice {
   int a;      // action
   float lp;   // its log-prob (0 in greedy mode)

@@ -12,10 +12,10 @@
 //   k_step_pointer   one warp per instance: logits 10 tanh(q^ · h_n), mask, argmax / Philox sample / teacher action,
 //                    log-prob; then one thread per instance runs the environment transition (env_rules.cuh)
 // Softmax, glimpse values and pointer phase are those of phases P2 and P4 of the persistent kernel: both call the helpers
-// of glimpse_mma.cuh (warp_node_softmax, warp_store_by_node, warp_glimpse_values_acc) and rollout.cuh
-// (warp_pointer_choice, rollout_env_step).  Against its classic loop the results differ only by the evaluation order of
-// the scores (tables) and the summation order inside GEMM-B.  The classic mode and resumed single-step calls run in the
-// persistent kernel.
+// of glimpse_mma.cuh (warp_load_by_head, warp_node_softmax, warp_store_by_node, warp_glimpse_values_acc) and rollout.cuh
+// (step0_query, record_trace, warp_masked_logits, warp_pointer_choice, rollout_env_step).  Against
+// its classic loop the results differ only by the evaluation order of the scores (tables) and the summation order inside
+// GEMM-B.  The classic mode and resumed single-step calls run in the persistent kernel.
 // The launches are asynchronous on the caller's stream: no host round trip per step.  An episode that finishes early
 // (VRP / IRP) turns the remaining launches into no-ops through the per-step `notdone` counters.
 #include "gemm.cuh"
@@ -50,13 +50,10 @@ __device__ __forceinline__ bool episode_over(const RolloutParams& p, int trel) {
 // "the depot is the only candidate while cur == depot" is exactly "finished".)
 __device__ __forceinline__ bool instance_idle(const uint32_t (&own)[4], int N, int cur, int depot) {
   if (cur != depot) return false;
+  const Bits128 full = full_bits(N);
   int cand = 0;
 #pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    const int rem = N - 32 * i;
-    const uint32_t range = rem >= 32 ? 0xffffffffu : (rem > 0 ? ((1u << rem) - 1u) : 0u);
-    cand += __popc(~own[i] & range);
-  }
+  for (int i = 0; i < 4; ++i) cand += __popc(~own[i] & full.w[i]);
   return cand == 1 && !((own[depot >> 5] >> (depot & 31)) & 1u);
 }
 
@@ -87,8 +84,7 @@ __global__ void __launch_bounds__(GW_MAX * 32, 2) k_step_glimpse(const RolloutPa
 #pragma unroll
     for (int i = 0; i < 4; ++i) own[i] = __ldcg(p.env.mask + b * 4 + i);
     if (instance_idle(own, N, __ldcg(p.env.cur + b), __ldg(p.env.depot + b))) {
-      if (p.mask_hist && lane < 4) p.mask_hist[((int64_t)trel * B + b) * 4 + lane] = __ldcg(p.env.mask + b * 4 + lane);
-      if (p.load_hist && lane == 0) p.load_hist[(int64_t)trel * B + b] = (float)p.env.load[b];
+      record_trace(p, b, trel, (float)p.env.load[b], lane);
       return;
     }
   }
@@ -98,8 +94,7 @@ __global__ void __launch_bounds__(GW_MAX * 32, 2) k_step_glimpse(const RolloutPa
     else cp_async_commit();
   }
   const float lf = (float)p.env.load[b];
-  if (p.mask_hist && lane < 4) p.mask_hist[((int64_t)trel * B + b) * 4 + lane] = __ldcg(p.env.mask + b * 4 + lane);
-  if (p.load_hist && lane == 0) p.load_hist[(int64_t)trel * B + b] = lf;
+  record_trace(p, b, trel, lf, lane);
 
   // ---- scores = S1[b][last] + S0[b] (+ load · SL[b]) + scrambled additive mask (graph_decoder.py:93-94)
   float pr[NH][4];
@@ -193,15 +188,14 @@ __global__ void __launch_bounds__(SW * 32) k_step_pointer(const RolloutParams p,
     const float4* hp = reinterpret_cast<const float4*>(p.h + b * N * E) + lane;
     // own mask (graph_decoder.py:98).  The logits of masked nodes are never used (they become -inf below), so only the
     // embedding rows of the CANDIDATE nodes are read: on average half of the instance over an episode.
+    const Bits128 full = full_bits(N);
     uint32_t mw[4], cand[4];
     int cum[5];
     cum[0] = 0;
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
       mw[i] = __ldcg(p.env.mask + b * 4 + i);
-      const int rem = N - 32 * i;   // nodes of this word
-      const uint32_t range = rem >= 32 ? 0xffffffffu : (rem > 0 ? ((1u << rem) - 1u) : 0u);
-      cand[i] = ~mw[i] & range;
+      cand[i] = ~mw[i] & full.w[i];
       cum[i + 1] = cum[i] + __popc(cand[i]);
     }
     // idle finished instance (see instance_idle): the depot is the only candidate and nobody reads its logit
@@ -258,12 +252,7 @@ __global__ void __launch_bounds__(SW * 32) k_step_pointer(const RolloutParams p,
     }
     __syncwarp();
     float u[4];
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      const int n = lane * 4 + i;
-      const bool ok = n < N && !((mw[n >> 5] >> (n & 31)) & 1u);
-      u[i] = ok ? (idle ? 0.f : slot[n]) : -INFINITY;   // idle: one candidate, any finite logit gives action = depot, log-prob 0
-    }
+    warp_masked_logits(u, slot, mw, N, lane, idle);
     const PointerChoice c = warp_pointer_choice(u, p, b, t, trel, lane);
     if (lane == 0) { s_act[warp] = c.a; s_lp[warp] = c.lp; }
   }
@@ -280,24 +269,10 @@ __global__ void __launch_bounds__(SW * 32) k_step_pointer(const RolloutParams p,
 // The first two steps have no table row yet: step 0 runs on the learned placeholders (q~ = Q~g + a_q0, graph_decoder.py:79-81),
 // step 1 completes the per-episode tables (Q~g += A_f h[first]; S0 = Q~g_head · h_n; IRP: SL = a_load_head · h_n).  They
 // used to run inside the persistent kernel (4.7 ms at C4, L2-bound on 16-instance tiles); here they are whole-batch
-// launches like every later step: a mean / gather kernel, a batched tcgen05 GEMM for the 128 -> 1024 query fold, and a
-// glimpse kernel that computes the scores from q~ itself (one warp per instance, mma.sync TF32 3-term: the score and value
-// contractions of glimpse_mma.cuh) instead of reading them from the tables.
-
-// G[b] = mean_n h[b, n]  (graph_decoder.py:75-77), one warp per instance
-__global__ void __launch_bounds__(256) k_episode_mean(const float* __restrict__ h, int64_t B, int N, float* __restrict__ G) {
-  const int lane = threadIdx.x & 31;
-  const int64_t b = (int64_t)blockIdx.x * 8 + (threadIdx.x >> 5);
-  if (b >= B) return;
-  const float4* hp = reinterpret_cast<const float4*>(h + b * N * E) + lane;
-  float4 g = make_float4(0.f, 0.f, 0.f, 0.f);
-  for (int n = 0; n < N; ++n) {   // same summation order as the persistent kernel's prologue
-    const float4 v = __ldg(hp + n * (E / 4));
-    g.x += v.x; g.y += v.y; g.z += v.z; g.w += v.w;
-  }
-  const float inv = 1.0f / (float)N;
-  reinterpret_cast<float4*>(G + b * E)[lane] = make_float4(g.x * inv, g.y * inv, g.z * inv, g.w * inv);
-}
+// launches like every later step: a mean / gather kernel (k_episode_gather in decoder_bwd.cu, k_gather_cur), a batched
+// tcgen05 GEMM for the 128 -> 1024 query fold, and a glimpse kernel that computes the scores from q~ itself (one warp per
+// instance, mma.sync TF32 3-term: the score and value contractions of glimpse_mma.cuh) instead of reading them from the
+// tables.
 
 // Xf[b] = h[b, cur[b]]: the first chosen node after step 0 (graph_decoder.py:108-113)
 __global__ void __launch_bounds__(256) k_gather_cur(const float* __restrict__ h, const int* __restrict__ cur, int64_t B, int N,
@@ -330,23 +305,12 @@ __global__ void __launch_bounds__(FW * 32, 2) k_step_glimpse_first(const Rollout
   const int tq = lane & 3;
   const float4* hrow = reinterpret_cast<const float4*>(p.h + b * N * E);
   const float lf = (float)p.env.load[b];
-  if (p.mask_hist && lane < 4) p.mask_hist[((int64_t)trel * B + b) * 4 + lane] = __ldcg(p.env.mask + b * 4 + lane);
-  if (p.load_hist && lane == 0) p.load_hist[(int64_t)trel * B + b] = lf;
+  record_trace(p, b, trel, lf, lane);
   // ---- q~: step 0 = Q~g + a_q0 (+ load · a_load); step 1 = the finished Q~g (its scores are S0, kept for every later step)
   {
-    const float4* qg4 = reinterpret_cast<const float4*>(p.qg + b * QW);
-    for (int i = lane; i < QW / 4; i += 32) {
-      float4 q = __ldcg(qg4 + i);
-      if (t == 0) {
-        const float4 a0 = __ldg(reinterpret_cast<const float4*>(p.w.a_q0) + i);
-        q.x += a0.x; q.y += a0.y; q.z += a0.z; q.w += a0.w;
-        if (kind == VRPX_IRP) {
-          const float4 al = __ldg(reinterpret_cast<const float4*>(p.w.a_load) + i);
-          q.x = fmaf(lf, al.x, q.x); q.y = fmaf(lf, al.y, q.y); q.z = fmaf(lf, al.z, q.z); q.w = fmaf(lf, al.w, q.w);
-        }
-      }
-      *reinterpret_cast<float4*>(slot + 4 * i) = q;
-    }
+    const float* qg = p.qg + b * QW;
+    for (int c = lane; c < QW; c += 32)
+      slot[c] = (t == 0) ? step0_query(qg, p.w.a_q0, p.w.a_load, kind == VRPX_IRP, lf, c) : qg[c];
   }
   __syncwarp();
   float* s0 = (t == 1) ? p.s0 + (size_t)b * NH * N : nullptr;
@@ -357,12 +321,7 @@ __global__ void __launch_bounds__(FW * 32, 2) k_step_glimpse_first(const Rollout
   __syncwarp();
   float pr[NH][4];
 #pragma unroll
-  for (int hh = 0; hh < NH; ++hh)
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      const int n = lane + 32 * i;
-      pr[hh][i] = (n < N) ? slot[hh * E + n] : -INFINITY;
-    }
+  for (int hh = 0; hh < NH; ++hh) warp_load_by_head(pr[hh], slot + hh * E, N, lane);
   __syncwarp();
   if (t == 1) {
     if (kind == VRPX_IRP) {   // SL = a_load_head · h_n, and its share of this step's scores
@@ -425,15 +384,8 @@ __global__ void k_rollout_finish(const int* __restrict__ notdone, int t0, int Tm
   *steps = t;
 }
 
-__global__ void k_transpose_m(const float* __restrict__ m_t, float* __restrict__ m_nt) {   // [1024][128] -> [128][1024]
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= QW * E) return;
-  const int k = i >> 7, n = i & (E - 1);
-  m_nt[n * QW + k] = m_t[i];
-}
-
 int prepare_split_weights(const RolloutParams& p, const SplitWorkspace& w, GemmPlan* plan_b, cudaStream_t stream) {
-  k_transpose_m<<<QW * E / 256, 256, 0, stream>>>(p.w.m_t, w.m_nt);
+  k_transpose<<<QW * E / 256, 256, 0, stream>>>(p.w.m_t, QW, E, w.m_nt);
   VRPX_LAUNCH_CHECK();
   k_transpose<<<QW * E / 256, 256, 0, stream>>>(p.w.ag_t, E, QW, w.ag_n);
   VRPX_LAUNCH_CHECK();
@@ -461,8 +413,7 @@ int run_first_steps(const RolloutParams& p, const SplitWorkspace& w, const GemmP
   const unsigned g8 = (unsigned)((B + 7) / 8), grid_p = (unsigned)((B + SW - 1) / SW), grid_f = (unsigned)((B + FW - 1) / FW);
   int rc;
   // ---- step 0: Q~g = A_g · mean_n h + a_c (the graph part of the folded query), then the placeholder step
-  k_episode_mean<<<g8, 256, 0, stream>>>(p.h, B, N, p.qhat);
-  VRPX_LAUNCH_CHECK();
+  if ((rc = launch_episode_gather(p.h, nullptr, B, N, p.qhat, nullptr, stream))) return rc;
   GemmArgs g0{p.qhat, B, E, w.ag_n, QW, p.w.a_c, 0, nullptr, nullptr, nullptr, p.qg};
   if ((rc = gemm_tc(g0, stream))) return rc;
   if (p.qg0) VRPX_CUDA(cudaMemcpyAsync(p.qg0, p.qg, (size_t)B * QW * sizeof(float), cudaMemcpyDeviceToDevice, stream));

@@ -10,8 +10,6 @@ namespace vrpx {
 constexpr int TM = 32;        // instances per tile
 constexpr int NT = 512;       // threads per CTA (16 warps; <= 128 registers per thread)
 constexpr int QW = NH * E;    // 1024: per-instance width of q~ / c
-constexpr size_t SMEM_X = (size_t)TM * E * sizeof(float);    // 16 KiB
-constexpr size_t SMEM_QC = (size_t)TM * QW * sizeof(float);  // 128 KiB
 constexpr size_t SMEM_W = 64 * 1024;                         // weight rings of the backward kernel: 16 warps x 2 x 2 KiB
 
 __device__ __forceinline__ unsigned ld_acquire(const unsigned* p) {
@@ -88,7 +86,6 @@ __device__ __forceinline__ int64_t quirk_row(int64_t b, int hh, long long G) {
 constexpr int XS_LD = E + 4;        // 132: A fragments (row g, col t): bank (4g + t) % 32
 constexpr int QC_LD = QW + 4;       // 1028
 template <int MT> constexpr size_t smem_x_mma() { return (size_t)(16 * MT) * XS_LD * sizeof(float); }
-template <int MT> constexpr size_t smem_qc_mma() { return (size_t)(16 * MT) * QC_LD * sizeof(float); }
 __device__ __forceinline__ void split_tf32(float x, uint32_t& hi, uint32_t& lo) {
   hi = __float_as_uint(x) & 0xffffe000u;
   lo = __float_as_uint(x - __uint_as_float(hi));

@@ -27,6 +27,7 @@ import torch
 from oracle_replay import check_logp as _check_logp
 from oracle_replay import host_inputs as _host_inputs
 from oracle_replay import partners as _partners
+from test_gpu_encoder_train import saved_stages
 
 pytestmark = pytest.mark.gpu
 
@@ -114,17 +115,16 @@ def _decoder_reference(sd, h, tape, masks, loads, partners, wts, visit):
 
 def _kernel_gate(saved, B, N):
     """relu hook for policy_oracle.encoder_forward: the float64 sign of the pre-activation decides the ReLU gate, except
-    within GATE_BAND of zero, where the f32 kernel's own saved activation F (encoder_bwd.cu: per layer l at
-    R*384 + l*R*1408 + R*768 of the saved block, [R][512]) decides.  There the sign is not determined by f32 inputs, and
-    each disagreement moves a ReLU weight gradient by ~1/sqrt(R) of its largest element: 2e-3 ... 5e-3 for a handful of
-    flips at R = 80,000 rows.  The band holds a few thousandths of a percent of the elements, so a wrong saved F stays
-    visible through the gradients that use it (dW2 = dy2^T F and the backward's own gate)."""
-    R = B * N
+    within GATE_BAND of zero, where the f32 kernel's own saved activation F of the layer (saved_stages) decides.  There
+    the sign is not determined by f32 inputs, and each disagreement moves a ReLU weight gradient by ~1/sqrt(R) of its
+    largest element: 2e-3 ... 5e-3 for a handful of flips at R = 80,000 rows.  The band holds a few thousandths of a
+    percent of the elements, so a wrong saved F stays visible through the gradients that use it (dW2 = dy2^T F and the
+    backward's own gate)."""
+    layers = saved_stages(saved, B, N)[1]
 
     def relu(pre, layer, first):
         b = pre.shape[0]
-        o = R * 384 + layer * R * 1408 + R * 768 + first * N * 512
-        on_kernel = saved[o:o + b * N * 512].view(b, N, 512) > 0
+        on_kernel = layers[layer]["f"][first * N:(first + b) * N].view(b, N, 512) > 0
         x = pre.detach()
         on = torch.where(x.abs() <= GATE_BAND * x.abs().max(), on_kernel, x > 0)
         return pre * on.to(pre.dtype)

@@ -25,7 +25,7 @@ extern "C" {
 #define VRPX_API
 #endif
 
-#define VRPX_ABI_VERSION 4
+#define VRPX_ABI_VERSION 5
 #define VRPX_MAX_NODES 128 /* visited bitmask = 4 x u32 per instance */
 #define VRPX_EMB 128       /* embedding width E (graph_tsp_agent.py:98) */
 #define VRPX_HEADS 8       /* heads (graph_tsp_agent.py:101, :55) */
@@ -254,6 +254,29 @@ VRPX_API int vrpx_rollout(const vrpx_env* env, const vrpx_decoder_weights* w, co
                  int64_t coupling, uint64_t seed, uint64_t offset, uint8_t* tape, int32_t t_begin, int32_t Tmax,
                  float* logp, float* cost, int32_t* steps, float* logits, const vrpx_rollout_trace* trace,
                  void* ws, int64_t ws_bytes, void* stream);
+
+/* K sampled episodes per instance from one set of embeddings and one score table (best-of-K decoding).
+ * The env holds Bb·K replicas in their reset state, copy-major: replica r = k·Bb + b is copy k of base instance b (same
+ * xy / depot / demand).  Copy k is bit-identical to vrpx_rollout(copy k alone, h, VRPX_SAMPLE, coupling, seed,
+ * offset + k·Bb, t_begin 0, Tmax) in table mode: tape rows, cost, log-prob and logits.  Each copy ends at its own step
+ * count; the launches run until the slowest copy is done, so `steps` is the maximum over the copies, a copy's tape rows
+ * after its own step count hold its depot and its logits rows there are not written.
+ * The embeddings h [Bb][N][128] and the score table S1 exist once per base instance: the table is built over the Bb
+ * base instances, and the decode kernels read both at the replica's base instance.  The always-sampling, whole-episode,
+ * table-mode decode loop of vrpx_rollout runs over the Bb·K replicas, the K copies of an instance on neighbouring warps.
+ *   Bb, K     base batch and sample count (K >= 1, env->B == Bb·K)
+ *   coupling  0 or a divisor of Bb (the partner rows of every copy stay inside the copy)
+ *   w         qk_w is required
+ *   tape      [Tmax][Bb·K] uint8 actions; logp, cost [Bb·K]; logits optional [Tmax][Bb·K][N]
+ *   Tmax      maximum number of steps; Tmax < 3 (TSP with N <= 3) returns VRPX_ERR_UNSUPPORTED
+ *   ws        at least vrpx_rollout_samples_workspace_bytes(kind, Bb, K, N) bytes
+ * VRPX_ERR_ARG for K < 1, env->B != Bb·K, a bad coupling, a NULL qk_w or a workspace that is too small.  No backward
+ * trace is recorded. */
+VRPX_API int64_t vrpx_rollout_samples_workspace_bytes(int32_t kind, int64_t Bb, int32_t K, int32_t N);
+VRPX_API int vrpx_rollout_samples(const vrpx_env* env, const vrpx_decoder_weights* w, const float* h, int64_t Bb,
+                                  int32_t K, int64_t coupling, uint64_t seed, uint64_t offset, uint8_t* tape, int32_t Tmax,
+                                  float* logp, float* cost, int32_t* steps, float* logits, void* ws, int64_t ws_bytes,
+                                  void* stream);
 
 /* Measurement hooks (bench.py, tools/): not part of the reference surface.
  *   vrpx_debug_rollout_profile  device buffer of 8 x int64 that accumulates per-phase cycles of thread 0 of every CTA

@@ -14,6 +14,7 @@ from __future__ import annotations
 
 import ctypes as C
 import logging
+from copy import deepcopy
 
 import numpy as np
 import torch
@@ -86,10 +87,7 @@ class GraphDecoder(nn.Module):
                 ws = None
         if ws is None:
             ws = torch.empty((nbytes,), dtype=torch.uint8, device=dev)
-        G = B if coupling is None else int(coupling)
-        if G < 0 or (G != 0 and (G > B or B % G != 0)):
-            raise ValueError(f"coupling group {G} must be 0 or a divisor of the batch size {B}: attention row (b, head) "
-                             "reads the mask of instance (8b + head) mod G of its group (graph_decoder.py:93)")
+        G = _coupling_group(coupling, B)
         trace, saved = None, None
         if save_for_backward:
             saved = {"mask_hist": torch.empty((Tmax, B, 4), dtype=torch.int32, device=dev),
@@ -113,6 +111,75 @@ class GraphDecoder(nn.Module):
             out["saved"] = saved
         if logits is not None:
             out["logits"] = logits[:T]
+        return out
+
+    def rollout_samples(self, env, h: torch.Tensor, num_samples: int, *, seed: int, offset: int = 0, coupling=None,
+                        want_logits: bool = False):
+        """K = num_samples sampled episodes of every instance from one set of embeddings (vrpx_rollout_samples).
+
+        env: device-resident TSPEnv/VRPEnv/IRPEnv of B instances in its reset state; it is left untouched (the K copies
+        run on a private copy-major replica, replica k·B + b = copy k of instance b).  h: (B,N,128) f32 CUDA embeddings.
+        Copy k is bit-identical to rollout_episode(copy of env, h, greedy=False, seed=seed, offset=offset + k·B,
+        coupling=coupling).  All copies run until the slowest is done; a finished VRP/IRP copy idles on its depot.
+        Returns dict(cost (K,B) f32, logp (K,B) f32, steps int = max over copies, tape (steps,K,B) uint8
+        [, logits (steps,K,B,N)])."""
+        K = int(num_samples)
+        if K < 1:
+            raise ValueError(f"num_samples must be at least 1, got {num_samples}")
+        dev = env._device
+        B, N, kind = env.batch_size, env.num_nodes, env._KIND
+        G = _coupling_group(coupling, B)
+        Tmax = (N - 1) if kind == vrpx.TSP else 2 * (N - 1) + 1
+        if Tmax < 3:
+            # TSP with N <= 3 has no table-mode decode loop: the definition itself, K episodes on copies of the env
+            runs = [self.rollout_episode(deepcopy(env), h, greedy=False, want_logits=want_logits, coupling=G, seed=seed,
+                                         offset=offset + k * B) for k in range(K)]
+            T = max(r["steps"] for r in runs)
+            tape = env._depot.to(torch.uint8).repeat(T, K, 1)
+            for k, r in enumerate(runs):
+                tape[:r["steps"], k] = r["tape"]
+            out = {"cost": torch.stack([r["cost"] for r in runs]), "logp": torch.stack([r["logp"] for r in runs]),
+                   "steps": T, "tape": tape, "coupling": G}
+            if want_logits:
+                logits = torch.full((T, K, B, N), float("nan"), dtype=torch.float32, device=dev)
+                for k, r in enumerate(runs):
+                    logits[:r["steps"], k] = r["logits"]
+                out["logits"] = logits
+            return out
+        if tuple(h.shape) != (B, N, vrpx.EMB) or h.dtype != torch.float32:
+            raise ValueError(f"h must be ({B}, {N}, {vrpx.EMB}) float32, got {tuple(h.shape)} {h.dtype}")
+        h = h.contiguous()
+        R = K * B
+        env._sync_instances()
+        # the replicated env: instances repeated copy-major, fresh episode state
+        xy, depot, demand = env._xy.repeat(K, 1, 1), env._depot.repeat(K), env._demand.repeat(K, 1)
+        visited = torch.zeros((R, 4), dtype=torch.int32, device=dev)
+        mask = visited if kind != vrpx.IRP else torch.zeros((R, 4), dtype=torch.int32, device=dev)
+        cur = torch.empty((R,), dtype=torch.int32, device=dev)
+        load = torch.ones((R,), dtype=torch.float64, device=dev)
+        v = vrpx.EnvView()
+        v.kind, v.N, v.B = kind, N, R
+        v.xy, v.depot, v.demand = xy.data_ptr(), depot.data_ptr(), demand.data_ptr()
+        v.visited, v.mask, v.cur, v.load = visited.data_ptr(), mask.data_ptr(), cur.data_ptr(), load.data_ptr()
+        L = vrpx.lib()
+        st = vrpx.stream_ptr(dev)
+        vrpx.check(L.vrpx_env_reset(C.byref(v), st))
+        w = self.packed(kind == vrpx.IRP, dev)
+        tape = torch.empty((Tmax, R), dtype=torch.uint8, device=dev)
+        logp = torch.empty((R,), dtype=torch.float32, device=dev)
+        cost = torch.empty((R,), dtype=torch.float32, device=dev)
+        steps = torch.zeros((1,), dtype=torch.int32, device=dev)
+        logits = torch.empty((Tmax, R, N), dtype=torch.float32, device=dev) if want_logits else None
+        nbytes = int(L.vrpx_rollout_samples_workspace_bytes(kind, B, K, N))
+        ws = torch.empty((nbytes,), dtype=torch.uint8, device=dev)
+        vrpx.check(L.vrpx_rollout_samples(C.byref(v), C.byref(w), vrpx.ptr(h), B, K, G, C.c_uint64(seed),
+                                          C.c_uint64(offset), vrpx.ptr(tape), Tmax, vrpx.ptr(logp), vrpx.ptr(cost),
+                                          vrpx.ptr(steps), vrpx.ptr(logits), vrpx.ptr(ws), nbytes, st))
+        T = int(steps.item())
+        out = {"cost": cost.view(K, B), "logp": logp.view(K, B), "steps": T, "tape": tape[:T].view(T, K, B),
+               "coupling": G}
+        if logits is not None:
+            out["logits"] = logits[:T].view(T, K, B, N)
         return out
 
     # ------------------------------------------------------------------ single-step entry (reference call style)
@@ -177,3 +244,11 @@ class GraphDecoder(nn.Module):
         self.last_ = None
         self.first_step = True
         self._ep = None
+
+
+def _coupling_group(coupling, B: int) -> int:
+    G = B if coupling is None else int(coupling)
+    if G < 0 or (G != 0 and (G > B or B % G != 0)):
+        raise ValueError(f"coupling group {G} must be 0 or a divisor of the batch size {B}: attention row (b, head) "
+                         "reads the mask of instance (8b + head) mod G of its group (graph_decoder.py:93)")
+    return G

@@ -84,6 +84,32 @@ class TSPModel(nn.Module):
         return -out["cost"], out["logp"]
 
 
+    @torch.no_grad()
+    def sample_best(self, env, num_samples: int) -> dict:
+        """Best of K = num_samples sampled tours per instance from one encoder pass (GraphDecoder.rollout_samples; the
+        Philox seed comes from the torch global RNG as in `forward`).  Records nothing for backward and leaves env
+        untouched.  Returns dict(cost (B,) smallest tour length, tour (steps,B) its actions, logp (B,) its log-prob,
+        index (B,) its copy k (the lowest k on ties), costs (K,B) every copy's tour length)."""
+        if not hasattr(env, "_view"):
+            raise vrpx.VrpxError("the fused rollout needs a device-resident gym_vrp env (TSPEnv/VRPEnv/IRPEnv of this package)")
+        dev = env._device
+        if next(self.parameters()).device != dev:
+            self.to(dev)
+        env._sync_instances()
+        h = run_encoder(self.encoder, env=env, depot=env._depot if self._USES_DEPOT_EMBED else None,
+                        gemm_path=self.encoder.gemm_path)
+        seed = int(torch.randint(0, 2 ** 62, (1,)).item())
+        out = self.decoder.rollout_samples(env, h, num_samples, seed=seed, offset=self.sample_offset,
+                                           coupling=self.coupling)
+        costs = out["cost"]
+        K, B = costs.shape
+        ks = torch.arange(K, device=dev)[:, None].expand(K, B)
+        best = torch.where(costs == costs.min(0, keepdim=True).values, ks, K).min(0).values
+        ar = torch.arange(B, device=dev)
+        return {"cost": costs[best, ar], "tour": out["tape"][:, best, ar], "logp": out["logp"][best, ar], "index": best,
+                "costs": costs}
+
+
 class TSPAgent:
     _MODEL = TSPModel
 
@@ -116,9 +142,12 @@ class TSPAgent:
             loss_b, _ = self.target_model(env_baseline, rollouts[0])
         return loss, loss_b, log_prob
 
-    def evaluate(self, env):
-        """Greedy rollout of the current model; returns the reward (-cost) per instance."""
+    def evaluate(self, env, samples: int = None):
+        """Reward (-cost) per instance of the current model: the greedy rollout, or with `samples` = K the best of K
+        sampled tours (TSPModel.sample_best; env is left untouched)."""
         self.model.eval()
+        if samples is not None:
+            return -self.model.sample_best(env, samples)["cost"]
         with torch.no_grad():
             loss, _ = self.model(env, rollout=True)
         return loss

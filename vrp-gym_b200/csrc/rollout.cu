@@ -301,57 +301,48 @@ int64_t vrpx_rollout_workspace_bytes(int64_t B, int32_t N) {
 
 int64_t vrpx_rollout_workspace_qg_offset(void) { return kRolloutHdr; }
 
-// table-mode workspace: header | Q~g | gmask | S0 | SL (IRP) | S1 | c | q^ | transposed and split weights, every segment
-// 256-byte aligned
+// table-mode workspace: header | Q~g | gmask | S0 | SL (IRP) | S1 | c | q^ | transposed and split weights | per-copy step
+// flags | per-replica flags (the flags for K > 1 only), every segment 256-byte aligned.  S1 holds the Bb base instances, every other per-instance segment the
+// Bb·K replicas.
 namespace {
 struct TableLayout {
-  int64_t s0, sl, s1, cbuf, qhat, mnt, agn, afn, w16b, qkw16, total;
+  int64_t s0, sl, s1, cbuf, qhat, mnt, agn, afn, w16b, qkw16, copy_left, replica_left, total;
 };
 inline int64_t align256(int64_t x) { return (x + 255) & ~(int64_t)255; }
-TableLayout table_layout(int kind, int64_t B, int N) {
+inline int64_t copy_left_bytes(int64_t K, int N) { return K > 1 ? K * 2 * N * (int64_t)sizeof(int) : 0; }   // [2N > Tmax][K]
+TableLayout table_layout(int kind, int64_t Bb, int64_t K, int N) {
   TableLayout L;
-  const int64_t f = (int64_t)sizeof(float);
+  const int64_t f = (int64_t)sizeof(float), B = Bb * K;
   L.s0 = align256(vrpx_rollout_workspace_bytes(B, N));
   L.sl = align256(L.s0 + B * NH * N * f);
   L.s1 = (kind == VRPX_IRP) ? align256(L.sl + B * NH * N * f) : L.sl;
   // split-step mode (rollout_steps.cu): glimpse vectors, folded queries, transposed m_t
-  L.cbuf = align256(L.s1 + B * N * NH * N * f);
+  L.cbuf = align256(L.s1 + Bb * N * NH * N * f);
   L.qhat = align256(L.cbuf + B * QW * f);
   L.mnt = align256(L.qhat + B * E * f);
   L.agn = align256(L.mnt + (int64_t)QW * E * f);
   L.afn = align256(L.agn + (int64_t)QW * E * f);
   L.w16b = align256(L.afn + (int64_t)QW * E * f);
   L.qkw16 = align256(L.w16b + (int64_t)2 * QW * E * 2);
-  L.total = align256(L.qkw16 + (int64_t)2 * 768 * E * 2);
+  L.copy_left = align256(L.qkw16 + (int64_t)2 * 768 * E * 2);
+  L.replica_left = align256(L.copy_left + copy_left_bytes(K, N));
+  L.total = align256(L.replica_left + (K > 1 ? B : 0));
   return L;
 }
-}  // namespace
 
-int64_t vrpx_rollout_table_workspace_bytes(int32_t kind, int64_t B, int32_t N) { return table_layout(kind, B, N).total; }
-
-int vrpx_rollout(const vrpx_env* env, const vrpx_decoder_weights* w, const float* h, int32_t mode,
-                 int64_t coupling, uint64_t seed, uint64_t offset, uint8_t* tape, int32_t t_begin, int32_t Tmax,
-                 float* logp, float* cost, int32_t* steps, float* logits, const vrpx_rollout_trace* trace,
-                 void* ws, int64_t ws_bytes, void* stream_) {
-  cudaStream_t stream = (cudaStream_t)stream_;
-  VRPX_CHECK_ARG(env && w && h && logp && cost && steps && ws, "NULL argument");
-  VRPX_DEVICE_GUARD(h);
-  NvtxRange nvtx_range("vrpx:rollout");
+int check_env_and_weights(const vrpx_env* env, const vrpx_decoder_weights* w) {
   VRPX_CHECK_ARG(env->kind >= 0 && env->kind <= 2 && env->N >= 2 && env->N <= VRPX_MAX_NODES && env->B >= 1,
                  "bad env header");
   VRPX_CHECK_ARG(env->xy && env->depot && env->visited && env->mask && env->cur && env->load, "env arrays");
   VRPX_CHECK_ARG(env->kind != VRPX_IRP || env->demand, "IRP env needs demand");
-  VRPX_CHECK_ARG(mode >= 0 && mode <= 2, "bad mode");
-  VRPX_CHECK_ARG(mode != VRPX_TEACHER || tape, "teacher mode needs a tape");
-  VRPX_CHECK_ARG(Tmax >= 1 && Tmax <= 1000 && t_begin >= 0, "t_begin / Tmax out of range");
-  // attention row (b, head) reads the mask of instance quirk_row(b, head, G): it must stay inside the batch
-  VRPX_CHECK_ARG(coupling >= 0 && (coupling == 0 || (coupling <= env->B && env->B % coupling == 0)),
-                 "coupling group must be 0 or a divisor of the batch size");
-  VRPX_CHECK_ARG(ws_bytes >= vrpx_rollout_workspace_bytes(env->B, env->N), "workspace too small");
-  VRPX_CHECK_ARG((reinterpret_cast<uintptr_t>(ws) & 15) == 0, "workspace must be 16-byte aligned");
   VRPX_CHECK_ARG(w->ag_t && w->al_t && w->a_c && w->a_q0 && w->m_t && w->m_c, "decoder weights");
   VRPX_CHECK_ARG(env->kind == VRPX_IRP ? (w->a_load != nullptr) : (w->af_t != nullptr), "decoder weights (kind)");
+  return VRPX_OK;
+}
 
+RolloutParams make_params(const vrpx_env* env, const vrpx_decoder_weights* w, const float* h, int mode, int64_t coupling,
+                          uint64_t seed, uint64_t offset, uint8_t* tape, int t_begin, int Tmax, float* logp, float* cost,
+                          int32_t* steps, float* logits, void* ws) {
   RolloutParams p;
   p.env = *env;
   p.w = *w;
@@ -367,9 +358,9 @@ int vrpx_rollout(const vrpx_env* env, const vrpx_decoder_weights* w, const float
   p.cost = cost;
   p.steps = steps;
   p.logits = logits;
-  p.qg0 = trace ? trace->qg0 : nullptr;
-  p.mask_hist = trace ? trace->mask_hist : nullptr;
-  p.load_hist = trace ? trace->load_hist : nullptr;
+  p.qg0 = nullptr;
+  p.mask_hist = nullptr;
+  p.load_hist = nullptr;
   p.prof = g_rollout_prof;
   p.bar = reinterpret_cast<unsigned*>(ws);
   p.notdone = reinterpret_cast<int*>(ws) + 8;
@@ -379,46 +370,14 @@ int vrpx_rollout(const vrpx_env* env, const vrpx_decoder_weights* w, const float
   p.s1 = nullptr;
   p.s0 = p.sl = nullptr;
   p.cbuf = p.qhat = nullptr;
-  SplitWorkspace sw{nullptr, nullptr, nullptr, nullptr};
-  // Split-step form (default for whole-episode calls with the large workspace and the rank-48 factors): per-episode score
-  // tables, then every step is a handful of launches over the whole batch (rollout_steps.cu).  The persistent kernel
-  // below serves the classic mode, resumed single-step calls and vrpx_debug_rollout_split(0).
-  if (g_split_steps && w->qk_w && t_begin == 0 && Tmax >= 3) {
-    const TableLayout L = table_layout(env->kind, env->B, env->N);
-    if (ws_bytes >= L.total) {
-      char* base = reinterpret_cast<char*>(ws);
-      float* s1 = reinterpret_cast<float*>(base + L.s1);
-      int rc;
-      {
-        NvtxRange nvtx_tables("vrpx:score_tables");
-        rc = build_score_table_fused(h, w->qk_w, env->B, env->N, reinterpret_cast<__half*>(base + L.qkw16), s1, stream);
-      }
-      if (rc) return rc;
-      p.s1 = s1;
-      p.s0 = reinterpret_cast<float*>(base + L.s0);
-      p.sl = reinterpret_cast<float*>(base + L.sl);
-      p.cbuf = reinterpret_cast<float*>(base + L.cbuf);
-      p.qhat = reinterpret_cast<float*>(base + L.qhat);
-      sw.m_nt = reinterpret_cast<float*>(base + L.mnt);
-      sw.ag_n = reinterpret_cast<float*>(base + L.agn);
-      sw.af_n = reinterpret_cast<float*>(base + L.afn);
-      sw.w16b = reinterpret_cast<__half*>(base + L.w16b);
-    }
-  }
-  const bool split = p.s1 != nullptr;
-  GemmPlan plan_b;
-  if (split) {
-    int rc = prepare_split_weights(p, sw, &plan_b, stream);
-    if (rc) return rc;
-  }
-  VRPX_CHECK_ARG((int64_t)(Tmax + 1 + 8) * 4 <= kRolloutSmall, "Tmax too large for workspace header");
+  p.Bb = env->B;
+  p.K = 1;
+  p.replica_left = nullptr;
+  p.copy_left = nullptr;
+  return p;
+}
 
-  VRPX_CUDA(cudaMemsetAsync(ws, 0, kRolloutSmall, stream));
-  if (!split) {
-    k_split_m16<<<(QW / 2) * E / 256, 256, 0, stream>>>(w->m_t, reinterpret_cast<uint2*>(reinterpret_cast<char*>(ws) + kRolloutSmall));
-    VRPX_LAUNCH_CHECK();
-    VRPX_CUDA(cudaFuncSetAttribute(k_rollout, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_TOTAL));
-  }
+int decode_timing_begin(cudaStream_t stream) {
   if (g_time_kernel) {
     if (!g_ev0) {
       VRPX_CUDA(cudaEventCreate(&g_ev0));
@@ -426,23 +385,129 @@ int vrpx_rollout(const vrpx_env* env, const vrpx_decoder_weights* w, const float
     }
     VRPX_CUDA(cudaEventRecord(g_ev0, stream));
   }
-  NvtxRange nvtx_decode("vrpx:decode_loop");
-  if (split) {
-    int rc = run_first_steps(p, sw, plan_b, stream);
-    if (rc) return rc;
-    if ((rc = run_split_steps(p, t_begin + 2, plan_b, stream))) return rc;   // also writes the step count
-  } else {
-    int64_t ntiles = (env->B + RTM - 1) / RTM;
-    int grid = (int)((ntiles < (int64_t)num_sms()) ? ntiles : (int64_t)num_sms());
-    void* args[] = {(void*)&p};
-    VRPX_CUDA(cudaLaunchCooperativeKernel((void*)k_rollout, dim3(grid), dim3(NT), args, SMEM_TOTAL, stream));
-    count_launch();
-  }
+  return VRPX_OK;
+}
+
+int decode_timing_end(cudaStream_t stream) {
   if (g_time_kernel) {
     VRPX_CUDA(cudaEventRecord(g_ev1, stream));
     g_ev_valid = true;
   }
   return VRPX_OK;
+}
+
+// Table mode: score tables over the p.Bb base instances (rollout_steps.cu reads them at each replica's base instance),
+// then every decode step as launches over the p.env.B replicas.
+int run_table_episode(RolloutParams& p, const TableLayout& L, void* ws, cudaStream_t stream) {
+  char* base = reinterpret_cast<char*>(ws);
+  float* s1 = reinterpret_cast<float*>(base + L.s1);
+  int rc;
+  {
+    NvtxRange nvtx_tables("vrpx:score_tables");
+    rc = build_score_table_fused(p.h, p.w.qk_w, p.Bb, p.env.N, reinterpret_cast<__half*>(base + L.qkw16), s1, stream);
+  }
+  if (rc) return rc;
+  p.s1 = s1;
+  p.s0 = reinterpret_cast<float*>(base + L.s0);
+  p.sl = reinterpret_cast<float*>(base + L.sl);
+  p.cbuf = reinterpret_cast<float*>(base + L.cbuf);
+  p.qhat = reinterpret_cast<float*>(base + L.qhat);
+  const SplitWorkspace sw{reinterpret_cast<float*>(base + L.mnt), reinterpret_cast<float*>(base + L.agn),
+                          reinterpret_cast<float*>(base + L.afn), reinterpret_cast<__half*>(base + L.w16b)};
+  GemmPlan plan_b;
+  if ((rc = prepare_split_weights(p, sw, &plan_b, stream))) return rc;
+  VRPX_CUDA(cudaMemsetAsync(ws, 0, kRolloutSmall, stream));
+  if ((rc = decode_timing_begin(stream))) return rc;
+  NvtxRange nvtx_decode("vrpx:decode_loop");
+  if ((rc = run_first_steps(p, sw, plan_b, stream))) return rc;
+  if ((rc = run_split_steps(p, p.t0 + 2, plan_b, stream))) return rc;   // also writes the step count
+  return decode_timing_end(stream);
+}
+}  // namespace
+
+int64_t vrpx_rollout_table_workspace_bytes(int32_t kind, int64_t B, int32_t N) { return table_layout(kind, B, 1, N).total; }
+
+int64_t vrpx_rollout_samples_workspace_bytes(int32_t kind, int64_t Bb, int32_t K, int32_t N) {
+  return table_layout(kind, Bb, K, N).total;
+}
+
+int vrpx_rollout(const vrpx_env* env, const vrpx_decoder_weights* w, const float* h, int32_t mode,
+                 int64_t coupling, uint64_t seed, uint64_t offset, uint8_t* tape, int32_t t_begin, int32_t Tmax,
+                 float* logp, float* cost, int32_t* steps, float* logits, const vrpx_rollout_trace* trace,
+                 void* ws, int64_t ws_bytes, void* stream_) {
+  cudaStream_t stream = (cudaStream_t)stream_;
+  VRPX_CHECK_ARG(env && w && h && logp && cost && steps && ws, "NULL argument");
+  VRPX_DEVICE_GUARD(h);
+  NvtxRange nvtx_range("vrpx:rollout");
+  if (int rc = check_env_and_weights(env, w)) return rc;
+  VRPX_CHECK_ARG(mode >= 0 && mode <= 2, "bad mode");
+  VRPX_CHECK_ARG(mode != VRPX_TEACHER || tape, "teacher mode needs a tape");
+  VRPX_CHECK_ARG(Tmax >= 1 && Tmax <= 1000 && t_begin >= 0, "t_begin / Tmax out of range");
+  // attention row (b, head) reads the mask of instance quirk_row(b, head, G): it must stay inside the batch
+  VRPX_CHECK_ARG(coupling >= 0 && (coupling == 0 || (coupling <= env->B && env->B % coupling == 0)),
+                 "coupling group must be 0 or a divisor of the batch size");
+  VRPX_CHECK_ARG(ws_bytes >= vrpx_rollout_workspace_bytes(env->B, env->N), "workspace too small");
+  VRPX_CHECK_ARG((reinterpret_cast<uintptr_t>(ws) & 15) == 0, "workspace must be 16-byte aligned");
+  VRPX_CHECK_ARG((int64_t)(Tmax + 1 + 8) * 4 <= kRolloutSmall, "Tmax too large for workspace header");
+
+  RolloutParams p = make_params(env, w, h, mode, coupling, seed, offset, tape, t_begin, Tmax, logp, cost, steps, logits, ws);
+  p.qg0 = trace ? trace->qg0 : nullptr;
+  p.mask_hist = trace ? trace->mask_hist : nullptr;
+  p.load_hist = trace ? trace->load_hist : nullptr;
+  // Split-step form (default for whole-episode calls with the large workspace and the rank-48 factors): per-episode score
+  // tables, then every step is a handful of launches over the whole batch (rollout_steps.cu).  The persistent kernel
+  // below serves the classic mode, resumed single-step calls and vrpx_debug_rollout_split(0).
+  if (g_split_steps && w->qk_w && t_begin == 0 && Tmax >= 3) {
+    const TableLayout L = table_layout(env->kind, env->B, 1, env->N);
+    if (ws_bytes >= L.total) return run_table_episode(p, L, ws, stream);
+  }
+
+  VRPX_CUDA(cudaMemsetAsync(ws, 0, kRolloutSmall, stream));
+  k_split_m16<<<(QW / 2) * E / 256, 256, 0, stream>>>(w->m_t, reinterpret_cast<uint2*>(reinterpret_cast<char*>(ws) + kRolloutSmall));
+  VRPX_LAUNCH_CHECK();
+  VRPX_CUDA(cudaFuncSetAttribute(k_rollout, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_TOTAL));
+  if (int rc = decode_timing_begin(stream)) return rc;
+  NvtxRange nvtx_decode("vrpx:decode_loop");
+  int64_t ntiles = (env->B + RTM - 1) / RTM;
+  int grid = (int)((ntiles < (int64_t)num_sms()) ? ntiles : (int64_t)num_sms());
+  void* args[] = {(void*)&p};
+  VRPX_CUDA(cudaLaunchCooperativeKernel((void*)k_rollout, dim3(grid), dim3(NT), args, SMEM_TOTAL, stream));
+  count_launch();
+  return decode_timing_end(stream);
+}
+
+int vrpx_rollout_samples(const vrpx_env* env, const vrpx_decoder_weights* w, const float* h, int64_t Bb, int32_t K,
+                         int64_t coupling, uint64_t seed, uint64_t offset, uint8_t* tape, int32_t Tmax, float* logp,
+                         float* cost, int32_t* steps, float* logits, void* ws, int64_t ws_bytes, void* stream_) {
+  cudaStream_t stream = (cudaStream_t)stream_;
+  VRPX_CHECK_ARG(env && w && h && tape && logp && cost && steps && ws, "NULL argument");
+  VRPX_DEVICE_GUARD(h);
+  NvtxRange nvtx_range("vrpx:rollout_samples");
+  if (int rc = check_env_and_weights(env, w)) return rc;
+  VRPX_CHECK_ARG(K >= 1, "sample count K must be at least 1");
+  VRPX_CHECK_ARG(Bb >= 1 && env->B % K == 0 && env->B / K == Bb, "env must hold Bb x K replicas");
+  // the partner rows of quirk_row must stay inside each copy
+  VRPX_CHECK_ARG(coupling >= 0 && (coupling == 0 || (coupling <= Bb && Bb % coupling == 0)),
+                 "coupling group must be 0 or a divisor of the base batch size");
+  VRPX_CHECK_ARG(w->qk_w, "sampling needs the score-table factors qk_w");
+  VRPX_CHECK_ARG(Tmax >= 1 && Tmax <= 1000, "Tmax out of range");
+  if (Tmax < 3) {
+    set_error("%s: episodes of fewer than 3 steps have no table-mode decode loop (use vrpx_rollout per copy)", __func__);
+    return VRPX_ERR_UNSUPPORTED;
+  }
+  const TableLayout L = table_layout(env->kind, Bb, K, env->N);
+  VRPX_CHECK_ARG(ws_bytes >= L.total, "workspace too small");
+  VRPX_CHECK_ARG((reinterpret_cast<uintptr_t>(ws) & 15) == 0, "workspace must be 16-byte aligned");
+
+  RolloutParams p = make_params(env, w, h, VRPX_SAMPLE, coupling, seed, offset, tape, 0, Tmax, logp, cost, steps, logits, ws);
+  p.Bb = Bb;
+  p.K = K;
+  if (K > 1) {
+    p.copy_left = reinterpret_cast<int*>(reinterpret_cast<char*>(ws) + L.copy_left);
+    p.replica_left = reinterpret_cast<uint8_t*>(ws) + L.replica_left;
+    VRPX_CUDA(cudaMemsetAsync(p.copy_left, 0, copy_left_bytes(K, env->N), stream));
+  }
+  return run_table_episode(p, L, ws, stream);
 }
 
 }  // extern "C"

@@ -40,7 +40,38 @@ struct RolloutParams {
   // split-step mode (rollout_steps.cu): glimpse vectors c [B][1024] and folded queries q^ [B][128] in global memory
   float* cbuf;
   float* qhat;
+  // K sampled copies of a batch of Bb base instances (vrpx_rollout_samples): replica r = k·Bb + b is copy k of base
+  // instance b and reads the embeddings and S1 of b; every other per-instance array is per replica (env.B = Bb·K).
+  // vrpx_rollout: Bb = env.B, K = 1.
+  int64_t Bb;
+  int K;
+  // K > 1 (NULL otherwise): replica_left[r] = replica r was unfinished after its last step (k_step_pointer), and
+  // copy_left[trel][k] != 0 when some replica of copy k was unfinished after step trel (k_copy_left).  A copy whose own
+  // episode is over skips the later steps: its cost, log-prob and env state stay those of the copy run alone, and its
+  // tape rows get the depot.
+  uint8_t* replica_left;
+  int* copy_left;
 };
+
+// Warp slot s of the split-step kernels -> the replica it runs (r), that replica's base instance (b) and copy (k).  Slot
+// s runs copy s mod K of base instance s / K, so the K warps that read h[b] and S1[b] are neighbours and run side by
+// side.  K = 1: the identity.
+struct SlotReplica {
+  int64_t r, b;
+  int k;
+};
+__device__ __forceinline__ SlotReplica slot_replica(const RolloutParams& p, int64_t s) {
+  if (p.K == 1) return {s, s, 0};
+  const int64_t b = s / p.K;
+  const int k = (int)(s - b * p.K);
+  return {k * p.Bb + b, b, k};
+}
+
+// true when copy k's own episode was over before step trel (K > 1; with K = 1 episode_over in rollout_steps.cu ends
+// every launch of the step instead)
+__device__ __forceinline__ bool copy_over(const RolloutParams& p, int k, int trel) {
+  return p.K > 1 && trel > 0 && __ldcg(p.copy_left + (int64_t)(trel - 1) * p.K + k) == 0;
+}
 
 // rollout_steps.cu: a whole-episode table-mode rollout as launches over the whole batch — steps 0 and 1 (run_first_steps:
 // they build Q~g and S0), then three launches per step (run_split_steps: glimpse, batched GEMM-B, pointer) and the final

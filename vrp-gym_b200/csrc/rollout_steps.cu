@@ -64,12 +64,15 @@ __global__ void __launch_bounds__(GW_MAX * 32, 2) k_step_glimpse(const RolloutPa
   if (episode_over(p, trel)) return;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int N = p.env.N, kind = p.env.kind;
-  const int64_t B = p.env.B, b = (int64_t)blockIdx.x * (blockDim.x >> 5) + warp;
-  if (b >= B) return;
+  const int64_t s = (int64_t)blockIdx.x * (blockDim.x >> 5) + warp;
+  if (s >= p.env.B) return;
+  const SlotReplica sr = slot_replica(p, s);
+  if (copy_over(p, sr.k, trel)) return;
+  const int64_t b = sr.r;
   unsigned char* ring = gsm + warp * glimpse_warp_bytes(N);
   float* slot = reinterpret_cast<float*>(ring + GNS * G_SLICE);
   const int g = lane >> 2, tq = lane & 3;
-  const float4* hrow = reinterpret_cast<const float4*>(p.h + b * N * E);
+  const float4* hrow = reinterpret_cast<const float4*>(p.h + sr.b * N * E);
   // slice s = node rows 8s .. 8s+7 -> ring stage s % GNS; lane = 16-byte chunk of the row
   auto issue_slice = [&](int sidx) {
     unsigned char* dst = ring + (sidx % GNS) * G_SLICE + lane * 16;
@@ -100,7 +103,7 @@ __global__ void __launch_bounds__(GW_MAX * 32, 2) k_step_glimpse(const RolloutPa
   float pr[NH][4];
   {
     const int last = __ldcg(p.env.cur + b);
-    const float* r1 = p.s1 + (((size_t)b * N + last) * NH) * N;
+    const float* r1 = p.s1 + (((size_t)sr.b * N + last) * NH) * N;
     const float* r0 = p.s0 + (size_t)b * NH * N;
     const float* rl = p.sl + (size_t)b * NH * N;
     // lane j holds mask word (j & 3) of the instance whose mask the reference adds to head j >> 2
@@ -171,21 +174,29 @@ __global__ void __launch_bounds__(GW_MAX * 32, 2) k_step_glimpse(const RolloutPa
 __global__ void __launch_bounds__(SW * 32) k_step_pointer(const RolloutParams p, int t) {
   __shared__ float s_slot[SW][VRPX_MAX_NODES];
   __shared__ float s_lp[SW];
+  __shared__ int64_t s_rep[SW];
   __shared__ int s_act[SW], s_anyleft;
   const int trel = t - p.t0;
   if (episode_over(p, trel)) return;
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int N = p.env.N, kind = p.env.kind;
-  // the CTAs walk the batch in the opposite direction to the glimpse kernel: the embeddings that kernel read last are
-  // still in L2 when this one starts, and the ones read last here are there for the next step's glimpse kernel
+  // the CTAs walk the warp slots (slot_replica) in the opposite direction to the glimpse kernel: the embeddings that
+  // kernel read last are still in L2 when this one starts, and the ones read last here are there for the next step's
+  // glimpse kernel
   const int64_t B = p.env.B, base = (int64_t)(gridDim.x - 1 - blockIdx.x) * SW;
   const int cnt = (int)((B - base < SW) ? (B - base) : SW);
   if (tid == 0) s_anyleft = 0;
-  if (warp < cnt) {
-    const int64_t b = base + warp;
+  const SlotReplica sr = slot_replica(p, base + (warp < cnt ? warp : 0));
+  if (warp < cnt && copy_over(p, sr.k, trel)) {   // the copy's own episode is over: depot in the tape, nothing else changes
+    if (lane == 0) {
+      if (p.tape) p.tape[(int64_t)trel * p.env.B + sr.r] = (uint8_t)__ldg(p.env.depot + sr.r);
+      s_act[warp] = -1;
+    }
+  } else if (warp < cnt) {
+    const int64_t b = sr.r;
     float* slot = s_slot[warp];
     const float4 qh = __ldcg(reinterpret_cast<const float4*>(p.qhat + b * E) + lane);
-    const float4* hp = reinterpret_cast<const float4*>(p.h + b * N * E) + lane;
+    const float4* hp = reinterpret_cast<const float4*>(p.h + sr.b * N * E) + lane;
     // own mask (graph_decoder.py:98).  The logits of masked nodes are never used (they become -inf below), so only the
     // embedding rows of the CANDIDATE nodes are read: on average half of the instance over an episode.
     const Bits128 full = full_bits(N);
@@ -254,14 +265,39 @@ __global__ void __launch_bounds__(SW * 32) k_step_pointer(const RolloutParams p,
     float u[4];
     warp_masked_logits(u, slot, mw, N, lane, idle);
     const PointerChoice c = warp_pointer_choice(u, p, b, t, trel, lane);
-    if (lane == 0) { s_act[warp] = c.a; s_lp[warp] = c.lp; }
+    if (lane == 0) { s_act[warp] = c.a; s_lp[warp] = c.lp; s_rep[warp] = b; }
   }
   __syncthreads();
   // environment transition: one THREAD per instance (the dependent global loads of the CTA's instances overlap)
-  if (tid < cnt && rollout_env_step(p, base + tid, s_act[tid], s_lp[tid], t, trel).unfinished)
-    s_anyleft = 1;   // benign race: all writers store 1
+  if (tid < cnt && s_act[tid] >= 0) {
+    const bool unfinished = rollout_env_step(p, s_rep[tid], s_act[tid], s_lp[tid], t, trel).unfinished;
+    if (unfinished) s_anyleft = 1;   // benign race: all writers store 1
+    if (p.replica_left) p.replica_left[s_rep[tid]] = unfinished;
+  }
   __syncthreads();
   if (tid == 0 && s_anyleft) atomicAdd(p.notdone + trel, 1);
+}
+
+// K > 1: copy_left[trel][k] = 1 when some replica of copy k was unfinished after step trel (replica_left, written by
+// k_step_pointer), one thread per replica and one store per warp and copy
+__global__ void __launch_bounds__(256) k_copy_left(const RolloutParams p, int t) {
+  const int trel = t - p.t0;
+  if (episode_over(p, trel)) return;
+  const int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  const bool unfinished = r < p.env.B && __ldcg(p.replica_left + r) != 0;
+  const int k = r < p.env.B ? (int)(r / p.Bb) : 0;
+  const unsigned peers = __match_any_sync(0xffffffffu, k) & __ballot_sync(0xffffffffu, unfinished);
+  if (unfinished && (threadIdx.x & 31) == __ffs(peers) - 1) p.copy_left[(int64_t)trel * p.K + k] = 1;
+}
+
+static int launch_pointer(const RolloutParams& p, int t, unsigned grid, cudaStream_t stream) {
+  k_step_pointer<<<grid, SW * 32, 0, stream>>>(p, t);
+  VRPX_LAUNCH_CHECK();
+  if (p.K > 1) {
+    k_copy_left<<<(unsigned)((p.env.B + 255) / 256), 256, 0, stream>>>(p, t);
+    VRPX_LAUNCH_CHECK();
+  }
+  return VRPX_OK;
 }
 
 
@@ -274,14 +310,15 @@ __global__ void __launch_bounds__(SW * 32) k_step_pointer(const RolloutParams p,
 // instance, mma.sync TF32 3-term: the score and value contractions of glimpse_mma.cuh) instead of reading them from the
 // tables.
 
-// Xf[b] = h[b, cur[b]]: the first chosen node after step 0 (graph_decoder.py:108-113)
-__global__ void __launch_bounds__(256) k_gather_cur(const float* __restrict__ h, const int* __restrict__ cur, int64_t B, int N,
-                                                    float* __restrict__ Xf) {
+// Xf[b] = h[b mod Bb, cur[b]]: the first chosen node after step 0 (graph_decoder.py:108-113) of every replica
+__global__ void __launch_bounds__(256) k_gather_cur(const float* __restrict__ h, const int* __restrict__ cur, int64_t B,
+                                                    int64_t Bb, int N, float* __restrict__ Xf) {
   const int lane = threadIdx.x & 31;
   const int64_t b = (int64_t)blockIdx.x * 8 + (threadIdx.x >> 5);
   if (b >= B) return;
   const int c = __ldcg(cur + b);
-  reinterpret_cast<float4*>(Xf + b * E)[lane] = __ldg(reinterpret_cast<const float4*>(h + (b * N + c) * E) + lane);
+  const int64_t hb = (b < Bb) ? b : b % Bb;
+  reinterpret_cast<float4*>(Xf + b * E)[lane] = __ldg(reinterpret_cast<const float4*>(h + (hb * N + c) * E) + lane);
 }
 
 // dst[c][r] = src[r][c]
@@ -299,11 +336,14 @@ __global__ void __launch_bounds__(FW * 32, 2) k_step_glimpse_first(const Rollout
   if (episode_over(p, trel)) return;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int N = p.env.N, kind = p.env.kind;
-  const int64_t B = p.env.B, b = (int64_t)blockIdx.x * FW + warp;
-  if (b >= B) return;
+  const int64_t s = (int64_t)blockIdx.x * FW + warp;
+  if (s >= p.env.B) return;
+  const SlotReplica sr = slot_replica(p, s);
+  if (copy_over(p, sr.k, trel)) return;
+  const int64_t b = sr.r;
   float* slot = s_slot[warp];
   const int tq = lane & 3;
-  const float4* hrow = reinterpret_cast<const float4*>(p.h + b * N * E);
+  const float4* hrow = reinterpret_cast<const float4*>(p.h + sr.b * N * E);
   const float lf = (float)p.env.load[b];
   record_trace(p, b, trel, lf, lane);
   // ---- q~: step 0 = Q~g + a_q0 (+ load · a_load); step 1 = the finished Q~g (its scores are S0, kept for every later step)
@@ -345,7 +385,7 @@ __global__ void __launch_bounds__(FW * 32, 2) k_step_glimpse_first(const Rollout
     }
     // + the table row of the node chosen at step 0: (A_l h[last])_head · h_n
     const int last = __ldcg(p.env.cur + b);
-    const float* r1 = p.s1 + (((size_t)b * N + last) * NH) * N;
+    const float* r1 = p.s1 + (((size_t)sr.b * N + last) * NH) * N;
 #pragma unroll
     for (int hh = 0; hh < NH; ++hh)
 #pragma unroll
@@ -412,20 +452,23 @@ int run_first_steps(const RolloutParams& p, const SplitWorkspace& w, const GemmP
   const int N = p.env.N;
   const unsigned g8 = (unsigned)((B + 7) / 8), grid_p = (unsigned)((B + SW - 1) / SW), grid_f = (unsigned)((B + FW - 1) / FW);
   int rc;
-  // ---- step 0: Q~g = A_g · mean_n h + a_c (the graph part of the folded query), then the placeholder step
-  if ((rc = launch_episode_gather(p.h, nullptr, B, N, p.qhat, nullptr, stream))) return rc;
-  GemmArgs g0{p.qhat, B, E, w.ag_n, QW, p.w.a_c, 0, nullptr, nullptr, nullptr, p.qg};
+  // ---- step 0: Q~g = A_g · mean_n h + a_c (the graph part of the folded query) over the base instances, copied into
+  // the rows of the other K - 1 copies (copy-major: one contiguous block each), then the placeholder step
+  if ((rc = launch_episode_gather(p.h, nullptr, p.Bb, N, p.qhat, nullptr, stream))) return rc;
+  GemmArgs g0{p.qhat, p.Bb, E, w.ag_n, QW, p.w.a_c, 0, nullptr, nullptr, nullptr, p.qg};
   if ((rc = gemm_tc(g0, stream))) return rc;
+  const size_t qg_block = (size_t)p.Bb * QW * sizeof(float);
+  for (int k = 1; k < p.K; ++k)
+    VRPX_CUDA(cudaMemcpyAsync(p.qg + (size_t)k * p.Bb * QW, p.qg, qg_block, cudaMemcpyDeviceToDevice, stream));
   if (p.qg0) VRPX_CUDA(cudaMemcpyAsync(p.qg0, p.qg, (size_t)B * QW * sizeof(float), cudaMemcpyDeviceToDevice, stream));
   k_step_glimpse_first<<<grid_f, FW * 32, 0, stream>>>(p, 0);
   VRPX_LAUNCH_CHECK();
   if ((rc = gemm_tc_launch(plan_b, stream))) return rc;
-  k_step_pointer<<<grid_p, SW * 32, 0, stream>>>(p, 0);
-  VRPX_LAUNCH_CHECK();
+  if ((rc = launch_pointer(p, 0, grid_p, stream))) return rc;
   if (p.Tmax < 2) return VRPX_OK;
   // ---- step 1: fold the first chosen node into Q~g (graph_decoder.py:111-113; IRP has no `first` term), build S0 (, SL)
   if (p.env.kind != VRPX_IRP) {
-    k_gather_cur<<<g8, 256, 0, stream>>>(p.h, p.env.cur, B, N, p.qhat);
+    k_gather_cur<<<g8, 256, 0, stream>>>(p.h, p.env.cur, B, p.Bb, N, p.qhat);
     VRPX_LAUNCH_CHECK();
     GemmArgs g1{p.qhat, B, E, w.af_n, QW, nullptr, 0, p.qg, nullptr, nullptr, p.qg};
     if ((rc = gemm_tc(g1, stream))) return rc;
@@ -433,8 +476,7 @@ int run_first_steps(const RolloutParams& p, const SplitWorkspace& w, const GemmP
   k_step_glimpse_first<<<grid_f, FW * 32, 0, stream>>>(p, 1);
   VRPX_LAUNCH_CHECK();
   if ((rc = gemm_tc_launch(plan_b, stream))) return rc;
-  k_step_pointer<<<grid_p, SW * 32, 0, stream>>>(p, 1);
-  VRPX_LAUNCH_CHECK();
+  if ((rc = launch_pointer(p, 1, grid_p, stream))) return rc;
   return VRPX_OK;
 }
 
@@ -449,8 +491,7 @@ int run_split_steps(const RolloutParams& p, int t_first, const GemmPlan& plan_b,
     VRPX_LAUNCH_CHECK();
     int rc = gemm_tc_launch(plan_b, stream);
     if (rc) return rc;
-    k_step_pointer<<<grid, SW * 32, 0, stream>>>(p, t);
-    VRPX_LAUNCH_CHECK();
+    if ((rc = launch_pointer(p, t, grid, stream))) return rc;
   }
   k_rollout_finish<<<1, 32, 0, stream>>>(p.notdone, p.t0, p.Tmax, p.steps);
   VRPX_LAUNCH_CHECK();

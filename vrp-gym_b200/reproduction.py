@@ -24,7 +24,8 @@ ENVS = {"TSP": TSPEnv, "VRP": VRPEnv, "IRP": IRPEnv}
 AGENTS = {"TSP": TSPAgent, "VRP": VRPAgent, "IRP": IRPAgent}
 
 
-def reproduce(seeds, num_nodes, batch_size, csv_path, model_path, num_draw, env_type, video=False, allow_untrained=False):
+def reproduce(seeds, num_nodes, batch_size, csv_path, model_path, num_draw, env_type, video=False, allow_untrained=False,
+              samples=None):
     # the reference loads the checkpoint unconditionally (reproduction.py:44) and fails without it; so does this script,
     # unless --allow_untrained asks for seed-initialised weights, which are then labelled as such in the CSV
     trained = bool(model_path) and os.path.exists(model_path)
@@ -43,7 +44,7 @@ def reproduce(seeds, num_nodes, batch_size, csv_path, model_path, num_draw, env_
             agent.model.load_state_dict(torch.load(model_path, map_location=agent.device))
         random_agent = RandomAgent(seed=seed)
         random_agent.eval()
-        cost_agent = agent.evaluate(env)
+        cost_agent = agent.evaluate(env, samples=samples)
         cost_random = random_agent(env_random)
         with open(csv_path, "a", newline="") as f:
             w = csv.writer(f)
@@ -62,6 +63,7 @@ if __name__ == "__main__":
     ap.add_argument("--model_path", type=str, default="./check_points/model_epoch__tsp_850.pt")
     ap.add_argument("--env_type", type=str, default="TSP", choices=sorted(ENVS))
     ap.add_argument("--video", action="store_true")
+    ap.add_argument("--samples", type=int, default=None, help="evaluate the best of K sampled tours per instance (default: greedy)")
     ap.add_argument("--allow_untrained", action="store_true", help="evaluate seed-initialised weights when the checkpoint is missing")
     args = ap.parse_args()
     print(vars(args))

@@ -22,7 +22,7 @@ EMB = 128
 LAYERS = 3
 
 
-ABI_VERSION = 4  # must equal VRPX_ABI_VERSION of include/vrpx.h
+ABI_VERSION = 5  # must equal VRPX_ABI_VERSION of include/vrpx.h
 
 
 class VrpxError(RuntimeError):
@@ -137,6 +137,10 @@ def lib():
     L.vrpx_rollout_workspace_qg_offset.restype = i64
     L.vrpx_rollout_table_workspace_bytes.argtypes = [i32, i64, i32]
     L.vrpx_rollout_table_workspace_bytes.restype = i64
+    L.vrpx_rollout_samples_workspace_bytes.argtypes = [i32, i64, i32, i32]
+    L.vrpx_rollout_samples_workspace_bytes.restype = i64
+    L.vrpx_rollout_samples.argtypes = [C.POINTER(EnvView), C.POINTER(DecoderWeights), vp, i64, i32, i64, u64, u64, vp,
+                                       i32, vp, vp, vp, vp, vp, i64, vp]
     L.vrpx_debug_rollout_profile.argtypes = [C.c_void_p]
     L.vrpx_debug_rollout_profile.restype = None
     L.vrpx_debug_rollout_split.argtypes = [i32]

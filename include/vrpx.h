@@ -25,7 +25,7 @@ extern "C" {
 #define VRPX_API
 #endif
 
-#define VRPX_ABI_VERSION 5
+#define VRPX_ABI_VERSION 6
 #define VRPX_MAX_NODES 128 /* visited bitmask = 4 x u32 per instance */
 #define VRPX_EMB 128       /* embedding width E (graph_tsp_agent.py:98) */
 #define VRPX_HEADS 8       /* heads (graph_tsp_agent.py:101, :55) */
@@ -270,13 +270,22 @@ VRPX_API int vrpx_rollout(const vrpx_env* env, const vrpx_decoder_weights* w, co
  *   tape      [Tmax][Bb·K] uint8 actions; logp, cost [Bb·K]; logits optional [Tmax][Bb·K][N]
  *   Tmax      maximum number of steps; Tmax < 3 (TSP with N <= 3) returns VRPX_ERR_UNSUPPORTED
  *   ws        at least vrpx_rollout_samples_workspace_bytes(kind, Bb, K, N) bytes
- * VRPX_ERR_ARG for K < 1, env->B != Bb·K, a bad coupling, a NULL qk_w or a workspace that is too small.  No backward
- * trace is recorded. */
+ * VRPX_ERR_ARG for K < 1, env->B != Bb·K, a bad coupling, a NULL qk_w or a workspace that is too small.
+ * vrpx_rollout_samples records no backward trace; it is vrpx_rollout_samples_traced with trace = NULL. */
 VRPX_API int64_t vrpx_rollout_samples_workspace_bytes(int32_t kind, int64_t Bb, int32_t K, int32_t N);
 VRPX_API int vrpx_rollout_samples(const vrpx_env* env, const vrpx_decoder_weights* w, const float* h, int64_t Bb,
                                   int32_t K, int64_t coupling, uint64_t seed, uint64_t offset, uint8_t* tape, int32_t Tmax,
                                   float* logp, float* cost, int32_t* steps, float* logits, void* ws, int64_t ws_bytes,
                                   void* stream);
+/* vrpx_rollout_samples plus the history vrpx_decoder_backward_samples replays (trace may be NULL; any field may be NULL):
+ *   mask_hist [Tmax][Bb·K][4], load_hist [Tmax][Bb·K], qg0 [Bb·K][1024], per replica.  Rows before a copy's own step count
+ *   equal those of vrpx_rollout(copy k alone, ..., trace) bit for bit; the rows after it, up to the returned step count,
+ *   hold the copy's terminal mask and load (the depot is then the only open node, so the replayed steps are inert).
+ *   The per-replica Q~g after the `first` fold stays in ws at vrpx_rollout_workspace_qg_offset(). */
+VRPX_API int vrpx_rollout_samples_traced(const vrpx_env* env, const vrpx_decoder_weights* w, const float* h, int64_t Bb,
+                                         int32_t K, int64_t coupling, uint64_t seed, uint64_t offset, uint8_t* tape,
+                                         int32_t Tmax, float* logp, float* cost, int32_t* steps, float* logits,
+                                         const vrpx_rollout_trace* trace, void* ws, int64_t ws_bytes, void* stream);
 
 /* Measurement hooks (bench.py, tools/): not part of the reference surface.
  *   vrpx_debug_rollout_profile  device buffer of 8 x int64 that accumulates per-phase cycles of thread 0 of every CTA
@@ -321,6 +330,18 @@ VRPX_API int vrpx_decoder_backward(const vrpx_env* env, const vrpx_decoder_weigh
                                    const float* h, const uint8_t* tape, int32_t T, int64_t coupling,
                                    const vrpx_rollout_trace* trace, const float* qg, const float* wts,
                                    const vrpx_decoder_grads* g, void* ws, int64_t ws_bytes, void* stream);
+
+/* Backward of vrpx_rollout_samples_traced: the K copies of Bb base instances in one launch.  env holds the Bb·K
+ * copy-major replicas (only kind, N and B are read); h [Bb][N][128] are the base embeddings the rollout read, and replica
+ * r = k·Bb + b reads them at row b.  tape [T][Bb·K], trace, qg [Bb·K][1024] (ws + vrpx_rollout_workspace_qg_offset() of the
+ * forward call), wts [Bb·K] and every per-instance gradient buffer of g (dH [Bb·K][N][128], D0, D1, Dl) are per replica:
+ * dH is NOT summed over the copies.  T = the step count of the forward call (the slowest copy's).  coupling: 0 or a divisor
+ * of Bb.  Workspace: vrpx_decoder_backward_workspace_bytes(Bb·K, N).  K = 1 is vrpx_decoder_backward. */
+VRPX_API int vrpx_decoder_backward_samples(const vrpx_env* env, const vrpx_decoder_weights* w,
+                                           const vrpx_decoder_bwd_weights* wb, const float* h, int64_t Bb, int32_t K,
+                                           const uint8_t* tape, int32_t T, int64_t coupling, const vrpx_rollout_trace* trace,
+                                           const float* qg, const float* wts, const vrpx_decoder_grads* g, void* ws,
+                                           int64_t ws_bytes, void* stream);
 
 /* Small per-episode helpers used by the backward passes (decoder epilogue, encoder weight gradients):
  *   C[M][N] += A^T · Bm  with A [R][M], Bm [R][N] (reduction over rows, red.add);  out[c] += sum_r X[r][c];

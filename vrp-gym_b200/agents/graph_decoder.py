@@ -114,22 +114,21 @@ class GraphDecoder(nn.Module):
         return out
 
     def rollout_samples(self, env, h: torch.Tensor, num_samples: int, *, seed: int, offset: int = 0, coupling=None,
-                        want_logits: bool = False):
-        """K = num_samples sampled episodes of every instance from one set of embeddings (vrpx_rollout_samples).
+                        want_logits: bool = False, save_for_backward: bool = False):
+        """K = num_samples sampled episodes of every instance from one set of embeddings (vrpx_rollout_samples_traced).
 
         env: device-resident TSPEnv/VRPEnv/IRPEnv of B instances in its reset state; it is left untouched (the K copies
         run on a private copy-major replica, replica k·B + b = copy k of instance b).  h: (B,N,128) f32 CUDA embeddings.
         Copy k is bit-identical to rollout_episode(copy of env, h, greedy=False, seed=seed, offset=offset + k·B,
         coupling=coupling).  All copies run until the slowest is done; a finished VRP/IRP copy idles on its depot.
-        Returns dict(cost (K,B) f32, logp (K,B) f32, steps int = max over copies, tape (steps,K,B) uint8
-        [, logits (steps,K,B,N)])."""
-        K = int(num_samples)
-        if K < 1:
-            raise ValueError(f"num_samples must be at least 1, got {num_samples}")
+        Returns dict(cost (K,B) f32, logp (K,B) f32, steps int = max over copies, tape (steps,K,B) uint8, samples K
+        [, logits (steps,K,B,N)]).  save_for_backward=True adds `saved`: the per-replica trace (mask_hist (Tmax,K·B,4),
+        load_hist (Tmax,K·B), qg0 (K·B,1024)), qg (K·B,1024) and the workspace holding it, and `replicas`, the vrpx_env
+        view of the replica env (with `replica_arrays` keeping its arrays alive) — what vrpx/backward.py replays."""
+        K, G = check_samples(env, num_samples, coupling, train=save_for_backward)
         dev = env._device
         B, N, kind = env.batch_size, env.num_nodes, env._KIND
-        G = _coupling_group(coupling, B)
-        Tmax = (N - 1) if kind == vrpx.TSP else 2 * (N - 1) + 1
+        Tmax = _max_steps(kind, N)
         if Tmax < 3:
             # TSP with N <= 3 has no table-mode decode loop: the definition itself, K episodes on copies of the env
             runs = [self.rollout_episode(deepcopy(env), h, greedy=False, want_logits=want_logits, coupling=G, seed=seed,
@@ -172,12 +171,26 @@ class GraphDecoder(nn.Module):
         logits = torch.empty((Tmax, R, N), dtype=torch.float32, device=dev) if want_logits else None
         nbytes = int(L.vrpx_rollout_samples_workspace_bytes(kind, B, K, N))
         ws = torch.empty((nbytes,), dtype=torch.uint8, device=dev)
-        vrpx.check(L.vrpx_rollout_samples(C.byref(v), C.byref(w), vrpx.ptr(h), B, K, G, C.c_uint64(seed),
-                                          C.c_uint64(offset), vrpx.ptr(tape), Tmax, vrpx.ptr(logp), vrpx.ptr(cost),
-                                          vrpx.ptr(steps), vrpx.ptr(logits), vrpx.ptr(ws), nbytes, st))
+        trace, saved = None, None
+        if save_for_backward:
+            saved = {"mask_hist": torch.empty((Tmax, R, 4), dtype=torch.int32, device=dev),
+                     "load_hist": torch.empty((Tmax, R), dtype=torch.float32, device=dev),
+                     "qg0": torch.empty((R, 1024), dtype=torch.float32, device=dev)}
+            trace = vrpx.RolloutTrace(saved["mask_hist"].data_ptr(), saved["load_hist"].data_ptr(), saved["qg0"].data_ptr())
+        vrpx.check(L.vrpx_rollout_samples_traced(C.byref(v), C.byref(w), vrpx.ptr(h), B, K, G, C.c_uint64(seed),
+                                                 C.c_uint64(offset), vrpx.ptr(tape), Tmax, vrpx.ptr(logp), vrpx.ptr(cost),
+                                                 vrpx.ptr(steps), vrpx.ptr(logits),
+                                                 C.byref(trace) if trace is not None else None, vrpx.ptr(ws), nbytes, st))
         T = int(steps.item())
         out = {"cost": cost.view(K, B), "logp": logp.view(K, B), "steps": T, "tape": tape[:T].view(T, K, B),
-               "coupling": G}
+               "coupling": G, "samples": K}
+        if saved is not None:
+            o = int(L.vrpx_rollout_workspace_qg_offset())
+            saved["qg"] = ws[o:o + R * 4096].view(torch.float32).view(R, 1024)  # Q~g incl. the `first` fold, per replica
+            saved["ws"] = ws
+            saved["replicas"] = v
+            saved["replica_arrays"] = (xy, depot, demand, visited, mask, cur, load)
+            out["saved"] = saved
         if logits is not None:
             out["logits"] = logits[:T].view(T, K, B, N)
         return out
@@ -244,6 +257,24 @@ class GraphDecoder(nn.Module):
         self.last_ = None
         self.first_step = True
         self._ep = None
+
+
+def _max_steps(kind: int, N: int) -> int:
+    """Rows of an episode's tape: a TSP tour visits N - 1 nodes, a VRP / IRP episode takes at most 2 (N - 1) + 1 steps."""
+    return (N - 1) if kind == vrpx.TSP else 2 * (N - 1) + 1
+
+
+def check_samples(env, num_samples, coupling=None, train: bool = False):
+    """Arguments of a K-sample rollout of env, checked before any work is done: returns (K, coupling group G).  train:
+    the rollout is recorded for the backward, which replays the table-mode decode loop (vrpx_rollout_samples_traced)."""
+    K = int(num_samples)
+    if K < 1:
+        raise ValueError(f"num_samples must be at least 1, got {num_samples}")
+    G = _coupling_group(coupling, env.batch_size)
+    if train and _max_steps(env._KIND, env.num_nodes) < 3:
+        raise ValueError(f"training on K sampled tours needs the table-mode decode loop, which TSP with N <= 3 does not "
+                         f"have (N = {env.num_nodes}); train on the K-fold replicated env instead")
+    return K, G
 
 
 def _coupling_group(coupling, B: int) -> int:

@@ -24,7 +24,7 @@ from scipy import stats
 
 import vrpx
 
-from .graph_decoder import GraphDecoder
+from .graph_decoder import GraphDecoder, check_samples
 from .graph_encoder import GraphEncoder, run_encoder
 
 logging.basicConfig(level=logging.INFO)
@@ -44,12 +44,19 @@ class TSPModel(nn.Module):
         self.last_rollout = None  # dict from GraphDecoder.rollout_episode (tape, steps, ...)
 
     def backward(self, wts: torch.Tensor):
-        """Accumulate d(sum_b wts[b] * log_prob[b])/d(theta) of the LAST sampled train-mode rollout into .grad."""
+        """Accumulate d(sum_b wts[b] * log_prob[b])/d(theta) of the LAST sampled train-mode rollout into .grad.  After
+        forward_samples(env, K), wts is (K,B) like its log-probs."""
         from vrpx import backward as bw
 
         ctx = self.last_rollout
         if ctx is None or "enc_saved" not in ctx:
-            raise vrpx.VrpxError("no rollout recorded for backward: call model(env, rollout=False) in train mode with grad enabled")
+            raise vrpx.VrpxError("no rollout recorded for backward: call model(env, rollout=False) or "
+                                 "model.forward_samples(env, K) in train mode with grad enabled")
+        if "samples" in ctx:
+            shape = (ctx["samples"], ctx["env"].batch_size)
+            if tuple(wts.shape) != shape:
+                raise ValueError(f"wts of a K-sample rollout must be (K, B) = {shape}, got {tuple(wts.shape)}")
+            wts = wts.reshape(-1)
         dH = bw.decoder_backward(self.decoder, ctx["env"], ctx["emb"], ctx, wts, gemm_path=self.encoder.gemm_path)
         bw.encoder_backward(self.encoder, ctx["env"], ctx["depot"], ctx["enc_saved"], dH, gemm_path=self.encoder.gemm_path)
         self.last_rollout = None  # the saved activations are large: release them
@@ -83,6 +90,38 @@ class TSPModel(nn.Module):
         self.decoder.reset()
         return -out["cost"], out["logp"]
 
+    def forward_samples(self, env, num_samples: int) -> Tuple[torch.Tensor, torch.Tensor]:
+        """K = num_samples sampled tours per instance from one encoder pass (GraphDecoder.rollout_samples; the Philox
+        seed comes from the torch global RNG as in `forward`, copy k uses offset sample_offset + k·B).  env is left
+        untouched.  Returns (-cost (K,B), log_prob (K,B)) on the device.
+
+        In train mode under grad this is the REINFORCE forward of K-sample training: the train-mode encoder runs ONCE,
+        over the B instances (BatchNorm batch statistics and one running-statistic update from them), and backward(wts)
+        with wts (K,B) back-propagates sum_kb wts[k,b] log_prob[k,b].  K identical copies have the batch mean and biased
+        variance of one copy and their BatchNorm backward sums over the copies, so the gradient equals that of the
+        K-fold replicated batch; only the running variance differs, by the replicated batch's unbiased-variance factor."""
+        if not hasattr(env, "_view"):
+            raise vrpx.VrpxError("the fused rollout needs a device-resident gym_vrp env (TSPEnv/VRPEnv/IRPEnv of this package)")
+        need_grad = self.training and torch.is_grad_enabled()
+        check_samples(env, num_samples, self.coupling, train=need_grad)
+        dev = env._device
+        if next(self.parameters()).device != dev:
+            self.to(dev)
+        env._sync_instances()
+        depot = env._depot if self._USES_DEPOT_EMBED else None
+        enc_saved = None
+        if need_grad:
+            h, enc_saved = run_encoder(self.encoder, env=env, depot=depot, gemm_path=self.encoder.gemm_path, save=True)
+        else:
+            h = run_encoder(self.encoder, env=env, depot=depot, gemm_path=self.encoder.gemm_path)
+        seed = int(torch.randint(0, 2 ** 62, (1,)).item())
+        out = self.decoder.rollout_samples(env, h, num_samples, seed=seed, offset=self.sample_offset,
+                                           coupling=self.coupling, save_for_backward=need_grad)
+        out["emb"] = h
+        if need_grad:
+            out["enc_saved"], out["env"], out["depot"] = enc_saved, env, depot
+        self.last_rollout = out
+        return -out["cost"], out["logp"]
 
     @torch.no_grad()
     def sample_best(self, env, num_samples: int) -> dict:
@@ -132,10 +171,16 @@ class TSPAgent:
         self.opt = torch.optim.Adam(self.model.parameters(), lr=lr)
 
     # ------------------------------------------------------------------ rollouts
-    def step(self, env, rollouts: Tuple[bool, bool]):
+    def step(self, env, rollouts: Tuple[bool, bool], samples: int = None):
         """Reset the env, then play it with the model and (on a snapshot) with the baseline.  As in the
-        reference (:251-253) BOTH use rollouts[0]."""
+        reference (:251-253) BOTH use rollouts[0].  samples = K: both play K sampled tours per instance instead
+        (TSPModel.forward_samples; rollouts is not read) and every result is (K,B)."""
         env.reset()
+        if samples is not None:
+            loss, log_prob = self.model.forward_samples(env, samples)
+            with torch.no_grad():
+                loss_b, _ = self.target_model.forward_samples(env, samples)
+            return loss, loss_b, log_prob
         env_baseline = deepcopy(env)
         loss, log_prob = self.model(env, rollouts[0])
         with torch.no_grad():
@@ -153,16 +198,22 @@ class TSPAgent:
         return loss
 
     # ------------------------------------------------------------------ training
-    def train(self, env, epochs: int = 100, eval_epochs: int = 1, check_point_dir: str = "./check_points/"):
+    def train(self, env, epochs: int = 100, eval_epochs: int = 1, check_point_dir: str = "./check_points/",
+              samples: int = None):
+        """REINFORCE with the rollout baseline (reference :155-177).  samples = K: every epoch trains on K sampled tours
+        per instance against K sampled baseline tours, from one train-mode encoder pass (TSPModel.forward_samples);
+        the baseline update is unchanged."""
+        if samples is not None:
+            check_samples(env, samples, self.model.coupling, train=True)
         logging.info("Start Training")
         with open(self.csv_path, "w+", newline="") as file:
             csv.writer(file).writerow(["Epoch", "Loss", "Cost", "Advantage", "Time"])
         start_time = time.time()
         for e in range(epochs):
             self.model.train()
-            loss_m, loss_b, log_prob = self.step(env, (False, True))
+            loss_m, loss_b, log_prob = self.step(env, (False, True), samples=samples)
             advantage = (loss_m - loss_b) * -1
-            loss = self.policy_gradient_step(advantage, log_prob)
+            loss = self.policy_gradient_step(advantage, log_prob, samples=samples)
             self.baseline_update(env, eval_epochs)
             logging.info(f"Epoch {e} finished - Loss: {loss}, Advantage: {advantage.mean()} Dist: {loss_m.mean()}")
             with open(self.csv_path, "a", newline="") as file:
@@ -170,9 +221,12 @@ class TSPAgent:
                                            time.time() - start_time])
             self.save_model(episode=e, check_point_dir=check_point_dir)
 
-    def policy_gradient_step(self, advantage, log_prob):
-        """loss = mean(advantage * log_prob); backward; Adam step (reference :179-186)."""
-        B = advantage.shape[0]
+    def policy_gradient_step(self, advantage, log_prob, samples: int = None):
+        """loss = mean(advantage * log_prob); backward; Adam step (reference :179-186).  samples = K: advantage and
+        log_prob are (K,B) from step(env, ..., samples=K) and the mean runs over all K·B tours."""
+        if samples is not None and (advantage.dim() != 2 or advantage.shape[0] != samples):
+            raise ValueError(f"with samples={samples} the advantage must be (K, B), got {tuple(advantage.shape)}")
+        B = advantage.numel()
         loss = (advantage * log_prob).mean()
         self.opt.zero_grad()
         # d loss / d log_prob_b = advantage_b / B; the gradient flows only through log_prob (advantage is data)

@@ -26,6 +26,10 @@ constexpr int SCQ = 4;   // 1024-float scratch slots per instance
 struct DecBwdParams {
   int kind, N, T;
   long long B, G;
+  // K sampled copies (vrpx_decoder_backward_samples): replica b = k·Bb + b' reads the embeddings h [Bb][N][128] of its
+  // base instance b' = b mod Bb; every other per-instance array (tape, trace, qg, wts, dH, D0, D1, Dl) is per replica.
+  // vrpx_decoder_backward: Bb = B.
+  long long Bb;
   const float* h;
   const uint8_t* tape;
   const uint32_t* mask_hist;
@@ -84,6 +88,11 @@ __device__ __forceinline__ void warp_outer_product_tm(const float* A, int lda, c
   }
 }
 
+// embedding rows of replica b: those of its base instance
+__device__ __forceinline__ const float* base_rows(const DecBwdParams& p, int64_t b) {
+  return p.h + ((b < p.Bb) ? b : b % p.Bb) * p.N * E;
+}
+
 __global__ void __launch_bounds__(NT, 1) k_decoder_bwd(const DecBwdParams p) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   float* Xs = reinterpret_cast<float*>(smem_raw);
@@ -97,7 +106,6 @@ __global__ void __launch_bounds__(NT, 1) k_decoder_bwd(const DecBwdParams p) {
   const int N = p.N, kind = p.kind;
   const int64_t B = p.B;
   const int64_t ntiles = (B + TM - 1) / TM;
-  const float* __restrict__ h = p.h;
   float* SC = p.scratch + (size_t)blockIdx.x * TM * SCQ * QW;
   float* su = Wb + warp * 128;  // per-warp scratch for u (Wb is idle outside the GEMM phases)
   float mc_acc = 0.f;           // d m_c[tid] for tid < 128, flushed once at the end
@@ -120,7 +128,7 @@ __global__ void __launch_bounds__(NT, 1) k_decoder_bwd(const DecBwdParams p) {
           lf = p.load_hist ? p.load_hist[(int64_t)t * B + b] : 0.f;
           if (t > 0) {
             prev = (int)p.tape[(int64_t)(t - 1) * B + b];
-            xv = __ldg(reinterpret_cast<const float4*>(h + (b * N + prev) * E) + lane);
+            xv = __ldg(reinterpret_cast<const float4*>(base_rows(p, b) + prev * E) + lane);
           }
           // an instance with a single feasible node has log p = 0 identically: no gradient
           uint32_t mw = p.mask_hist[((int64_t)t * B + b) * 4 + (lane & 3)];
@@ -178,7 +186,7 @@ __global__ void __launch_bounds__(NT, 1) k_decoder_bwd(const DecBwdParams p) {
 #pragma unroll
           for (int i = 0; i < 4; ++i) nb[which][i] = nbm[i];
         }
-        const float4* hrow = reinterpret_cast<const float4*>(h + b * N * E);
+        const float4* hrow = reinterpret_cast<const float4*>(base_rows(p, b));
         warp_glimpse_scores(slot, hrow, N, lane, [&](int n, int which, float v) {
           const int wi = n >> 5;
           const uint32_t w0 = which ? nb[1][0] : nb[0][0], w1 = which ? nb[1][1] : nb[0][1];
@@ -210,7 +218,7 @@ __global__ void __launch_bounds__(NT, 1) k_decoder_bwd(const DecBwdParams p) {
         if (m < cnt && s_live[m]) {
           const int64_t b = base + m;
           const float4 qh = *reinterpret_cast<const float4*>(DQ + m * XS_LD + lane * 4);
-          const float4* hp = reinterpret_cast<const float4*>(h + b * N * E) + lane;
+          const float4* hp = reinterpret_cast<const float4*>(base_rows(p, b)) + lane;
           for (int n0 = 0; n0 < N; n0 += 8) {
             float v[8];
 #pragma unroll
@@ -305,7 +313,7 @@ __global__ void __launch_bounds__(NT, 1) k_decoder_bwd(const DecBwdParams p) {
           const float* sc_p = sc_q + QW;
           const float* sc_z = sc_q + 2 * QW;
           float* sc_dc = SC + (size_t)m * SCQ * QW + 3 * QW;
-          const float4* hrow = reinterpret_cast<const float4*>(h + b * N * E);
+          const float4* hrow = reinterpret_cast<const float4*>(base_rows(p, b));
           const int tq = lane & 3;
           // dc is parked in the scratch (pass Y needs it after the slot has been reused)
 #pragma unroll
@@ -658,24 +666,21 @@ int64_t vrpx_decoder_backward_workspace_bytes(int64_t B, int32_t N) {
   return grid * (int64_t)TM * SCQ * QW * (int64_t)sizeof(float);
 }
 
-int vrpx_decoder_backward(const vrpx_env* env, const vrpx_decoder_weights* w, const vrpx_decoder_bwd_weights* wb,
-                          const float* h, const uint8_t* tape, int32_t T, int64_t coupling,
-                          const vrpx_rollout_trace* trace, const float* qg, const float* wts,
-                          const vrpx_decoder_grads* g, void* ws, int64_t ws_bytes, void* stream_) {
-  cudaStream_t stream = (cudaStream_t)stream_;
-  VRPX_CHECK_ARG(env && w && wb && h && tape && trace && qg && wts && g && ws, "NULL argument");
-  VRPX_DEVICE_GUARD(h);
-  NvtxRange nvtx_range("vrpx:decoder_backward");
-  // the glimpse mask of attention row (b, head) is read at quirk_row(): it must stay inside the batch
-  VRPX_CHECK_ARG(coupling >= 0 && (coupling == 0 || (coupling <= env->B && env->B % coupling == 0)),
-                 "coupling group must be 0 or a divisor of the batch size");
+}  // extern "C"
+
+namespace {
+// one launch of k_decoder_bwd over env->B replicas of Bb base instances (Bb = env->B: vrpx_decoder_backward)
+int decoder_backward(const vrpx_env* env, const vrpx_decoder_weights* w, const vrpx_decoder_bwd_weights* wb,
+                     const float* h, int64_t Bb, const uint8_t* tape, int32_t T, int64_t coupling,
+                     const vrpx_rollout_trace* trace, const float* qg, const float* wts, const vrpx_decoder_grads* g,
+                     void* ws, int64_t ws_bytes, cudaStream_t stream) {
   VRPX_CHECK_ARG(env->N >= 2 && env->N <= VRPX_MAX_NODES && env->B >= 1 && T >= 1, "bad shape");
   VRPX_CHECK_ARG(trace->mask_hist && trace->qg0 && (env->kind != VRPX_IRP || trace->load_hist), "trace incomplete");
   VRPX_CHECK_ARG(g->dH && g->D0 && g->D1 && g->d_al_t && g->d_m_t && g->d_m_c && (env->kind != VRPX_IRP || g->Dl),
                  "gradient buffers");
   VRPX_CHECK_ARG(ws_bytes >= vrpx_decoder_backward_workspace_bytes(env->B, env->N), "workspace too small");
   DecBwdParams p;
-  p.kind = env->kind; p.N = env->N; p.T = T; p.B = env->B; p.G = coupling;
+  p.kind = env->kind; p.N = env->N; p.T = T; p.B = env->B; p.G = coupling; p.Bb = Bb;
   p.h = h; p.tape = tape; p.mask_hist = trace->mask_hist; p.load_hist = trace->load_hist;
   p.qg0 = trace->qg0; p.qg = qg; p.wts = wts;
   p.al_t = w->al_t; p.a_q0 = w->a_q0; p.a_load = w->a_load; p.m_t = w->m_t; p.m_c = w->m_c;
@@ -688,6 +693,39 @@ int vrpx_decoder_backward(const vrpx_env* env, const vrpx_decoder_weights* w, co
   k_decoder_bwd<<<grid, NT, BWD_SMEM, stream>>>(p);
   VRPX_LAUNCH_CHECK();
   return VRPX_OK;
+}
+}  // namespace
+
+extern "C" {
+
+int vrpx_decoder_backward(const vrpx_env* env, const vrpx_decoder_weights* w, const vrpx_decoder_bwd_weights* wb,
+                          const float* h, const uint8_t* tape, int32_t T, int64_t coupling,
+                          const vrpx_rollout_trace* trace, const float* qg, const float* wts,
+                          const vrpx_decoder_grads* g, void* ws, int64_t ws_bytes, void* stream_) {
+  VRPX_CHECK_ARG(env && w && wb && h && tape && trace && qg && wts && g && ws, "NULL argument");
+  VRPX_DEVICE_GUARD(h);
+  NvtxRange nvtx_range("vrpx:decoder_backward");
+  // the glimpse mask of attention row (b, head) is read at quirk_row(): it must stay inside the batch
+  VRPX_CHECK_ARG(coupling >= 0 && (coupling == 0 || (coupling <= env->B && env->B % coupling == 0)),
+                 "coupling group must be 0 or a divisor of the batch size");
+  return decoder_backward(env, w, wb, h, env->B, tape, T, coupling, trace, qg, wts, g, ws, ws_bytes,
+                          (cudaStream_t)stream_);
+}
+
+int vrpx_decoder_backward_samples(const vrpx_env* env, const vrpx_decoder_weights* w, const vrpx_decoder_bwd_weights* wb,
+                                  const float* h, int64_t Bb, int32_t K, const uint8_t* tape, int32_t T, int64_t coupling,
+                                  const vrpx_rollout_trace* trace, const float* qg, const float* wts,
+                                  const vrpx_decoder_grads* g, void* ws, int64_t ws_bytes, void* stream_) {
+  VRPX_CHECK_ARG(env && w && wb && h && tape && trace && qg && wts && g && ws, "NULL argument");
+  VRPX_DEVICE_GUARD(h);
+  NvtxRange nvtx_range("vrpx:decoder_backward_samples");
+  VRPX_CHECK_ARG(K >= 1, "sample count K must be at least 1");
+  VRPX_CHECK_ARG(Bb >= 1 && env->B % K == 0 && env->B / K == Bb, "env must hold Bb x K replicas");
+  // the partner rows of quirk_row must stay inside each copy
+  VRPX_CHECK_ARG(coupling >= 0 && (coupling == 0 || (coupling <= Bb && Bb % coupling == 0)),
+                 "coupling group must be 0 or a divisor of the base batch size");
+  return decoder_backward(env, w, wb, h, Bb, tape, T, coupling, trace, qg, wts, g, ws, ws_bytes,
+                          (cudaStream_t)stream_);
 }
 
 void vrpx_debug_gemm_tn_path(int32_t path) { g_tn_path = path; }

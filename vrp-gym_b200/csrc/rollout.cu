@@ -479,6 +479,14 @@ int vrpx_rollout(const vrpx_env* env, const vrpx_decoder_weights* w, const float
 int vrpx_rollout_samples(const vrpx_env* env, const vrpx_decoder_weights* w, const float* h, int64_t Bb, int32_t K,
                          int64_t coupling, uint64_t seed, uint64_t offset, uint8_t* tape, int32_t Tmax, float* logp,
                          float* cost, int32_t* steps, float* logits, void* ws, int64_t ws_bytes, void* stream_) {
+  return vrpx_rollout_samples_traced(env, w, h, Bb, K, coupling, seed, offset, tape, Tmax, logp, cost, steps, logits,
+                                     nullptr, ws, ws_bytes, stream_);
+}
+
+int vrpx_rollout_samples_traced(const vrpx_env* env, const vrpx_decoder_weights* w, const float* h, int64_t Bb, int32_t K,
+                                int64_t coupling, uint64_t seed, uint64_t offset, uint8_t* tape, int32_t Tmax, float* logp,
+                                float* cost, int32_t* steps, float* logits, const vrpx_rollout_trace* trace, void* ws,
+                                int64_t ws_bytes, void* stream_) {
   cudaStream_t stream = (cudaStream_t)stream_;
   VRPX_CHECK_ARG(env && w && h && tape && logp && cost && steps && ws, "NULL argument");
   VRPX_DEVICE_GUARD(h);
@@ -502,6 +510,9 @@ int vrpx_rollout_samples(const vrpx_env* env, const vrpx_decoder_weights* w, con
   RolloutParams p = make_params(env, w, h, VRPX_SAMPLE, coupling, seed, offset, tape, 0, Tmax, logp, cost, steps, logits, ws);
   p.Bb = Bb;
   p.K = K;
+  p.qg0 = trace ? trace->qg0 : nullptr;
+  p.mask_hist = trace ? trace->mask_hist : nullptr;
+  p.load_hist = trace ? trace->load_hist : nullptr;
   if (K > 1) {
     p.copy_left = reinterpret_cast<int*>(reinterpret_cast<char*>(ws) + L.copy_left);
     p.replica_left = reinterpret_cast<uint8_t*>(ws) + L.replica_left;

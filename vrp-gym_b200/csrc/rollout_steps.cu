@@ -57,6 +57,13 @@ __device__ __forceinline__ bool instance_idle(const uint32_t (&own)[4], int N, i
   return cand == 1 && !((own[depot >> 5] >> (depot & 31)) & 1u);
 }
 
+// A copy whose own episode is over skips the step, but the backward replays every replica for the launches' step count
+// (the slowest copy's): its trace rows there get the copy's terminal mask and load, the tape rows get the depot
+// (k_step_pointer), so the replayed step has the depot as its only open node (instance_idle) and contributes nothing.
+__device__ __forceinline__ void record_terminal(const RolloutParams& p, int64_t r, int trel, int lane) {
+  if (p.mask_hist || p.load_hist) record_trace(p, r, trel, (float)p.env.load[r], lane);
+}
+
 // ---------------------------------------------------------------- glimpse: tables -> softmax -> c
 __global__ void __launch_bounds__(GW_MAX * 32, 2) k_step_glimpse(const RolloutParams p, int t) {
   extern __shared__ __align__(16) unsigned char gsm[];
@@ -67,7 +74,10 @@ __global__ void __launch_bounds__(GW_MAX * 32, 2) k_step_glimpse(const RolloutPa
   const int64_t s = (int64_t)blockIdx.x * (blockDim.x >> 5) + warp;
   if (s >= p.env.B) return;
   const SlotReplica sr = slot_replica(p, s);
-  if (copy_over(p, sr.k, trel)) return;
+  if (copy_over(p, sr.k, trel)) {   // see record_terminal
+    record_terminal(p, sr.r, trel, lane);
+    return;
+  }
   const int64_t b = sr.r;
   unsigned char* ring = gsm + warp * glimpse_warp_bytes(N);
   float* slot = reinterpret_cast<float*>(ring + GNS * G_SLICE);
@@ -339,7 +349,10 @@ __global__ void __launch_bounds__(FW * 32, 2) k_step_glimpse_first(const Rollout
   const int64_t s = (int64_t)blockIdx.x * FW + warp;
   if (s >= p.env.B) return;
   const SlotReplica sr = slot_replica(p, s);
-  if (copy_over(p, sr.k, trel)) return;
+  if (copy_over(p, sr.k, trel)) {
+    record_terminal(p, sr.r, trel, lane);
+    return;
+  }
   const int64_t b = sr.r;
   float* slot = s_slot[warp];
   const int tq = lane & 3;

@@ -22,7 +22,7 @@ EMB = 128
 LAYERS = 3
 
 
-ABI_VERSION = 5  # must equal VRPX_ABI_VERSION of include/vrpx.h
+ABI_VERSION = 6  # must equal VRPX_ABI_VERSION of include/vrpx.h
 
 
 class VrpxError(RuntimeError):
@@ -126,6 +126,9 @@ def lib():
     L.vrpx_decoder_backward_workspace_bytes.restype = i64
     L.vrpx_decoder_backward.argtypes = [C.POINTER(EnvView), C.POINTER(DecoderWeights), C.POINTER(DecoderBwdWeights), vp, vp,
                                         i32, i64, C.POINTER(RolloutTrace), vp, vp, C.POINTER(DecoderGrads), vp, i64, vp]
+    L.vrpx_decoder_backward_samples.argtypes = [C.POINTER(EnvView), C.POINTER(DecoderWeights), C.POINTER(DecoderBwdWeights),
+                                                vp, i64, i32, vp, i32, i64, C.POINTER(RolloutTrace), vp, vp,
+                                                C.POINTER(DecoderGrads), vp, i64, vp]
     L.vrpx_gemm_tn_accumulate.argtypes = [vp, vp, vp, i64, i32, i32, vp]
     L.vrpx_gemm_tn_colsum_accumulate.argtypes = [vp, vp, vp, vp, i64, i32, i32, vp]
     L.vrpx_colsum_accumulate.argtypes = [vp, i64, i32, vp, vp]
@@ -141,6 +144,8 @@ def lib():
     L.vrpx_rollout_samples_workspace_bytes.restype = i64
     L.vrpx_rollout_samples.argtypes = [C.POINTER(EnvView), C.POINTER(DecoderWeights), vp, i64, i32, i64, u64, u64, vp,
                                        i32, vp, vp, vp, vp, vp, i64, vp]
+    L.vrpx_rollout_samples_traced.argtypes = [C.POINTER(EnvView), C.POINTER(DecoderWeights), vp, i64, i32, i64, u64, u64,
+                                              vp, i32, vp, vp, vp, vp, C.POINTER(RolloutTrace), vp, i64, vp]
     L.vrpx_debug_rollout_profile.argtypes = [C.c_void_p]
     L.vrpx_debug_rollout_profile.restype = None
     L.vrpx_debug_rollout_split.argtypes = [i32]

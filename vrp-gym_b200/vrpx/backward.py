@@ -63,17 +63,24 @@ def _grad_gain(dH, target_log2=None):
 
 def decoder_backward(dec, env, h, roll, wts, gemm_path=0):
     """Back-propagate wts[b] = dL/d(logp_b) through the rollout `roll` (dict from GraphDecoder.rollout_episode with
-    save_for_backward=True).  Accumulates the decoder parameters' .grad and returns dL/dh (B,N,128)."""
+    save_for_backward=True).  Accumulates the decoder parameters' .grad and returns dL/dh (B,N,128).
+
+    A K-sample rollout (GraphDecoder.rollout_samples with save_for_backward=True) is replayed over its K·B replicas in one
+    vrpx_decoder_backward_samples launch on the B base embeddings h, with wts (K·B,) copy-major.  The per-episode terms
+    are added to each replica's dL/dh, which is then summed over the copies."""
     L = vrpx.lib()
     dev = h.device
     st = vrpx.stream_ptr(dev)
-    B, N = env.batch_size, env.num_nodes
+    Bb, N = env.batch_size, env.num_nodes
     irp = env._KIND == vrpx.IRP
     w = dec.packed(irp, dev)
     tens = dec._packed[irp].tensors
     sv = roll["saved"]
-    tape = roll["tape"].contiguous()
-    T = int(tape.shape[0])
+    rep = sv.get("replicas")          # the replica env of a K-sample rollout
+    K = 1 if rep is None else rep.B // Bb
+    B = Bb * K
+    T = int(roll["tape"].shape[0])
+    tape = roll["tape"].reshape(T, B).contiguous()
     z = lambda *s: torch.zeros(s, dtype=torch.float32, device=dev)
     g = {"dH": z(B, N, 128), "D0": z(B, 1024), "D1": z(B, 1024), "Dl": z(B, 1024) if irp else None,
          "d_al_t": z(128, 1024), "d_m_t": z(1024, 128), "d_m_c": z(128)}
@@ -85,9 +92,14 @@ def decoder_backward(dec, env, h, roll, wts, gemm_path=0):
     nbytes = int(L.vrpx_decoder_backward_workspace_bytes(B, N))
     ws = torch.empty((nbytes,), dtype=torch.uint8, device=dev)
     wts = wts.detach().to(dev, torch.float32).contiguous()
-    vrpx.check(L.vrpx_decoder_backward(C.byref(env._view()), C.byref(w), C.byref(wb), vrpx.ptr(h), vrpx.ptr(tape), T,
-                                       int(roll["coupling"]), C.byref(trace), vrpx.ptr(sv["qg"]), vrpx.ptr(wts),
-                                       C.byref(gs), vrpx.ptr(ws), nbytes, st))
+    if rep is None:
+        vrpx.check(L.vrpx_decoder_backward(C.byref(env._view()), C.byref(w), C.byref(wb), vrpx.ptr(h), vrpx.ptr(tape), T,
+                                           int(roll["coupling"]), C.byref(trace), vrpx.ptr(sv["qg"]), vrpx.ptr(wts),
+                                           C.byref(gs), vrpx.ptr(ws), nbytes, st))
+    else:
+        vrpx.check(L.vrpx_decoder_backward_samples(C.byref(rep), C.byref(w), C.byref(wb), vrpx.ptr(h), Bb, K,
+                                                   vrpx.ptr(tape), T, int(roll["coupling"]), C.byref(trace),
+                                                   vrpx.ptr(sv["qg"]), vrpx.ptr(wts), C.byref(gs), vrpx.ptr(ws), nbytes, st))
     # ---- per-episode terms: q~ also contains A_g·g + a_c (every step), A_f·h[first] (steps >= 1), a_q0 (step 0)
     # the per-episode sums D are gradients too: the products below run on the f16-split tensor-core kernels (the weight
     # gradients ag_t / af_t at B >= 8192 on either gemm_path), so they get them scaled to 2^-2 (see _grad_gain; the sums
@@ -96,10 +108,15 @@ def decoder_backward(dec, env, h, roll, wts, gemm_path=0):
     gs_, g1_ = _grad_gain(Dsum, -2), _grad_gain(g["D1"], -2)
     DsumS = Dsum * gs_ if gs_ != 1.0 else Dsum
     D1S = g["D1"] * g1_ if g1_ != 1.0 else g["D1"]
-    G = torch.empty((B, 128), dtype=torch.float32, device=dev)
+    G = torch.empty((Bb, 128), dtype=torch.float32, device=dev)
     Xf = None if irp else torch.empty((B, 128), dtype=torch.float32, device=dev)
     tape0 = tape[0].contiguous()
-    vrpx.check(L.vrpx_episode_gather(vrpx.ptr(h), vrpx.ptr(tape0), B, N, vrpx.ptr(G), vrpx.ptr(Xf) if Xf is not None else None, st))
+    for k in range(K):   # Xf of copy k from the base embeddings; G does not depend on the copy
+        r = slice(k * Bb, (k + 1) * Bb)
+        vrpx.check(L.vrpx_episode_gather(vrpx.ptr(h), vrpx.ptr(tape0[r]), Bb, N, vrpx.ptr(G),
+                                         vrpx.ptr(Xf[r]) if Xf is not None else None, st))
+    if K > 1:
+        G = G.repeat(K, 1)
     dG = _gemm_nt(DsumS, tens["ag_t"], path=gemm_path)                      # (B,128) = Dsum · A_g
     dXf = None if irp else _gemm_nt(D1S, tens["af_t"], path=gemm_path)       # (B,128) = D1 · A_f
     if gs_ != 1.0:
@@ -135,6 +152,8 @@ def decoder_backward(dec, env, h, roll, wts, gemm_path=0):
     for p, gp in zip(params, pg):
         if gp is not None:
             _acc_grad(p, gp)
+    if K > 1:
+        return g["dH"].view(K, Bb, N, 128).sum(0)
     return g["dH"]
 
 

@@ -180,7 +180,8 @@ typedef struct vrpx_encoder_grads {
 VRPX_API int64_t vrpx_encoder_backward_workspace_bytes(int64_t B, int32_t N);
 
 /* Backward of the train-mode encoder forward (BatchNorm with batch statistics).  `saved` is the buffer the forward
- * filled; `g` [B][N][128] holds dL/dh on entry and is overwritten (it ends as dL/d(embedding)). */
+ * filled; `g` [B][N][128] holds dL/dh on entry and is overwritten (it ends as dL/d(embedding output), in the scale of
+ * dL/dh on entry). */
 VRPX_API int vrpx_encoder_backward(const vrpx_encoder_weights* w, const vrpx_encoder_weights_t* wt, const vrpx_env* env,
                                    const float* x, const int32_t* depot, int64_t B, int32_t N, const float* saved,
                                    float* g, const vrpx_encoder_grads* grads, void* ws, int64_t ws_bytes,
@@ -393,6 +394,20 @@ VRPX_API int vrpx_debug_score_table(const float* h, const float* qk_w, int64_t B
  * (path 0: mma.sync f16-split kernel = production; path 1: fp32 SIMT kernel). */
 VRPX_API int vrpx_debug_attention_backward(const float* qkv, const float* att, const float* datt, float* dqkv, int64_t B,
                                            int32_t N, int32_t path, void* stream);
+
+/* Test hook of the encoder backward (csrc/encoder_bwd.cu): vrpx_encoder_backward with the same arguments and launches,
+ * plus, for every layer whose bit is set in layer_mask (1..7), the gradients its kernels hold inside that layer, in the
+ * scale of g on entry.  The selected layers' blocks follow each other in ascending layer order in `stages`; each layer's
+ * part is eight stage-major blocks of R = B·N rows, 1,664 floats per row:
+ *   dOUT [R][128] (g on entry to the layer), dY2 [R][128] (after the BN2 backward), dPRE [R][512] (after the ReLU-gate
+ *   GEMM), dH1 [R][128] (after the residual GEMM), dY1 [R][128] (after the BN1 backward), dATT [R][128],
+ *   dQKV [R][384] (after the attention backward), dX [R][128] (g after the in-projection GEMM).
+ * Each block is one device-to-device cudaMemcpyAsync on `stream`. */
+VRPX_API int vrpx_debug_encoder_backward_stages(const vrpx_encoder_weights* w, const vrpx_encoder_weights_t* wt,
+                                                const vrpx_env* env, const float* x, const int32_t* depot, int64_t B,
+                                                int32_t N, const float* saved, float* g, const vrpx_encoder_grads* grads,
+                                                void* ws, int64_t ws_bytes, int32_t gemm_path, float* stages,
+                                                int32_t layer_mask, void* stream);
 
 /* Number of kernels this library has launched since load (bench.py's gpu_launches claim). */
 VRPX_API int64_t vrpx_launch_count(void);

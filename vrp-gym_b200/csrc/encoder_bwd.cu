@@ -4,9 +4,12 @@
 //
 // Input: dL/d(out of the last layer) (from the decoder backward) and the activations the train-mode forward saved
 // (encoder.cu, vrpx_encoder_saved_bytes).  Output: gradients of every encoder parameter, accumulated (+=).
-// Dense products reuse the forward GEMM kernels (dX = dY · W through gemm_tc/gemm_simt on the transposed weight;
-// dW = dY^T · X through k_gemm_tn_atomic, bias gradients through k_colsum_atomic); the per-instance attention
-// backward and the BatchNorm backward (two batch-wide reductions per BN) are SIMT kernels here.
+// Dense products reuse the forward GEMM kernels (dX = dY · W through gemm_tc/gemm_simt on the transposed weight, the
+// ReLU gate and the residual in its epilogue).  Weight and bias gradients go through gemm_tn_accumulate: k_gemm_tn_tc
+// with its colsum_A bias sums at R >= 8192 rows, k_gemm_tn_mma + k_colsum_atomic below (decoder_bwd.cu); the embedding
+// [128][4] products always take the warp-level kernels.  The per-instance attention backward runs on mma.sync
+// (attention_bwd.cu; gemm_path 1: the fp32 SIMT k_enc_attention_bwd below); the BatchNorm backward (two batch-wide f64
+// reductions per BN) is the pair of SIMT kernels below.
 #include "gemm.cuh"
 
 namespace vrpx {
@@ -39,7 +42,7 @@ __global__ void __launch_bounds__(256) k_bn_bwd_reduce(const float* __restrict__
 }
 
 // dy = gamma * invstd * (dout - mean(dout) - xhat * mean(dout * xhat));  in place on `g` (dout -> dy).
-// Block 0 also accumulates dgamma / dbeta and clears the slot for the next use.
+// Block 0 also accumulates dgamma / dbeta.  Each of the six slots serves one BN of one call (zeroed by the call's memset).
 __global__ void __launch_bounds__(256) k_bn_bwd_apply(float* __restrict__ g, const float* __restrict__ y,
                                                        const float* __restrict__ stat, const float* __restrict__ gamma,
                                                        int64_t R, const BnBwdSlot* __restrict__ slot,
@@ -194,6 +197,7 @@ __global__ void k_embed_grad_unpack(const float* __restrict__ C, int nf, float* 
 }
 
 constexpr int64_t kBwdSmall = 16384;  // 6 BnBwdSlot (2 KiB each) + 2 x [128][4] embedding scratch
+constexpr int64_t kStageWidth = 9 * E + FF;  // floats per row and layer of vrpx_debug_encoder_backward_stages
 
 }  // namespace vrpx
 
@@ -221,11 +225,15 @@ int64_t vrpx_encoder_backward_workspace_bytes(int64_t B, int32_t N) {
   return kBwdSmall + B * (int64_t)N * (512 + 128 + 8) * (int64_t)sizeof(float);
 }
 
-int vrpx_encoder_backward(const vrpx_encoder_weights* w, const vrpx_encoder_weights_t* wt, const vrpx_env* env,
-                          const float* x, const int32_t* depot, int64_t B, int32_t N, const float* saved,
-                          float* g, const vrpx_encoder_grads* grads, void* ws, int64_t ws_bytes, int32_t gemm_path,
-                          void* stream_) {
-  cudaStream_t stream = (cudaStream_t)stream_;
+}  // extern "C"
+
+// The body of vrpx_encoder_backward.  stages == NULL: the production call.  Otherwise, for every layer l whose bit is set
+// in layer_mask, the eight gradients the kernels hold inside layer l are copied into stages (see
+// vrpx_debug_encoder_backward_stages) on the call's stream.
+static int encoder_backward_impl(const vrpx_encoder_weights* w, const vrpx_encoder_weights_t* wt, const vrpx_env* env,
+                                 const float* x, const int32_t* depot, int64_t B, int32_t N, const float* saved, float* g,
+                                 const vrpx_encoder_grads* grads, void* ws, int64_t ws_bytes, int32_t gemm_path,
+                                 cudaStream_t stream, float* stages, int32_t layer_mask) {
   VRPX_CHECK_ARG(w && wt && saved && g && grads && ws, "NULL argument");
   VRPX_DEVICE_GUARD(g);
   NvtxRange nvtx_range("vrpx:encoder_backward");
@@ -250,6 +258,15 @@ int vrpx_encoder_backward(const vrpx_encoder_weights* w, const vrpx_encoder_weig
     const vrpx_encoder_layer& L = w->layer[l];
     const vrpx_encoder_layer_t& LT = wt->layer[l];
     const vrpx_encoder_layer_grads& G = grads->layer[l];
+    // this layer's stage blocks: behind those of the selected layers below it
+    float* st = (stages && (layer_mask >> l & 1))
+                    ? stages + (int64_t)__builtin_popcount(layer_mask & ((1 << l) - 1)) * R * kStageWidth
+                    : nullptr;
+    auto stage = [&](const float* src, int64_t col0, int width) -> int {
+      if (st) VRPX_CUDA(cudaMemcpyAsync(st + R * col0, src, (size_t)(R * width) * sizeof(float), cudaMemcpyDeviceToDevice, stream));
+      return VRPX_OK;
+    };
+    if ((rc = stage(g, 0, E))) return rc;                                                      // dOUT
     const float* Lb = saved + R * 384 + (int64_t)l * R * 1408;
     const float *QKV = Lb, *ATT = Lb + R * 384, *Y1 = Lb + R * 512, *H1 = Lb + R * 640, *F = Lb + R * 768,
                 *Y2 = Lb + R * 1280;
@@ -260,6 +277,7 @@ int vrpx_encoder_backward(const vrpx_encoder_weights* w, const vrpx_encoder_weig
     k_bn_bwd_apply<<<ew_grid, 256, 0, stream>>>(g, Y2, sv_stats + (2 * l + 1) * 256, L.bn2_w, R, slots + 2 * l + 1,
                                                 G.bn2_w, G.bn2_b);
     VRPX_LAUNCH_CHECK();
+    if ((rc = stage(g, E, E))) return rc;                                                      // dY2
     // ---- FF backward:  y2 = h1 + relu(h1 W1^T + b1) W2^T + b2
     if ((rc = gemm_tn_accumulate(g, F, G.ff2_w, G.ff2_b, R, E, FF, stream))) return rc;       // dW2 [128][512] += dy2^T F, db2 += colsum(dy2)
     {
@@ -267,23 +285,27 @@ int vrpx_encoder_backward(const vrpx_encoder_weights* w, const vrpx_encoder_weig
       a.gate = F;
       if ((rc = gemm(a, stream))) return rc;
     }
+    if ((rc = stage(T512, 2 * E, FF))) return rc;                                              // dPRE
     if ((rc = gemm_tn_accumulate(T512, H1, G.ff0_w, G.ff0_b, R, FF, E, stream))) return rc;   // dW1 [512][128] += dpre^T h1, db1
     {
       GemmArgs a{T512, R, FF, LT.ff0_wT, E, nullptr, 0, g, nullptr, nullptr, g};              // dh1 = dy2 + dpre W1
       if ((rc = gemm(a, stream))) return rc;
     }
+    if ((rc = stage(g, 2 * E + FF, E))) return rc;                                             // dH1
     // ---- BN1 backward: g = d(h1) -> d(y1)
     k_bn_bwd_reduce<<<num_sms() * 4, 256, 0, stream>>>(g, Y1, sv_stats + (2 * l) * 256, R, slots + 2 * l);
     VRPX_LAUNCH_CHECK();
     k_bn_bwd_apply<<<ew_grid, 256, 0, stream>>>(g, Y1, sv_stats + (2 * l) * 256, L.bn1_w, R, slots + 2 * l, G.bn1_w,
                                                 G.bn1_b);
     VRPX_LAUNCH_CHECK();
+    if ((rc = stage(g, 3 * E + FF, E))) return rc;                                             // dY1
     // ---- attention block backward:  y1 = x + att W_o^T + b_o,  att = MHA_core(x W_in^T + b_in)
     if ((rc = gemm_tn_accumulate(g, ATT, G.out_proj_w, G.out_proj_b, R, E, E, stream))) return rc;   // dW_o += dy1^T att, db_o
     {
       GemmArgs a{g, R, E, LT.out_proj_wT, E, nullptr, 0, nullptr, nullptr, nullptr, T128};    // datt = dy1 W_o
       if ((rc = gemm(a, stream))) return rc;
     }
+    if ((rc = stage(T128, 4 * E + FF, E))) return rc;                                          // dATT
     float* dQKV = T512;  // [R][384]
     if (gemm_path == 0) {   // tensor pipe (attention_bwd.cu); the fp32 SIMT kernel stays as the cross-check path
       if ((rc = attention_backward_mma(QKV, ATT, T128, dQKV, B, N, stream))) return rc;
@@ -291,11 +313,13 @@ int vrpx_encoder_backward(const vrpx_encoder_weights* w, const vrpx_encoder_weig
       k_enc_attention_bwd<<<(unsigned)(B * 2), 128, attn_smem, stream>>>(QKV, ATT, T128, dQKV, N);
       VRPX_LAUNCH_CHECK();
     }
+    if ((rc = stage(dQKV, 5 * E + FF, 3 * E))) return rc;                                      // dQKV
     if ((rc = gemm_tn_accumulate(dQKV, Hin, G.in_proj_w, G.in_proj_b, R, 3 * E, E, stream))) return rc;   // dW_in [384][128], db_in
     {
       GemmArgs a{dQKV, R, 3 * E, LT.in_proj_wT, E, nullptr, 0, g, nullptr, nullptr, g};       // dx = dy1 + dqkv W_in
       if ((rc = gemm(a, stream))) return rc;
     }
+    if ((rc = stage(g, 8 * E + FF, E))) return rc;                                             // dX
   }
   // ---- embedding backward (graph_encoder.py:54 / :110-132)
   k_embed_features<<<(unsigned)((R + 255) / 256), 256, 0, stream>>>(
@@ -311,6 +335,26 @@ int vrpx_encoder_backward(const vrpx_encoder_weights* w, const vrpx_encoder_weig
     VRPX_LAUNCH_CHECK();
   }
   return VRPX_OK;
+}
+
+extern "C" {
+
+int vrpx_encoder_backward(const vrpx_encoder_weights* w, const vrpx_encoder_weights_t* wt, const vrpx_env* env,
+                          const float* x, const int32_t* depot, int64_t B, int32_t N, const float* saved,
+                          float* g, const vrpx_encoder_grads* grads, void* ws, int64_t ws_bytes, int32_t gemm_path,
+                          void* stream) {
+  return encoder_backward_impl(w, wt, env, x, depot, B, N, saved, g, grads, ws, ws_bytes, gemm_path, (cudaStream_t)stream,
+                               nullptr, 0);
+}
+
+int vrpx_debug_encoder_backward_stages(const vrpx_encoder_weights* w, const vrpx_encoder_weights_t* wt,
+                                       const vrpx_env* env, const float* x, const int32_t* depot, int64_t B, int32_t N,
+                                       const float* saved, float* g, const vrpx_encoder_grads* grads, void* ws,
+                                       int64_t ws_bytes, int32_t gemm_path, float* stages, int32_t layer_mask,
+                                       void* stream) {
+  VRPX_CHECK_ARG(stages && layer_mask >= 1 && layer_mask < (1 << VRPX_LAYERS), "stages buffer and a layer mask in 1..7");
+  return encoder_backward_impl(w, wt, env, x, depot, B, N, saved, g, grads, ws, ws_bytes, gemm_path, (cudaStream_t)stream,
+                               stages, layer_mask);
 }
 
 }  // extern "C"

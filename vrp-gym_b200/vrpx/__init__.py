@@ -167,6 +167,9 @@ def lib():
     L.vrpx_debug_encoder_fuse_attention.argtypes = [i32]
     L.vrpx_debug_encoder_fuse_attention.restype = None
     L.vrpx_debug_score_table.argtypes = [vp, vp, i64, i32, vp, vp]
+    L.vrpx_debug_encoder_backward_stages.argtypes = [C.POINTER(EncoderWeights), C.POINTER(EncoderWeightsT),
+                                                     C.POINTER(EnvView), vp, vp, i64, i32, vp, vp, C.POINTER(EncoderGrads),
+                                                     vp, i64, i32, vp, i32, vp]
     if L.vrpx_abi_version() != ABI_VERSION:
         raise VrpxError("libvrpx.so ABI version mismatch")
     _lib = L

@@ -157,8 +157,13 @@ def decoder_backward(dec, env, h, roll, wts, gemm_path=0):
     return g["dH"]
 
 
-def encoder_backward(enc, env, depot, saved, dH, gemm_path=0):
-    """Back-propagate dL/dh (overwritten) through the train-mode encoder; accumulates the parameters' .grad."""
+def encoder_backward(enc, env, depot, saved, dH, gemm_path=0, stages=None, stage_layers=0b111):
+    """Back-propagate dL/dh through the train-mode encoder; accumulates the parameters' .grad.  dH is overwritten with
+    dL/d(embedding output), which is also returned.
+
+    stages (tests): a float32 CUDA buffer of B·N·1664 floats per layer set in the bit mask stage_layers; the call then
+    goes through vrpx_debug_encoder_backward_stages, which fills it with every layer's stage gradients (include/vrpx.h)
+    in the scale of dL/dh times _grad_gain(dL/dh)."""
     L = vrpx.lib()
     dev = dH.device
     B, N = env.batch_size, env.num_nodes
@@ -206,11 +211,16 @@ def encoder_backward(enc, env, depot, saved, dH, gemm_path=0):
         G_.bn2_w, G_.bn2_b = vp_(layer.bn2.norm.weight), vp_(layer.bn2.norm.bias)
     nbytes = int(L.vrpx_encoder_backward_workspace_bytes(B, N))
     ws = torch.empty((nbytes,), dtype=torch.uint8, device=dev)
-    vrpx.check(L.vrpx_encoder_backward(C.byref(w), C.byref(wt), C.byref(env._view()), None,
-                                       vrpx.ptr(depot) if depot is not None else None, B, N, vrpx.ptr(saved),
-                                       vrpx.ptr(dH), C.byref(gr), vrpx.ptr(ws), nbytes, gemm_path, vrpx.stream_ptr(dev)))
+    args = (C.byref(w), C.byref(wt), C.byref(env._view()), None, vrpx.ptr(depot) if depot is not None else None, B, N,
+            vrpx.ptr(saved), vrpx.ptr(dH), C.byref(gr), vrpx.ptr(ws), nbytes, gemm_path)
+    if stages is None:
+        vrpx.check(L.vrpx_encoder_backward(*args, vrpx.stream_ptr(dev)))
+    else:
+        assert stages.dtype == torch.float32 and stages.numel() >= B * N * 1664 * bin(stage_layers).count("1")
+        vrpx.check(L.vrpx_debug_encoder_backward_stages(*args, vrpx.ptr(stages), stage_layers, vrpx.stream_ptr(dev)))
     if gain != 1.0:
         flat.mul_(1.0 / gain)
+        dH.mul_(1.0 / gain)
     if not bool(torch.isfinite(flat.sum())):
         raise vrpx.VrpxError("encoder backward: non-finite gradient (an operand of the f16-split GEMMs left the f16 range; "
                              "gain %g)" % gain)
